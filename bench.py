@@ -5,6 +5,7 @@
     python -m torch.distributed.run --nnodes=1 --nproc-per-node 8 --master-addr 127.0.0.1 --master-port P \
         bench.py --gpus 8 --steps 10 --warmup 3
     python bench.py --impl reference ...          # CPU restatement of the reference algorithm on the host cores
+    python bench.py ... --dump-outputs DIR        # also writes the last timed step's logL vector to DIR/logl.npy
 
 A "step" is one pass of the hot path — fused approx (K1) + batched celerite factor/solve/logdet (K2) — over one batch
 of B parameter vectors per GPU against one resident time series.  The batch is sharded over the ranks with no
@@ -48,7 +49,32 @@ def parse_args():
     ap.add_argument("--single-process", action="store_true",
                     help="ONE process drives --gpus N devices through a device-group context (pioran_ctx_create_multi): "
                          "end-to-end host-pointer call only; not the driver's contract line (that one is torchrun, one rank per GPU)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the logL vector the timed path returned in its last step to DIR/logl.npy (float64)")
+    args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    return args
+
+
+DUMP_MAX_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, logl):
+    """Writes logL as out_dir/logl.npy (float64) so that two builds can be compared output for output on the same seeded
+    inputs.  A vector larger than DUMP_MAX_BYTES is replaced by a fixed, seeded sample of its rows, whose row numbers go to
+    out_dir/logl_rows.npy; the two files together stay within DUMP_MAX_BYTES."""
+    os.makedirs(out_dir, exist_ok=True)
+    logl = np.asarray(logl, dtype=np.float64)
+    rows_path = os.path.join(out_dir, "logl_rows.npy")
+    if logl.nbytes > DUMP_MAX_BYTES:
+        k = DUMP_MAX_BYTES // 16 - 512                      # room for two .npy headers
+        rows = np.sort(np.random.default_rng(0).choice(logl.size, k, replace=False))
+        np.save(rows_path, rows.astype(np.float64))
+        logl = logl[rows]
+    elif os.path.exists(rows_path):
+        os.remove(rows_path)
+    np.save(os.path.join(out_dir, "logl.npy"), logl)
 
 
 # ------------------------------------------------------------------------------------------------ helpers
@@ -207,7 +233,9 @@ def run_reference(args, rank, world):
     t, y, s2, f_min, f_max, theta = build_workload(args.N, args.J, args.basis, min(args.B, 8192), 1234, 42)
     # each step ≈ 60 s / (steps + warmup) of CPU work so the whole run ends within a few minutes
     target = max(1.0, 60.0 / max(1, args.steps + args.warmup))
-    cb, per_step, _ = cpu_leg(t, y, s2, f_min, f_max, args.J, args.basis, theta, target, steps=args.steps, warmup=args.warmup)
+    cb, per_step, ref = cpu_leg(t, y, s2, f_min, f_max, args.J, args.basis, theta, target, steps=args.steps, warmup=args.warmup)
+    if args.dump_outputs:   # rows theta[:n]; n follows the measured CPU speed, so runs may dump prefixes of different length
+        dump_outputs(args.dump_outputs, ref)
     line = {"impl": "reference", "metric": METRIC, "value": cb["value"], "unit": UNIT, "n_gpus": args.gpus,
             "steps": args.steps, "warmup": args.warmup, "ms_per_step": per_step * 1e3, "higher_is_better": True,
             "scaling": "weak", "vs_baseline": None, "dtype": "f64", "data": "synthetic",
@@ -269,6 +297,7 @@ def measure(torch, ctx, pb, t, y, s2, f_min, f_max, J, basis, theta, steps, warm
             dist.all_gather_into_tensor(gathered, out_dev)
 
     sec = time_steps(torch, step_dev, steps, warmup, flush, dist_on)
+    last = (gathered if dist_on else out_dev).cpu().numpy()   # what the last timed step returned to the caller
     n0 = ctx.launch_count
     step_dev()
     launches = (ctx.launch_count - n0) * steps   # library kernels per step (K1 + K2) x timed steps
@@ -277,7 +306,7 @@ def measure(torch, ctx, pb, t, y, s2, f_min, f_max, J, basis, theta, steps, warm
         flush.zero_()
         ctx.approx_logl_dev([ser], [spec], B, th_dev.data_ptr(), out_dev.data_ptr())
         k2_ms.append(ctx.last_kernel_ms())
-    res = {"sec": sec, "launches": launches, "k2_ms": float(np.mean(k2_ms)), "out": out_dev.cpu().numpy()}
+    res = {"sec": sec, "launches": launches, "k2_ms": float(np.mean(k2_ms)), "out": out_dev.cpu().numpy(), "last": last}
 
     if want_e2e:
         th_pin = torch.from_numpy(theta).pin_memory()
@@ -744,6 +773,8 @@ def run_single_process(args):
     for _ in range(args.steps):
         out = ctx.approx_logl(ser, spec, th)[0]
     dt = time.perf_counter() - t0
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, out)
     line = {"metric": METRIC, "mode": "single-process device group", "value": args.B * ndev * args.steps / dt, "unit": UNIT,
             "n_gpus": ndev, "steps": args.steps, "warmup": args.warmup, "ms_per_step": dt / args.steps * 1e3,
             "higher_is_better": True, "scaling": "weak", "dtype": "f64", "data": "synthetic", "config": workload_config(args, R),
@@ -781,6 +812,8 @@ def run_b200(args, rank, world, local_rank):
         m = measure(torch, ctx, pb, t, y, s2, f_min, f_max, args.J, args.basis, theta, args.steps, args.warmup, flush,
                     world, rank)
     clocks = clk.summary()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, m["last"])
 
     def maxred(x):
         if not dist_on:

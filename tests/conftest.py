@@ -66,10 +66,10 @@ def pytest_terminal_summary(terminalreporter):
 class GoldenRun:
     """One shipped ultranest run of the reference: the series it used and the (θ, logL) pairs it produced."""
 
-    def __init__(self, stem, model, n_psd_par, log_transform):
+    def __init__(self, stem, model, n_psd_par, log_transform, chains_file="chains.npz"):
         ts = np.loadtxt(os.path.join(GOLDEN, f"{stem}_subset_time_series.txt"))
         self.t, self.y_raw, self.yerr = (np.ascontiguousarray(c) for c in ts.T)
-        chains = np.load(os.path.join(GOLDEN, "chains.npz"))
+        chains = np.load(os.path.join(GOLDEN, chains_file))
         self.chain = chains[stem]
         self.columns = [str(c) for c in chains[stem + "_columns"]]
         self.model, self.n_psd_par = model, n_psd_par
@@ -98,7 +98,7 @@ def golden_double():
 
 @pytest.fixture(scope="session")
 def golden_periodic():
-    g = GoldenRun("simu_periodic_rednoise", "SingleBendingPowerLaw", 3, False)
+    g = GoldenRun("simu_periodic_rednoise", "SingleBendingPowerLaw", 3, False, "simu_periodic_rednoise_chains.npz")
     return g
 
 
