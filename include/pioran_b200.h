@@ -185,6 +185,27 @@ int pioran_ctx_set_sweep_kernel(pioran_ctx *ctx, int which);
 int pioran_approx_logl_logshift_grad(pioran_ctx *ctx, int series_id, const pioran_approx_spec *spec, int B,
                                      const double *theta, double *logl_out, double *grad_out);
 
+/* ---- K5g: forward-mode derivatives of the explicit-coefficient likelihood ----------------------------------
+ * d/dε of pioran_celerite_logl along P directions per parameter vector (ForwardDiff's chunk over logl): for set i and
+ * direction p,  logl(a_i + ε da_ip, b_i + ε db_ip, c_i + ε dc_ip, d_i + ε dd_ip, τ, ỹ, σ̃²)  with  ỹ = y_i + ε dy_ip − (μ_i + ε dμ_ip)
+ * and  σ̃² = (ν_i + ε dν_ip)(s2_i + ε ds2_ip);  y_i, s2_i are the resident series or the rows of y_batch/s2_batch.
+ * Tangent arrays may be NULL (zero): da/db/dc/dd [B × P × Jt], dmu/dnu [B × P], dy/ds2 [B × P × N].  logl_out [B] or NULL;
+ * dlogl_out [B × P].  A term that is real for every set of the batch (b = d = 0) ignores its db, dd (exact: ∂k/∂b and ∂k/∂d
+ * vanish there).  Ranks <= 96 (PIORAN_EUNSUPPORTED above); P < 1, a NULL dlogl_out, an unknown series or B·P beyond
+ * INT_MAX give PIORAN_EINVAL.  Data tangents are uploaded in θ-chunks of at most 1 GiB. */
+int pioran_celerite_logl_jvp(pioran_ctx *ctx, int series_id, int B, int Jt, int P,
+                             const double *a, const double *b, const double *c, const double *d,
+                             const double *mu, const double *nu, const double *y_batch, const double *s2_batch,
+                             const double *da, const double *db, const double *dc, const double *dd,
+                             const double *dmu, const double *dnu, const double *dy, const double *ds2,
+                             double *logl_out, double *dlogl_out);
+/* Gradient of pioran_approx_features_logl: theta and grad_out [B × (n_psd_par + 3 + 3 n_features)], same column order
+ * (psd parameters…, norm, ν, μ, (S₀, f₀, Q)…).  The coefficients and their tangents along every θ column are formed on the
+ * device (K1 on dual numbers with the feature branch) and swept by the K5g kernel.  logl_out [B] or NULL.  Ranks <= 96,
+ * 1 … 8 features (PIORAN_EUNSUPPORTED beyond 8). */
+int pioran_approx_features_logl_grad(pioran_ctx *ctx, int series_id, const pioran_approx_spec *spec, int n_features, int B,
+                                     const double *theta, double *logl_out, double *grad_out);
+
 /* ---- K3: long single series, parallel-in-time (same recursion, N ~ 1e6) --------------------------------- */
 /* Prior transform on the device (the `prior_transform(cube)` callback of examples/ultranest/single_pl.jl:96-104, batched):
  * cube [B x ncol] unit-cube points -> theta_out [B x ncol], columns left to right.  pioran_prior_transform_logl does the

@@ -111,6 +111,33 @@ function logl_b200(a, b, c, d, τ, y, σ2)
     return out[]
 end
 
+"""
+    logl_jvp_b200(a, b, c, d, τ, y, σ2, da, db, dc, dd, dy, dσ2)
+
+Value and P directional derivatives of `logl(a, b, c, d, τ, y, σ2)` for one coefficient set (pioran_celerite_logl_jvp with B = 1):
+`da … dd` are [J × P] (column p = direction p), `dy`, `dσ2` are [N × P]; any of them may be `nothing` (zero tangent).  Returns
+`(logL, dlogL::Vector{Float64})` with `dlogL[p]` the derivative along direction p.  Ranks up to 96.
+"""
+function logl_jvp_b200(a, b, c, d, τ, y, σ2, da, db, dc, dd, dy, dσ2)
+    P = maximum(x === nothing ? 0 : size(x, 2) for x in (da, db, dc, dd, dy, dσ2))
+    P >= 1 || throw(ArgumentError("logl_jvp_b200 needs at least one tangent"))
+    s = b200_resident_series(τ)
+    out = Ref{Float64}(NaN)
+    dout = Vector{Float64}(undef, P)
+    # the C ABI takes [P × J] / [P × N] row-major per parameter vector, i.e. one direction after another: Julia's column-major
+    # [J × P] matrix already has that memory order
+    tan(x) = x === nothing ? C_NULL : Matrix{Float64}(x)
+    _b200_check(ccall((:pioran_celerite_logl_jvp, libpioran_b200), Cint,
+        (Ptr{Cvoid}, Cint, Cint, Cint, Cint, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64},
+         Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64},
+         Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64},
+         Ptr{Float64}, Ptr{Float64}),
+        b200_context().h, s.id, 1, length(a), P, Vector{Float64}(a), Vector{Float64}(b), Vector{Float64}(c), Vector{Float64}(d),
+        C_NULL, C_NULL, collect(Float64, y), collect(Float64, σ2),
+        tan(da), tan(db), tan(dc), tan(dd), C_NULL, C_NULL, tan(dy), tan(dσ2), out, dout))
+    return out[], dout
+end
+
 "Same against an explicitly uploaded series (its own y and σ² are used): B coefficient sets per call, rows of the [B × J] matrices."
 function logl_b200(a::Matrix{Float64}, b::Matrix{Float64}, c::Matrix{Float64}, d::Matrix{Float64}, s::B200Series;
         μ::Union{Nothing, Vector{Float64}} = nothing, ν::Union{Nothing, Vector{Float64}} = nothing)

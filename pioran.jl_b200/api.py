@@ -515,7 +515,7 @@ class BatchedLikelihood:
         (test/test_likelihood.jl:55, examples/turing_distributed/single_pl.jl), for a whole batch of chains at once."""
         theta = np.atleast_2d(np.asarray(theta, dtype=np.float64))
         if self.n_features:
-            raise NotImplementedError("gradients with PSD features are not built")
+            return self.ctx.approx_features_logl_grad(self.series, self.spec, self.n_features, theta)
         if self.log_shift:
             return self.ctx.approx_logl_logshift_grad(self.series, self.spec, theta)
         return self.ctx.approx_logl_grad(self.series, self.spec, theta)

@@ -254,6 +254,50 @@ class Context:
         check(self.lib.pioran_approx_logl_logshift_grad(self.h, series.id, C.byref(spec), B, _p(theta), _p(out), _p(grad)))
         return out, grad
 
+    # -- K5g: forward-mode derivatives of the explicit-coefficient likelihood
+    def celerite_logl_jvp(self, series, a, b, c, d, *, da=None, db=None, dc=None, dd=None, mu=None, nu=None, dmu=None,
+                          dnu=None, y_batch=None, s2_batch=None, dy=None, ds2=None):
+        """d/dε of celerite_logl along P directions per coefficient set (ForwardDiff's chunk mode over logl).
+        a, b, c, d [B × Jt]; tangents da, db, dc, dd [B × P × Jt], dmu, dnu [B × P], dy, ds2 [B × P × N]; a tangent left out is
+        zero, and at least one must be given (P is read from their shapes).  Returns (logL [B], dlogL [B × P])."""
+        a, b, c, d = (np.atleast_2d(_f64(x)) for x in (a, b, c, d))
+        B, Jt = a.shape
+        for x in (b, c, d):
+            if x.shape != (B, Jt):
+                raise ValueError("a, b, c, d must have the same shape")
+        N = series.N
+        tangents = {"da": (da, Jt), "db": (db, Jt), "dc": (dc, Jt), "dd": (dd, Jt), "dmu": (dmu, None), "dnu": (dnu, None),
+                    "dy": (dy, N), "ds2": (ds2, N)}
+        Ps = {name: np.shape(x)[1] for name, (x, _) in tangents.items() if x is not None and np.ndim(x) >= 2}
+        if not any(x is not None for x, _ in tangents.values()):
+            raise ValueError("at least one tangent (da, db, dc, dd, dmu, dnu, dy, ds2) must be given")
+        if len(set(Ps.values())) != 1:
+            raise ValueError(f"the tangents disagree on the number of directions P: {Ps}")
+        P = next(iter(Ps.values()))
+        conv = {name: (_f64(x, (B, P) if inner is None else (B, P, inner)) if x is not None else None)
+                for name, (x, inner) in tangents.items()}
+        mu = _f64(mu, (B,)) if mu is not None else None
+        nu = _f64(nu, (B,)) if nu is not None else None
+        yb = _f64(y_batch, (B, N)) if y_batch is not None else None
+        sb = _f64(s2_batch, (B, N)) if s2_batch is not None else None
+        out, grad = np.empty(B), np.empty((B, P))
+        check(self.lib.pioran_celerite_logl_jvp(self.h, series.id, B, Jt, P, _p(a), _p(b), _p(c), _p(d), _p(mu), _p(nu), _p(yb),
+                                                _p(sb), *[_p(conv[n]) for n in ("da", "db", "dc", "dd", "dmu", "dnu", "dy", "ds2")],
+                                                _p(out), _p(grad)))
+        return out, grad
+
+    def approx_features_logl_grad(self, series, spec, n_features, theta):
+        """theta rows = [psd parameters…, norm, ν, μ, (S₀, f₀, Q)…] → (logL [B], ∂logL/∂θ [B × n_col]) in the column order of theta."""
+        theta = np.atleast_2d(_f64(theta))
+        ncol = N_PSD_PAR[spec.psd_model] + 3 + 3 * int(n_features)
+        if theta.shape[1] != ncol:
+            raise ValueError(f"theta must have {ncol} columns")
+        B = theta.shape[0]
+        out, grad = np.empty(B), np.empty((B, ncol))
+        check(self.lib.pioran_approx_features_logl_grad(self.h, series.id, C.byref(spec), int(n_features), B, _p(theta), _p(out),
+                                                        _p(grad)))
+        return out, grad
+
     def approx_logl_grad_dev(self, series, spec, B, theta_ptr, logl_ptr, grad_ptr):
         """Device-resident variant: raw device pointers (ints); logl_ptr may be 0."""
         check(self.lib.pioran_approx_logl_grad_dev(self.h, series.id, C.byref(spec), int(B), C.c_void_p(theta_ptr),

@@ -32,6 +32,7 @@
 #include "wide_grad.cuh"
 #include "scan_wide.cuh"
 #include "scan_blocked.cuh"
+#include "jvp.cuh"
 
 using namespace pioran;
 
@@ -63,7 +64,7 @@ static int guard_fail() {
     } while (0)
 
 extern "C" const char* pioran_last_error(void) { return g_err.c_str(); }
-extern "C" int pioran_version(void) { return 200; }   // 0.2.0: device groups, sweep-kernel selector
+extern "C" int pioran_version(void) { return 300; }   // 0.3.0: JVP of the explicit-coefficient likelihood, gradients with PSD features
 
 // ------------------------------------------------------------------------------------------------ context
 namespace {
@@ -1932,6 +1933,184 @@ extern "C" int pioran_approx_features_logl(pioran_ctx* c, int series_id, const p
     for (int i = 0; i < B; i++) { nu[i] = theta[(size_t)i * ts + npar + 1]; mu[i] = theta[(size_t)i * ts + npar + 2]; }
     return generic_logl_locked(c, s, B, Jt, co.data(), co.data() + n, co.data() + 2 * n, co.data() + 3 * n, mu.data(), nu.data(),
                                nullptr, nullptr, logl_out);
+} catch (...) { return guard_fail(); }
+
+// ------------------------------------------------------------------------------------------------ K5g: JVP on explicit coefficients
+// Shared by pioran_celerite_logl_jvp and pioran_approx_features_logl_grad: `ja` holds the device pointers of the inputs and
+// outputs (B parameter vectors, P directions); the series, term rows and shape are filled in here.  The context is locked by
+// the caller; R <= JVP_MAX_RANK.
+static int jvp_dev_locked(pioran_ctx* c, Series* s, int B, int Jt, int P, int R, const std::vector<int>& term_row, JvpArgs ja) {
+    int rc;
+    if ((rc = c->rows.ensure(sizeof(int) * (Jt + 1)))) return rc;
+    CUDA_TRY(cudaMemcpyAsync(c->rows.p, term_row.data(), sizeof(int) * Jt, cudaMemcpyHostToDevice, c->stream));
+    ja.t = s->t; ja.y = s->y; ja.s2 = s->s2; ja.N = s->N;
+    ja.term_row = c->rows.as<int>();
+    ja.Jt = Jt; ja.P = P;
+    const int TS = std::max(1, (R + 15) / 16);
+    const unsigned grid = (unsigned)B * (unsigned)P;
+    cudaEventRecord(c->ev_beg, c->stream);
+    switch (TS) {
+        case 1: celerite_jvp_kernel<1><<<grid, WIDE_THREADS, 0, c->stream>>>(ja); break;
+        case 2: celerite_jvp_kernel<2><<<grid, WIDE_THREADS, 0, c->stream>>>(ja); break;
+        case 3: celerite_jvp_kernel<3><<<grid, WIDE_THREADS, 0, c->stream>>>(ja); break;
+        case 4: celerite_jvp_kernel<4><<<grid, WIDE_THREADS, 0, c->stream>>>(ja); break;
+        case 5: celerite_jvp_kernel<5><<<grid, WIDE_THREADS, 0, c->stream>>>(ja); break;
+        case 6: celerite_jvp_kernel<6><<<grid, WIDE_THREADS, 0, c->stream>>>(ja); break;
+        default: return fail(PIORAN_EUNSUPPORTED, "the JVP is built for ranks <= %d (rank %d)", JVP_MAX_RANK, R);
+    }
+    cudaEventRecord(c->ev_end, c->stream);
+    c->ev_valid = true;
+    c->launches++;
+    CUDA_TRY(cudaGetLastError());
+    // term_row is the caller's host vector: the copy must have left it before the caller may drop it
+    CUDA_TRY(cudaStreamSynchronize(c->stream));
+    return 0;
+}
+
+extern "C" int pioran_celerite_logl_jvp(pioran_ctx* c, int series_id, int B, int Jt, int P, const double* a, const double* b,
+                                        const double* cc, const double* d, const double* mu, const double* nu,
+                                        const double* y_batch, const double* s2_batch, const double* da, const double* db,
+                                        const double* dc, const double* dd, const double* dmu, const double* dnu,
+                                        const double* dy, const double* ds2, double* logl_out, double* dlogl_out) try {
+    if (!c || !a || !b || !cc || !d || !dlogl_out) return fail(PIORAN_EINVAL, "NULL argument");
+    if (B < 1 || Jt < 1) return fail(PIORAN_EINVAL, "B and Jt must be >= 1");
+    if (P < 1) return fail(PIORAN_EINVAL, "P must be >= 1 (got %d)", P);
+    if ((long long)B * P > 0x7fffffffLL) return fail(PIORAN_EINVAL, "B * P too large");
+    if (is_group(c)) {
+        std::vector<int> cid(c->children.size());
+        int64_t Ng = 0;
+        { std::lock_guard<std::mutex> lk(c->mu); for (size_t k = 0; k < cid.size(); k++) { const int rc = group_series_id(c, series_id, k, &cid[k]); if (rc) return rc; } }
+        if (y_batch || s2_batch || dy || ds2) { const int rc = pioran_series_length(c->children[0], cid[0], &Ng); if (rc) return rc; }
+        return group_split(c, B, [&](int k, int beg, int nb) -> int {
+            const size_t o = (size_t)beg * Jt, op = (size_t)beg * P;
+            return pioran_celerite_logl_jvp(c->children[k], cid[k], nb, Jt, P, a + o, b + o, cc + o, d + o, mu ? mu + beg : nullptr,
+                                            nu ? nu + beg : nullptr, y_batch ? y_batch + (size_t)beg * Ng : nullptr,
+                                            s2_batch ? s2_batch + (size_t)beg * Ng : nullptr, da ? da + op * Jt : nullptr,
+                                            db ? db + op * Jt : nullptr, dc ? dc + op * Jt : nullptr, dd ? dd + op * Jt : nullptr,
+                                            dmu ? dmu + op : nullptr, dnu ? dnu + op : nullptr, dy ? dy + op * Ng : nullptr,
+                                            ds2 ? ds2 + op * Ng : nullptr, logl_out ? logl_out + beg : nullptr, dlogl_out + op);
+        });
+    }
+    PIORAN_COMPUTE_LOCK(c);
+    CUDA_TRY(cudaSetDevice(c->device));
+    Series* s = get_series(c, series_id);
+    if (!s) return fail(PIORAN_EINVAL, "unknown series id %d", series_id);
+    std::vector<int> term_row;
+    const int R = make_term_rows(B, Jt, b, d, term_row);
+    if (R > JVP_MAX_RANK) return fail(PIORAN_EUNSUPPORTED, "the JVP is built for ranks <= %d (rank %d, Jt = %d)", JVP_MAX_RANK, R, Jt);
+    int rc;
+    GenericInputs gi;
+    const int64_t N = s->N;
+    if ((rc = upload_generic(c, B, Jt, N, a, b, cc, d, mu, nu, y_batch, s2_batch, gi))) return rc;
+    // coefficient tangents [B × P × Jt] each, then dμ, dν [B × P]
+    const size_t nt = (size_t)B * P * Jt, np = (size_t)B * P;
+    if ((rc = c->gradws.ensure(sizeof(double) * (4 * nt + 2 * np)))) return rc;
+    double* tb = c->gradws.as<double>();
+    const double* hsrc[6] = {da, db, dc, dd, dmu, dnu};
+    double* dsrc[6] = {tb, tb + nt, tb + 2 * nt, tb + 3 * nt, tb + 4 * nt, tb + 4 * nt + np};
+    for (int q = 0; q < 6; q++) {
+        if (!hsrc[q]) { dsrc[q] = nullptr; continue; }
+        CUDA_TRY(cudaMemcpyAsync(dsrc[q], hsrc[q], sizeof(double) * (q < 4 ? nt : np), cudaMemcpyHostToDevice, c->stream));
+    }
+    if ((rc = c->out.ensure(sizeof(double) * (size_t)B * (P + 1)))) return rc;
+    double* gl = c->out.as<double>();
+    double* gg = gl + B;
+    // data tangents [B × P × N]: θ-chunks of at most 1 GiB for dy and ds2 together
+    const bool dt = dy || ds2;
+    const int chunk = dt ? (int)std::max<int64_t>(1, std::min<int64_t>(B, ((int64_t)1 << 30) / (16 * (int64_t)P * std::max<int64_t>(N, 1)))) : B;
+    const size_t nc = (size_t)chunk * P * N;
+    if (dt && (rc = c->post.ensure(sizeof(double) * 2 * nc))) return rc;
+    for (int off = 0; off < B; off += chunk) {
+        const int nb = std::min(chunk, B - off);
+        const size_t o = (size_t)off * Jt, op = (size_t)off * P, nd = (size_t)nb * P * N;
+        JvpArgs ja{};
+        ja.a = gi.a + o; ja.b = gi.b + o; ja.c = gi.c + o; ja.d = gi.d + o;
+        ja.mu = gi.mu ? gi.mu + off : nullptr; ja.nu = gi.nu ? gi.nu + off : nullptr;
+        ja.y_batch = gi.yb ? gi.yb + (size_t)off * N : nullptr; ja.s2_batch = gi.sb ? gi.sb + (size_t)off * N : nullptr;
+        ja.da = dsrc[0] ? dsrc[0] + op * Jt : nullptr; ja.db = dsrc[1] ? dsrc[1] + op * Jt : nullptr;
+        ja.dc = dsrc[2] ? dsrc[2] + op * Jt : nullptr; ja.dd = dsrc[3] ? dsrc[3] + op * Jt : nullptr;
+        ja.dmu = dsrc[4] ? dsrc[4] + op : nullptr; ja.dnu = dsrc[5] ? dsrc[5] + op : nullptr;
+        if (dy) {
+            ja.dy = c->post.as<double>();
+            CUDA_TRY(cudaMemcpyAsync(c->post.p, dy + op * N, sizeof(double) * nd, cudaMemcpyHostToDevice, c->stream));
+        }
+        if (ds2) {
+            ja.ds2 = c->post.as<double>() + nc;
+            CUDA_TRY(cudaMemcpyAsync(c->post.as<double>() + nc, ds2 + op * N, sizeof(double) * nd, cudaMemcpyHostToDevice, c->stream));
+        }
+        ja.logl = gl + off; ja.dlogl = gg + op;
+        if ((rc = jvp_dev_locked(c, s, nb, Jt, P, R, term_row, ja))) return rc;
+    }
+    if (logl_out) CUDA_TRY(cudaMemcpyAsync(logl_out, gl, sizeof(double) * (size_t)B, cudaMemcpyDeviceToHost, c->stream));
+    CUDA_TRY(cudaMemcpyAsync(dlogl_out, gg, sizeof(double) * np, cudaMemcpyDeviceToHost, c->stream));
+    CUDA_TRY(cudaStreamSynchronize(c->stream));
+    return PIORAN_OK;
+} catch (...) { return guard_fail(); }
+
+// Gradient with PSD features: K1 on pairs (approx_features_grad_kernel) writes the coefficients and their tangents along every θ
+// column into the JVP's device layout, then one K5g sweep with P = θ columns.  Nothing returns to the host in between.
+extern "C" int pioran_approx_features_logl_grad(pioran_ctx* c, int series_id, const pioran_approx_spec* spec, int n_features,
+                                                int B, const double* theta, double* logl_out, double* grad_out) try {
+    if (!c || !spec || !theta || !grad_out) return fail(PIORAN_EINVAL, "NULL argument");
+    if (B < 1) return fail(PIORAN_EINVAL, "B must be >= 1");
+    const int npar = n_psd_par_of(spec->psd_model);
+    if (npar < 0) return fail(PIORAN_EINVAL, "unknown psd_model %d", spec->psd_model);
+    if (n_features < 1) return fail(PIORAN_EINVAL, "n_features must be >= 1 (got %d)", n_features);
+    if (n_features > MAXFEAT) return fail(PIORAN_EUNSUPPORTED, "at most %d features (got %d)", MAXFEAT, n_features);
+    const int ts = npar + 3 + 3 * n_features;
+    if ((long long)B * ts > 0x7fffffffLL) return fail(PIORAN_EINVAL, "B too large");
+    if (is_group(c)) {
+        std::vector<int> cid(c->children.size());
+        { std::lock_guard<std::mutex> lk(c->mu); for (size_t k = 0; k < cid.size(); k++) { const int rc = group_series_id(c, series_id, k, &cid[k]); if (rc) return rc; } }
+        return group_split(c, B, [&](int k, int beg, int nb) -> int {
+            return pioran_approx_features_logl_grad(c->children[k], cid[k], spec, n_features, nb, theta + (size_t)beg * ts,
+                                                    logl_out ? logl_out + beg : nullptr, grad_out + (size_t)beg * ts);
+        });
+    }
+    PIORAN_COMPUTE_LOCK(c);
+    CUDA_TRY(cudaSetDevice(c->device));
+    int rc;
+    if ((rc = check_spec(*spec))) return rc;
+    Series* s = get_series(c, series_id);
+    if (!s) return fail(PIORAN_EINVAL, "unknown series id %d", series_id);
+    const int J = spec->n_components, nf = n_features;
+    const int Jc = spec->basis == PIORAN_BASIS_SHO ? J : 2 * J, Jt = Jc + nf;
+    const int Rc = rank_of(spec->basis, J), R = Rc + 2 * nf;
+    if (R > JVP_MAX_RANK) return fail(PIORAN_EUNSUPPORTED, "gradients with features are built for ranks <= %d (rank %d)", JVP_MAX_RANK, R);
+    ApproxPlan* plan;
+    if ((rc = get_plan(c, *spec, &plan))) return rc;
+    // term rows: continuum as in the approx path (SHO complex; DRWCelerite complex ++ real), features complex
+    std::vector<int> term_row(Jt + 1, 0);
+    for (int j = 0; j < J; j++) {
+        term_row[j] = 2 * j;
+        if (spec->basis != PIORAN_BASIS_SHO) term_row[J + j] = -(2 * J + j + 1);
+    }
+    for (int f = 0; f < nf; f++) term_row[Jc + f] = Rc + 2 * f;
+    const int P = ts;
+    const size_t n = (size_t)B * Jt, nt = (size_t)B * P * Jt, np = (size_t)B * P;
+    if ((rc = c->theta.ensure(sizeof(double) * (size_t)B * ts))) return rc;
+    if ((rc = c->coef.ensure(sizeof(double) * (4 * n + 2 * (size_t)B)))) return rc;
+    if ((rc = c->gradws.ensure(sizeof(double) * (4 * nt + 2 * np)))) return rc;
+    if ((rc = c->out.ensure(sizeof(double) * (size_t)B * (P + 1)))) return rc;
+    CUDA_TRY(cudaMemcpyAsync(c->theta.p, theta, sizeof(double) * (size_t)B * ts, cudaMemcpyHostToDevice, c->stream));
+    double* co = c->coef.as<double>();
+    double* tg = c->gradws.as<double>();
+    double* gl = c->out.as<double>();
+    double* gg = gl + B;
+    approx_features_grad_kernel<<<(unsigned)((np + 127) / 128), 128, 0, c->stream>>>(
+        plan, B, c->theta.as<double>(), ts, nf, npar + 3, co, co + n, co + 2 * n, co + 3 * n, co + 4 * n, co + 4 * n + B,
+        tg, tg + nt, tg + 2 * nt, tg + 3 * nt, tg + 4 * nt, tg + 4 * nt + np);
+    c->launches++;
+    CUDA_TRY(cudaGetLastError());
+    JvpArgs ja{};
+    ja.a = co; ja.b = co + n; ja.c = co + 2 * n; ja.d = co + 3 * n; ja.mu = co + 4 * n; ja.nu = co + 4 * n + B;
+    ja.da = tg; ja.db = tg + nt; ja.dc = tg + 2 * nt; ja.dd = tg + 3 * nt; ja.dmu = tg + 4 * nt; ja.dnu = tg + 4 * nt + np;
+    ja.logl = gl; ja.dlogl = gg;
+    if ((rc = jvp_dev_locked(c, s, B, Jt, P, R, term_row, ja))) return rc;
+    if (logl_out) CUDA_TRY(cudaMemcpyAsync(logl_out, gl, sizeof(double) * (size_t)B, cudaMemcpyDeviceToHost, c->stream));
+    CUDA_TRY(cudaMemcpyAsync(grad_out, gg, sizeof(double) * np, cudaMemcpyDeviceToHost, c->stream));
+    CUDA_TRY(cudaStreamSynchronize(c->stream));
+    return PIORAN_OK;
 } catch (...) { return guard_fail(); }
 
 // ------------------------------------------------------------------------------------------------ posterior mean, draws

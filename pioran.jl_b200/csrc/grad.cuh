@@ -410,4 +410,130 @@ __global__ void __launch_bounds__(NW * 32, 1) celerite_grad_kernel(const GradArg
     }
 }
 
+// ------------------------------------------------------------------------------------------------ K1 on pairs with PSD features
+// Gradient of pioran_approx_features_logl: the feature branch of approx_kernel (src/psd.jl:15-44, 229-243) on pairs, one thread
+// per (parameter vector i, θ-direction k), k over every column of the θ row [psd parameters…, norm, ν, μ, (S₀, f₀, Q)…].  Unlike
+// approx_grad_kernel, c and d of the feature terms depend on θ (f₀, Q), so the output is the full coefficient set (a, b, c, d)
+// with its tangent, written straight into the layout of celerite_jvp_kernel (jvp.cuh): the sweep that follows is the JVP with
+// P = tstride directions.  The coupling runs both ways: the continuum parameters move the feature amplitudes (division by the
+// PSD at the first grid point, and the normalisation integral), the feature parameters move the continuum amplitudes through
+// the normalisation when it is the integrated power.  norm is one more direction (every amplitude is ∝ norm, so da = a/norm);
+// ν and μ carry no coefficient tangent and enter as dν = 1, dμ = 1.
+__device__ __forceinline__ D2 sqrt2d(D2 x) { const double r = sqrt(x.v); return mk2(r, 0.5 * x.d / r); }
+__device__ __forceinline__ D2 atan2d(D2 y, D2 x) {
+    return mk2(atan2(y.v, x.v), (x.v * y.d - y.v * x.d) / (x.v * x.v + y.v * y.v));
+}
+// integral_celerite (approx.cuh) on pairs
+__device__ __forceinline__ D2 integral_celerite2(D2 a, D2 b, D2 c, D2 d, double x) {
+    const double TWO_PI = 6.283185307179586;
+    const D2 dp = d + mk2(TWO_PI * x, 0.0), dm = d - mk2(TWO_PI * x, 0.0);
+    const D2 num = c * c + dp * dp, den = c * c + dm * dm;
+    const D2 r = div2(num, den);
+    const D2 lg = mk2(log(r.v), r.d / r.v);
+    return (1.0 / TWO_PI) * (2.0 * (a * (atan2d(c, dm) - atan2d(c, dp))) + b * lg);
+}
+
+// theta [B × tstride]; nfeat features at columns feat_off + 3f (S₀, f₀, Q); norm at n_psd_par, ν, μ at n_psd_par + 1, + 2.
+// Outputs (P = tstride directions, Jt = continuum terms + nfeat):
+//   a, b, c, d [B × Jt], mu, nu [B]                      written by the k = 0 thread
+//   da, db, dc, dd [B × P × Jt], dmu, dnu [B × P]
+__global__ void approx_features_grad_kernel(const ApproxPlan* __restrict__ plan, int B, const double* __restrict__ theta,
+                                            int tstride, int nfeat, int feat_off, double* __restrict__ a, double* __restrict__ b,
+                                            double* __restrict__ c, double* __restrict__ d, double* __restrict__ mu,
+                                            double* __restrict__ nu, double* __restrict__ da, double* __restrict__ db,
+                                            double* __restrict__ dc, double* __restrict__ dd, double* __restrict__ dmu,
+                                            double* __restrict__ dnu) {
+    const ApproxPlan& P = *plan;
+    const int ND = tstride, npar = P.n_psd_par;
+    const int gid = blockIdx.x * blockDim.x + threadIdx.x;
+    if (gid >= B * ND) return;
+    const int i = gid / ND, k = gid - i * ND;
+    const int J = P.J;
+    const double* th = theta + (size_t)i * tstride;
+    D2 par[8];
+    for (int q = 0; q < npar; q++) par[q] = mk2(th[q], q == k ? 1.0 : 0.0);
+    const D2 norm = mk2(th[npar], k == npar ? 1.0 : 0.0);
+    double x[MAXJ], dx[MAXJ];
+    // get_normalised_psd (src/psd.jl:52-56)
+    const D2 p0 = psd_eval2(P.model, par, P.fj[0]);
+    for (int j = 0; j < J; j++) {
+        const D2 r = div2(psd_eval2(P.model, par, P.fj[j]), p0);
+        x[j] = r.v; dx[j] = r.d;
+    }
+    // amplitudes = B \ p (src/psd.jl:109-112), value and tangent through the same LU
+    for (int kk = 0; kk < J; kk++) {
+        const int pk = P.piv[kk];
+        if (pk != kk) {
+            double tmp = x[kk]; x[kk] = x[pk]; x[pk] = tmp;
+            tmp = dx[kk]; dx[kk] = dx[pk]; dx[pk] = tmp;
+        }
+    }
+    for (int kk = 0; kk < J; kk++) {
+        const double xk = x[kk], dxk = dx[kk];
+        for (int r = kk + 1; r < J; r++) { const double l = P.lu[r + kk * J]; x[r] -= l * xk; dx[r] -= l * dxk; }
+    }
+    for (int kk = J - 1; kk >= 0; kk--) {
+        const double u = P.lu[kk + kk * J];
+        x[kk] /= u; dx[kk] /= u;
+        const double xk = x[kk], dxk = dx[kk];
+        for (int r = 0; r < kk; r++) { const double l = P.lu[r + kk * J]; x[r] -= l * xk; dx[r] -= l * dxk; }
+    }
+    // normalisation (src/psd.jl:236-238, 375-395): linear in the amplitudes
+    D2 integ;
+    if (P.is_integrated_power) {
+        integ.v = basis_integral(P.basis, J, x, P.fj, P.f_max) - basis_integral(P.basis, J, x, P.fj, P.f_min);
+        integ.d = basis_integral(P.basis, J, dx, P.fj, P.f_max) - basis_integral(P.basis, J, dx, P.fj, P.f_min);
+    } else {
+        double s = 0.0, ds = 0.0;
+        for (int j = 0; j < J; j++) { s += x[j] * P.fj[j]; ds += dx[j] * P.fj[j]; }
+        const double cst = (P.basis == 0) ? 3.141592653589793 / 1.4142135623730951 : 2.0 * 3.141592653589793 / 3.0;
+        integ = mk2(s * cst, ds * cst);
+    }
+    // features: convert_feature (src/psd.jl:15-28), amplitudes divided by the continuum's PSD at the first grid point
+    D2 fa[MAXFEAT], fb[MAXFEAT], fc[MAXFEAT], fd[MAXFEAT];
+    for (int f = 0; f < nfeat; f++) {
+        const int col = feat_off + 3 * f;
+        const D2 S0 = mk2(th[col], k == col ? 1.0 : 0.0);
+        const D2 f0q = mk2(th[col + 1], k == col + 1 ? 1.0 : 0.0);
+        const D2 Q = mk2(th[col + 2], k == col + 2 ? 1.0 : 0.0);
+        const D2 dl = sqrt2d(4.0 * (Q * Q) - mk2(1.0, 0.0));
+        const D2 w0 = 6.283185307179586 * f0q;
+        const D2 ak = 0.25 * (S0 * w0 * Q);
+        fa[f] = div2(ak, p0); fb[f] = div2(div2(ak, dl), p0);
+        fc[f] = 0.5 * div2(w0, Q); fd[f] = fc[f] * dl;
+        if (P.is_integrated_power)
+            integ = integ + (integral_celerite2(fa[f], fb[f], fc[f], fd[f], P.f_max) - integral_celerite2(fa[f], fb[f], fc[f], fd[f], P.f_min));
+    }
+    const D2 scale = div2(norm, integ);
+    const int Jc = P.basis == 0 ? J : 2 * J, Jt = Jc + nfeat;
+    const size_t ro = (size_t)i * Jt, to = ((size_t)i * ND + k) * Jt;
+    const bool v = k == 0;
+    const double PI = 3.141592653589793, S2 = 1.4142135623730951, S3 = 1.7320508075688772;
+    for (int j = 0; j < J; j++) {
+        if (P.basis == 0) {   // SHO: a = b = A f π/√2, c = d = √2 π f   (src/psd.jl:249-252)
+            const D2 aj = (PI / S2) * (P.fj[j] * (mk2(x[j], dx[j]) * scale));
+            const double cj = S2 * PI * P.fj[j];
+            if (v) { a[ro + j] = aj.v; b[ro + j] = aj.v; c[ro + j] = cj; d[ro + j] = cj; }
+            da[to + j] = aj.d; db[to + j] = aj.d; dc[to + j] = 0.0; dd[to + j] = 0.0;
+        } else {              // DRWCelerite: (a, √3a, πf, √3πf) ++ (a, 0, 2πf, 0)   (src/psd.jl:264-275)
+            const D2 aj = (PI / 3.0) * (P.fj[j] * (mk2(x[j], dx[j]) * scale));
+            const double cj = PI * P.fj[j];
+            if (v) {
+                a[ro + j] = aj.v; b[ro + j] = S3 * aj.v; c[ro + j] = cj; d[ro + j] = S3 * cj;
+                a[ro + J + j] = aj.v; b[ro + J + j] = 0.0; c[ro + J + j] = 2.0 * cj; d[ro + J + j] = 0.0;
+            }
+            da[to + j] = aj.d; db[to + j] = S3 * aj.d; dc[to + j] = 0.0; dd[to + j] = 0.0;
+            da[to + J + j] = aj.d; db[to + J + j] = 0.0; dc[to + J + j] = 0.0; dd[to + J + j] = 0.0;
+        }
+    }
+    for (int f = 0; f < nfeat; f++) {                           // src/psd.jl:254-259, 277-282
+        const D2 af = 2.0 * (fa[f] * scale), bf = 2.0 * (fb[f] * scale);
+        if (v) { a[ro + Jc + f] = af.v; b[ro + Jc + f] = bf.v; c[ro + Jc + f] = fc[f].v; d[ro + Jc + f] = fd[f].v; }
+        da[to + Jc + f] = af.d; db[to + Jc + f] = bf.d; dc[to + Jc + f] = fc[f].d; dd[to + Jc + f] = fd[f].d;
+    }
+    if (v) { nu[i] = th[npar + 1]; mu[i] = th[npar + 2]; }
+    dnu[(size_t)i * ND + k] = k == npar + 1 ? 1.0 : 0.0;
+    dmu[(size_t)i * ND + k] = k == npar + 2 ? 1.0 : 0.0;
+}
+
 }  // namespace pioran
