@@ -95,6 +95,13 @@ int64_t pioran_ctx_launch_count(pioran_ctx *ctx);
 /* Device time (ms, CUDA events on the context's stream) of the most recent main-kernel launch — the batched
  * celerite kernel K2, the scan K3 or the dense K4.  Waits for that launch to finish. */
 int pioran_ctx_last_kernel_ms(pioran_ctx *ctx, double *ms);
+/* Name of the kernel that launch ran, with its template integers, as a NUL-terminated string in buf[len]: one format per
+ * family, e.g. "blocked<5,5,true,16>", "blocked_wide<9,10,4>", "shared<8,4>", "shared_pair<4,8>", "generic<5,12>",
+ * "wide_reg<7>", "wide", "blocked_grad<3,3,false,4>", "grad<4,8>", "grad_pipe<8,5>", "wide_grad<5>", "jvp<4>",
+ * "scan_finish", "dense_finish".  Empty before the first launch.  Which kernel serves a shape is an implementation
+ * detail that may change between versions; this is for tests and profiles.  PIORAN_EINVAL when len is too small for the
+ * name; PIORAN_EUNSUPPORTED on a device group. */
+int pioran_ctx_last_kernel_name(pioran_ctx *ctx, char *buf, int len);
 
 /* Uploads one time series (τ, y, σ²) — the (x, Y, diag Σy) of logpdf(f(t, σ²), y), src/scalable_GP.jl:162-166 —
  * and keeps it resident.  t must be strictly increasing.  A sampler uploads once and evaluates ~1e5 times. */

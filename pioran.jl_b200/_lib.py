@@ -35,6 +35,7 @@ SYMBOLS = {
     "pioran_ctx_synchronize": (C.c_int, [C.c_void_p]),
     "pioran_ctx_launch_count": (C.c_int64, [C.c_void_p]),
     "pioran_ctx_last_kernel_ms": (C.c_int, [C.c_void_p, C.POINTER(C.c_double)]),
+    "pioran_ctx_last_kernel_name": (C.c_int, [C.c_void_p, C.c_char_p, C.c_int]),
     "pioran_series_upload": (C.c_int, [C.c_void_p, C.c_int64, _dp, _dp, _dp, _ip]),
     "pioran_series_free": (C.c_int, [C.c_void_p, C.c_int]),
     "pioran_series_length": (C.c_int, [C.c_void_p, C.c_int, C.POINTER(C.c_int64)]),

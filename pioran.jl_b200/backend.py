@@ -101,6 +101,12 @@ class Context:
         check(self.lib.pioran_ctx_last_kernel_ms(self.h, C.byref(ms)))
         return ms.value
 
+    def last_kernel_name(self):
+        """Kernel of that launch with its template integers, e.g. "blocked<5,5,true,16>" ("" before the first launch)."""
+        buf = C.create_string_buffer(64)
+        check(self.lib.pioran_ctx_last_kernel_name(self.h, buf, len(buf)))
+        return buf.value.decode()
+
     def upload_series(self, t, y, s2):
         t, y, s2 = _f64(t), _f64(y), _f64(s2)
         if not (t.ndim == 1 and t.shape == y.shape == s2.shape):

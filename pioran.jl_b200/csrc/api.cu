@@ -64,7 +64,7 @@ static int guard_fail() {
     } while (0)
 
 extern "C" const char* pioran_last_error(void) { return g_err.c_str(); }
-extern "C" int pioran_version(void) { return 300; }   // 0.3.0: JVP of the explicit-coefficient likelihood, gradients with PSD features
+extern "C" int pioran_version(void) { return 301; }   // 0.3.1: pioran_ctx_last_kernel_name
 
 // ------------------------------------------------------------------------------------------------ context
 namespace {
@@ -99,6 +99,15 @@ struct Series {
 
 using PlanKey = std::tuple<int, int, int, int, double, double, double, double>;
 
+// The most recent main-kernel launch (pioran_ctx_last_kernel_name): a kernel family and its template integers, formatted
+// only when queried so that the launch path stores four ints.
+enum KernelFamily : int {
+    KF_NONE = 0, KF_BLOCKED, KF_BLOCKED_WIDE, KF_SHARED, KF_SHARED_PAIR, KF_GENERIC, KF_WIDE_REG, KF_WIDE_REG_STORE, KF_WIDE_REG_SIM,
+    KF_WIDE, KF_BLOCKED_GRAD, KF_GRAD, KF_GRAD_PIPE, KF_WIDE_GRAD, KF_JVP, KF_PREDICT, KF_GENERIC_SIM, KF_SCAN_FINISH,
+    KF_SCAN_PARTIAL, KF_DENSE_FINISH
+};
+struct KernelTag { int family = KF_NONE; int p[4] = {0, 0, 0, 0}; };
+
 }  // namespace
 
 struct pioran_ctx {
@@ -115,6 +124,7 @@ struct pioran_ctx {
     // device time of the most recent main-kernel launch (K2/K3/K4), for bench.py's roofline line
     cudaEvent_t ev_beg = nullptr, ev_end = nullptr;
     bool ev_valid = false;
+    KernelTag last_kernel;   // which kernel that launch ran (note_kernel)
     // the work-item list of the last fused call, kept on the device while the call shape repeats (a sampler
     // evaluates the same series × batch-size shape ~1e5 times)
     std::vector<int64_t> work_key;
@@ -143,6 +153,12 @@ struct pioran_ctx {
 // Entry points that launch work or touch the context's workspaces: take the lock and invalidate a range left pending by
 // pioran_celerite_scan_range_begin (its record points into those workspaces).
 #define PIORAN_COMPUTE_LOCK(c) std::lock_guard<std::mutex> lk((c)->mu); (c)->epoch++
+// Every main-kernel launch site: the events around it are valid, and the kernel is named for pioran_ctx_last_kernel_name.
+static void note_kernel(pioran_ctx* c, int family, int p0 = 0, int p1 = 0, int p2 = 0, int p3 = 0) {
+    c->ev_valid = true;
+    c->last_kernel.family = family;
+    c->last_kernel.p[0] = p0; c->last_kernel.p[1] = p1; c->last_kernel.p[2] = p2; c->last_kernel.p[3] = p3;
+}
 static int make_term_rows(int B, int Jt, const double* b, const double* d, std::vector<int>& term_row);
 
 static int bs_for_rank(int R) {
@@ -347,6 +363,40 @@ extern "C" int pioran_ctx_last_kernel_ms(pioran_ctx* c, double* ms) try {
     float f = 0.f;
     CUDA_TRY(cudaEventElapsedTime(&f, c->ev_beg, c->ev_end));
     *ms = (double)f;
+    return PIORAN_OK;
+} catch (...) { return guard_fail(); }
+extern "C" int pioran_ctx_last_kernel_name(pioran_ctx* c, char* buf, int len) try {
+    if (!c || !buf) return fail(PIORAN_EINVAL, "NULL argument");
+    if (is_group(c)) return fail(PIORAN_EUNSUPPORTED, "a device group launches on several devices; ask a single-device context");
+    KernelTag k;
+    { std::lock_guard<std::mutex> lk(c->mu); k = c->last_kernel; }
+    const int* p = k.p;
+    char name[64];
+    switch (k.family) {
+        case KF_BLOCKED: snprintf(name, sizeof name, "blocked<%d,%d,%s,%d>", p[0], p[1], p[2] ? "true" : "false", p[3]); break;
+        case KF_BLOCKED_WIDE: snprintf(name, sizeof name, "blocked_wide<%d,%d,%d>", p[0], p[1], p[2]); break;
+        case KF_SHARED: snprintf(name, sizeof name, "shared<%d,%d>", p[0], p[1]); break;
+        case KF_SHARED_PAIR: snprintf(name, sizeof name, "shared_pair<%d,%d>", p[0], p[1]); break;
+        case KF_GENERIC: snprintf(name, sizeof name, "generic<%d,%d>", p[0], p[1]); break;
+        case KF_WIDE_REG: snprintf(name, sizeof name, "wide_reg<%d>", p[0]); break;
+        case KF_WIDE_REG_STORE: snprintf(name, sizeof name, "wide_reg_store<%d>", p[0]); break;
+        case KF_WIDE_REG_SIM: snprintf(name, sizeof name, "wide_reg_sim<%d>", p[0]); break;
+        case KF_WIDE: snprintf(name, sizeof name, "wide"); break;
+        case KF_BLOCKED_GRAD: snprintf(name, sizeof name, "blocked_grad<%d,%d,%s,%d>", p[0], p[1], p[2] ? "true" : "false", p[3]); break;
+        case KF_GRAD: snprintf(name, sizeof name, "grad<%d,%d>", p[0], p[1]); break;
+        case KF_GRAD_PIPE: snprintf(name, sizeof name, "grad_pipe<%d,%d>", p[0], p[1]); break;
+        case KF_WIDE_GRAD: snprintf(name, sizeof name, "wide_grad<%d>", p[0]); break;
+        case KF_JVP: snprintf(name, sizeof name, "jvp<%d>", p[0]); break;
+        case KF_PREDICT: snprintf(name, sizeof name, "predict<%d>", p[0]); break;
+        case KF_GENERIC_SIM: snprintf(name, sizeof name, "generic_sim<%d,%d>", p[0], p[1]); break;
+        case KF_SCAN_FINISH: snprintf(name, sizeof name, "scan_finish"); break;
+        case KF_SCAN_PARTIAL: snprintf(name, sizeof name, "scan_partial"); break;
+        case KF_DENSE_FINISH: snprintf(name, sizeof name, "dense_finish"); break;
+        default: name[0] = '\0'; break;
+    }
+    const int need = (int)strlen(name) + 1;
+    if (len < need) return fail(PIORAN_EINVAL, "buffer of %d bytes is too small for the %d-byte kernel name", len, need);
+    memcpy(buf, name, need);
     return PIORAN_OK;
 } catch (...) { return guard_fail(); }
 
@@ -641,7 +691,7 @@ static int launch_blocked_nw(pioran_ctx* c, const BatchArgs& args, int nitems, i
     cudaEventRecord(c->ev_beg, c->stream);
     kern<<<nitems, NW * 32, smem, c->stream>>>(args, R, amp_stride, blk_layout(R, false).RG);
     cudaEventRecord(c->ev_end, c->stream);
-    c->ev_valid = true;
+    note_kernel(c, KF_BLOCKED, NT, NTR, HALF, NW);
     c->launches++;
     CUDA_TRY(cudaGetLastError());
     return 0;
@@ -687,7 +737,7 @@ static int launch_blocked_wide(pioran_ctx* c, const BatchArgs& args, int nitems,
     cudaEventRecord(c->ev_beg, c->stream);
     kern<<<nitems, W * 32, smem, c->stream>>>(args, R, amp_stride, blk_layout(R, false).RG);
     cudaEventRecord(c->ev_end, c->stream);
-    c->ev_valid = true;
+    note_kernel(c, KF_BLOCKED_WIDE, NT, NTR, W);
     c->launches++;
     CUDA_TRY(cudaGetLastError());
     return 0;
@@ -740,7 +790,7 @@ static int launch_shared(pioran_ctx* c, const BatchArgs& args, int nitems) {
     cudaEventRecord(c->ev_beg, c->stream);
     kern<<<nitems, NW * 32, smem, c->stream>>>(args);
     cudaEventRecord(c->ev_end, c->stream);
-    c->ev_valid = true;
+    note_kernel(c, KF_SHARED, BS, NW);
     c->launches++;
     CUDA_TRY(cudaGetLastError());
     return 0;
@@ -764,7 +814,7 @@ static int launch_shared_pair(pioran_ctx* c, const BatchArgs& args, int nitems) 
     cudaEventRecord(c->ev_beg, c->stream);
     kern<<<nitems, NW * 32, smem, c->stream>>>(args);
     cudaEventRecord(c->ev_end, c->stream);
-    c->ev_valid = true;
+    note_kernel(c, KF_SHARED_PAIR, BS, NW);
     c->launches++;
     CUDA_TRY(cudaGetLastError());
     return 0;
@@ -778,7 +828,7 @@ static int launch_generic(pioran_ctx* c, const BatchArgs& args, int nitems) {
     cudaEventRecord(c->ev_beg, c->stream);
     kern<<<nitems, NW * 32, smem, c->stream>>>(args);
     cudaEventRecord(c->ev_end, c->stream);
-    c->ev_valid = true;
+    note_kernel(c, KF_GENERIC, BS, NW);
     c->launches++;
     CUDA_TRY(cudaGetLastError());
     return 0;
@@ -959,7 +1009,7 @@ static int launch_wide(pioran_ctx* c, const BatchArgs& args, int nitems) {
             default: celerite_wide_reg_kernel<5, MODE><<<nitems, WIDE_THREADS, 0, c->stream>>>(args); break;
         }
         cudaEventRecord(c->ev_end, c->stream);
-        c->ev_valid = true;
+        note_kernel(c, MODE == STEP_STORE ? KF_WIDE_REG_STORE : MODE == STEP_SIM ? KF_WIDE_REG_SIM : KF_WIDE_REG, std::max(5, TS));
         c->launches++;
         CUDA_TRY(cudaGetLastError());
         return 0;
@@ -971,7 +1021,7 @@ static int launch_wide(pioran_ctx* c, const BatchArgs& args, int nitems) {
     cudaEventRecord(c->ev_beg, c->stream);
     celerite_wide_kernel<<<nitems, WIDE_THREADS, smem, c->stream>>>(args);
     cudaEventRecord(c->ev_end, c->stream);
-    c->ev_valid = true;
+    note_kernel(c, KF_WIDE);
     c->launches++;
     CUDA_TRY(cudaGetLastError());
     return 0;
@@ -1384,7 +1434,7 @@ static int launch_grad_nw(pioran_ctx* c, const GradArgs& args, int nitems) {
     cudaEventRecord(c->ev_beg, c->stream);
     kern<<<nitems, NW * 32, smem, c->stream>>>(args);
     cudaEventRecord(c->ev_end, c->stream);
-    c->ev_valid = true;
+    note_kernel(c, KF_GRAD, BS, NW);
     c->launches++;
     CUDA_TRY(cudaGetLastError());
     return 0;
@@ -1399,7 +1449,7 @@ static int launch_grad_pipe(pioran_ctx* c, const GradArgs& args, int nitems) {
     cudaEventRecord(c->ev_beg, c->stream);
     kern<<<nitems, nthreads, smem, c->stream>>>(args);
     cudaEventRecord(c->ev_end, c->stream);
-    c->ev_valid = true;
+    note_kernel(c, KF_GRAD_PIPE, BS, NWARPS);
     c->launches++;
     CUDA_TRY(cudaGetLastError());
     return 0;
@@ -1419,7 +1469,7 @@ static int launch_blocked_grad(pioran_ctx* c, const GradArgs& args, int nitems, 
     cudaEventRecord(c->ev_beg, c->stream);
     kern<<<nitems, (1 + NTAN) * 32, smem, c->stream>>>(args, R, amp_stride, blk_layout(R, true).RG, blk_layout(R, true).RM);
     cudaEventRecord(c->ev_end, c->stream);
-    c->ev_valid = true;
+    note_kernel(c, KF_BLOCKED_GRAD, NT, NTR, HALF, NTAN);
     c->launches++;
     CUDA_TRY(cudaGetLastError());
     return 0;
@@ -1504,7 +1554,7 @@ static int wide_grad_locked(pioran_ctx* c, Series* ser, const pioran_approx_spec
     if (TS == 5) celerite_wide_grad_kernel<5><<<B * (ND + 1), WIDE_THREADS, 0, c->stream>>>(ga);
     else celerite_wide_grad_kernel<6><<<B * (ND + 1), WIDE_THREADS, 0, c->stream>>>(ga);
     cudaEventRecord(c->ev_end, c->stream);
-    c->ev_valid = true;
+    note_kernel(c, KF_WIDE_GRAD, TS == 5 ? 5 : 6);
     c->launches += 2;
     CUDA_TRY(cudaGetLastError());
     return 0;
@@ -1959,7 +2009,7 @@ static int jvp_dev_locked(pioran_ctx* c, Series* s, int B, int Jt, int P, int R,
         default: return fail(PIORAN_EUNSUPPORTED, "the JVP is built for ranks <= %d (rank %d)", JVP_MAX_RANK, R);
     }
     cudaEventRecord(c->ev_end, c->stream);
-    c->ev_valid = true;
+    note_kernel(c, KF_JVP, TS);
     c->launches++;
     CUDA_TRY(cudaGetLastError());
     // term_row is the caller's host vector: the copy must have left it before the caller may drop it
@@ -2205,7 +2255,7 @@ extern "C" int pioran_celerite_predict(pioran_ctx* c, int series_id, int B, int 
     }
     c->launches += 2;
     cudaEventRecord(c->ev_end, c->stream);
-    c->ev_valid = true;
+    note_kernel(c, KF_PREDICT, Jt <= 64 ? 2 : 4);
     CUDA_TRY(cudaGetLastError());
     CUDA_TRY(cudaMemcpyAsync(mean_out, mean, sizeof(double) * nBM, cudaMemcpyDeviceToHost, c->stream));
     CUDA_TRY(cudaStreamSynchronize(c->stream));   // n0 is a local
@@ -2236,7 +2286,8 @@ extern "C" int pioran_celerite_simulate(pioran_ctx* c, int series_id, int B, int
     cudaEventRecord(c->ev_beg, c->stream);
     if ((rc = BS > 8 ? launch_wide<STEP_SIM>(c, args, nitems) : dispatch_generic_mode<STEP_SIM>(c, BS, args, nitems))) return rc;
     cudaEventRecord(c->ev_end, c->stream);
-    c->ev_valid = true;
+    if (BS > 8) note_kernel(c, KF_WIDE_REG_SIM, std::max(5, (args.R + 15) / 16));
+    else note_kernel(c, KF_GENERIC_SIM, BS, nw_for_bs(BS));
     CUDA_TRY(cudaMemcpyAsync(y_out, c->post.p, sizeof(double) * nBN, cudaMemcpyDeviceToHost, c->stream));
     CUDA_TRY(cudaStreamSynchronize(c->stream));
     return PIORAN_OK;
@@ -2843,7 +2894,7 @@ static int scan_logl_locked(pioran_ctx* c, Series* s, int series_id, int B, int 
         scan_finish_kernel<<<(B + 127) / 128, 128, 0, c->stream>>>(run.parts, run.chk, run.check_scale, PS, B, s->N, run.out, run.err);
         c->launches++;
         cudaEventRecord(c->ev_end, c->stream);
-        c->ev_valid = true;
+        note_kernel(c, KF_SCAN_FINISH);
         CUDA_TRY(cudaGetLastError());
         CUDA_TRY(cudaMemcpyAsync(val.data(), run.out, sizeof(double) * (size_t)B, cudaMemcpyDeviceToHost, c->stream));
         CUDA_TRY(cudaMemcpyAsync(est.data(), run.err, sizeof(double) * (size_t)B, cudaMemcpyDeviceToHost, c->stream));
@@ -2976,7 +3027,7 @@ extern "C" int pioran_celerite_scan_range_end(pioran_ctx* c, int nprev, const do
     scan_partial_kernel<<<1, 32, 0, c->stream>>>(run.parts, run.chk, run.check_scale, run.P * run.SUB, 1, run.sums);
     c->launches++;
     cudaEventRecord(c->ev_end, c->stream);
-    c->ev_valid = true;
+    note_kernel(c, KF_SCAN_PARTIAL);
     CUDA_TRY(cudaGetLastError());
     double sums3[3], chk_first[4], chk_last[4];
     const size_t nsub = (size_t)run.P * run.SUB;
@@ -3208,6 +3259,6 @@ extern "C" int pioran_direct_logl(pioran_ctx* c, int series_id, int B, int Jt, c
         if (!marks.empty()) cudaEventDestroy(marks[0].second);
     }
     cudaEventRecord(c->ev_end, c->stream);
-    c->ev_valid = true;
+    note_kernel(c, KF_DENSE_FINISH);
     return PIORAN_OK;
 } catch (...) { return guard_fail(); }

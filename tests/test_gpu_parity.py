@@ -244,8 +244,11 @@ def test_permutation_and_split_invariance(pb, ctx, golden_single):
 
 @pytest.mark.parametrize("basis", ["SHO", "DRWCelerite"])
 def test_dispatch_tiers_agree(pb, ctx, golden_single, basis):
-    """The same rows through every CTA shape of the shared-table kernel (csrc/api.cu dispatch_shared): 4-warp CTAs (≤ 592
-    evaluations), 8 un-paired warps (≤ 1 184), the full-size kernel (θ-paired for block sizes ≤ 5)."""
+    """The same rows through the tensor-pipe kernels the default dispatch picks as the batch grows (csrc/api.cu
+    approx_logl_dev_locked): one 4-warp CTA per evaluation (blocked_wide, ≤ 296 evaluations), then the warp kernel (blocked)
+    with 4-warp CTAs (≤ 592), 8-warp CTAs (≤ 1 184) and the full-size CTA.  Each batch is compared with the rows of the full
+    batch, i.e. with the same kernel family; the scalar-pipe tiers of dispatch_shared and the oracle parity of every tier are
+    in test_gpu_sweep_matrix.py."""
     g = golden_single
     like = pb.BatchedLikelihood(g.t, g.y, g.s2, g.model, 20, basis, ctx=ctx)
     th = g.theta[:3000].copy()
