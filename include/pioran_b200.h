@@ -213,6 +213,28 @@ int pioran_celerite_logl_jvp(pioran_ctx *ctx, int series_id, int B, int Jt, int 
 int pioran_approx_features_logl_grad(pioran_ctx *ctx, int series_id, const pioran_approx_spec *spec, int n_features, int B,
                                      const double *theta, double *logl_out, double *grad_out);
 
+/* ---- K5r: reverse-mode gradient of the explicit-coefficient likelihood -------------------------------------
+ * For every set i of pioran_celerite_logl's inputs (same arguments), one backward sweep gives logL_i and its gradient with
+ * respect to a, b, c, d (ga … gd [B × Jt]), μ_i and ν_i (gmu, gnu [B]) and the data row as it enters, ỹ = y − μ and σ̃² = ν·s2
+ * (gy, gs2 [B × N]; y, s2 are the resident series or the rows of y_batch/s2_batch).  It is the function K5g differentiates:
+ * <gradient, v> = pioran_celerite_logl_jvp along v.  A term real for every set of the batch (b = d = 0) gets gb = gd = 0 exactly.
+ * Every output may be NULL, but at least one gradient output must be given.  Ranks <= 96 (PIORAN_EUNSUPPORTED above); no
+ * gradient output, an unknown series or B < 1 give PIORAN_EINVAL.  The workspace (per-step values and checkpoints of the state,
+ * about (2R + 2)·N + (⌈N/K⌉ + K)·256·⌈R/16⌉² doubles per set with K ≈ √N) is bounded by processing the batch in θ-chunks of at
+ * most 1 GiB (pioran_ctx_set_vjp_workspace). */
+int pioran_celerite_logl_vjp(pioran_ctx *ctx, int series_id, int B, int Jt,
+                             const double *a, const double *b, const double *c, const double *d,
+                             const double *mu, const double *nu, const double *y_batch, const double *s2_batch,
+                             double *logl_out, double *ga, double *gb, double *gc, double *gd,
+                             double *gmu, double *gnu, double *gy, double *gs2);
+/* Same arguments, columns and limits as pioran_approx_features_logl_grad, computed by one K5r sweep and a contraction with the
+ * coefficient tangents instead of one forward direction per θ column. */
+int pioran_approx_features_logl_grad_reverse(pioran_ctx *ctx, int series_id, const pioran_approx_spec *spec, int n_features,
+                                             int B, const double *theta, double *logl_out, double *grad_out);
+/* Cap in bytes of the K5r workspace of one θ-chunk (0 = 1 GiB, the default).  The result does not depend on it; a small cap
+ * splits a batch into many chunks (one set per chunk at least). */
+int pioran_ctx_set_vjp_workspace(pioran_ctx *ctx, long long bytes);
+
 /* ---- K3: long single series, parallel-in-time (same recursion, N ~ 1e6) --------------------------------- */
 /* Prior transform on the device (the `prior_transform(cube)` callback of examples/ultranest/single_pl.jl:96-104, batched):
  * cube [B x ncol] unit-cube points -> theta_out [B x ncol], columns left to right.  pioran_prior_transform_logl does the

@@ -138,6 +138,30 @@ function logl_jvp_b200(a, b, c, d, τ, y, σ2, da, db, dc, dd, dy, dσ2)
     return out[], dout
 end
 
+"""
+    logl_vjp_b200(a, b, c, d, τ, y, σ2)
+
+Value and gradient of `logl(a, b, c, d, τ, y, σ2)` for one coefficient set from one reverse-mode sweep
+(pioran_celerite_logl_vjp with B = 1).  Returns `(logL, (a = ∂a, b = ∂b, c = ∂c, d = ∂d, y = ∂y, σ2 = ∂σ2))`, each a
+`Vector{Float64}` of the input's length.  A term with b = d = 0 gets ∂b = ∂d = 0 exactly.  Ranks up to 96.
+"""
+function logl_vjp_b200(a, b, c, d, τ, y, σ2)
+    s = b200_resident_series(τ)
+    J, N = length(a), length(τ)
+    out = Ref{Float64}(NaN)
+    ga, gb, gc, gd = (Vector{Float64}(undef, J) for _ in 1:4)
+    gy, gσ2 = Vector{Float64}(undef, N), Vector{Float64}(undef, N)
+    _b200_check(ccall((:pioran_celerite_logl_vjp, libpioran_b200), Cint,
+        (Ptr{Cvoid}, Cint, Cint, Cint, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64},
+         Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64},
+         Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64},
+         Ptr{Float64}),
+        b200_context().h, s.id, 1, J, Vector{Float64}(a), Vector{Float64}(b), Vector{Float64}(c), Vector{Float64}(d),
+        C_NULL, C_NULL, collect(Float64, y), collect(Float64, σ2),
+        out, ga, gb, gc, gd, C_NULL, C_NULL, gy, gσ2))
+    return out[], (a = ga, b = gb, c = gc, d = gd, y = gy, σ2 = gσ2)
+end
+
 "Same against an explicitly uploaded series (its own y and σ² are used): B coefficient sets per call, rows of the [B × J] matrices."
 function logl_b200(a::Matrix{Float64}, b::Matrix{Float64}, c::Matrix{Float64}, d::Matrix{Float64}, s::B200Series;
         μ::Union{Nothing, Vector{Float64}} = nothing, ν::Union{Nothing, Vector{Float64}} = nothing)

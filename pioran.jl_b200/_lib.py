@@ -51,6 +51,9 @@ SYMBOLS = {
     "pioran_approx_logl_grad_dev": (C.c_int, [C.c_void_p, C.c_int, C.POINTER(ApproxSpec), C.c_int, C.c_void_p, C.c_void_p, C.c_void_p]),
     "pioran_celerite_logl_jvp": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int] + [_dp] * 18),
     "pioran_approx_features_logl_grad": (C.c_int, [C.c_void_p, C.c_int, C.POINTER(ApproxSpec), C.c_int, C.c_int, _dp, _dp, _dp]),
+    "pioran_celerite_logl_vjp": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_int] + [_dp] * 17),
+    "pioran_approx_features_logl_grad_reverse": (C.c_int, [C.c_void_p, C.c_int, C.POINTER(ApproxSpec), C.c_int, C.c_int, _dp, _dp, _dp]),
+    "pioran_ctx_set_vjp_workspace": (C.c_int, [C.c_void_p, C.c_longlong]),
     "pioran_ctx_set_auto_scan": (C.c_int, [C.c_void_p, C.c_int]),
     "pioran_ctx_set_sweep_kernel": (C.c_int, [C.c_void_p, C.c_int]),
     "pioran_ctx_set_scan_chunks": (C.c_int, [C.c_void_p, C.c_int]),

@@ -243,6 +243,79 @@ def carma_celerite_coefs(p, rα, β, norm=1.0, is_integrated_power=True):
     return a * scale, b * scale, c, d
 
 
+def carma_celerite_coefs_jacobian(p, q, qa, qb, variance):
+    """carma_celerite_coefs ∘ (quad2roots, roots2coeffs) for one Θ row of BatchedCARMALikelihood (is_integrated_power) and its
+    Jacobian, in forward mode on complex numbers along the p + q + 1 unit directions of (qa…, qb…, variance).
+    Returns ((a, b, c, d) [J] each, (∂a, ∂b, ∂c, ∂d) [J × (p + q + 1)] each)."""
+    qa, qb = np.asarray(qa, dtype=np.float64), np.asarray(qb, dtype=np.float64)
+    P = p + q + 1
+    eye = np.eye(P)
+
+    def roots(quad, off):   # quad2roots with tangents [n × P]
+        n = quad.shape[0]
+        r, dr = np.zeros(n, dtype=np.complex128), np.zeros((n, P), dtype=np.complex128)
+        dq = eye[off:off + n]
+        if n % 2 == 1:
+            r[-1], dr[-1] = -quad[-1], -dq[-1]
+        for k in range(0, n - n % 2, 2):
+            lin, const, dlin, dconst = quad[k + 1], quad[k], dq[k + 1], dq[k]
+            disc, ddisc = lin * lin - 4.0 * const, 2.0 * lin * dlin - 4.0 * dconst
+            if disc < 0:
+                sq = np.sqrt(-disc)
+                r[k], dr[k] = (-lin + 1j * sq) / 2.0, (-dlin - 1j * ddisc / (2.0 * sq)) / 2.0
+                r[k + 1], dr[k + 1] = np.conj(r[k]), np.conj(dr[k])
+            else:
+                sq = np.sqrt(disc)
+                dsq = ddisc / (2.0 * sq)
+                r[k], dr[k] = (-lin + sq) / 2.0, (-dlin + dsq) / 2.0
+                r[k + 1], dr[k + 1] = (-lin - sq) / 2.0, (-dlin - dsq) / 2.0
+        return r, dr
+
+    rα, drα = roots(qa, 0)
+    if q > 0:
+        rβ, drβ = roots(qb, p)
+        co, dco = np.ones(1, dtype=np.complex128), np.zeros((1, P), dtype=np.complex128)   # constant term first
+        for rj, drj in zip(rβ, drβ):
+            nco, ndco = np.zeros(co.shape[0] + 1, dtype=np.complex128), np.zeros((co.shape[0] + 1, P), dtype=np.complex128)
+            nco[1:], ndco[1:] = co, dco
+            nco[:-1] -= rj * co
+            ndco[:-1] -= rj * dco + co[:, None] * drj[None, :]
+            co, dco = nco, ndco
+        β, dβ = co.real, dco.real
+    else:
+        β, dβ = np.ones(1), np.zeros((1, P))
+    J = (p + 1) // 2
+    a, b, c, d = (np.empty(J) for _ in range(4))
+    da, db, dc, dd = (np.zeros((J, P)) for _ in range(4))
+    pw = np.arange(β.shape[0])
+    for k in range(J):
+        rk, drk = rα[2 * k], drα[2 * k]
+        # the residue of _carma_residue and its tangent
+        A = np.sum(β * rk ** pw)
+        dA = dβ.T @ (rk ** pw) + np.sum(β[1:] * pw[1:] * rk ** (pw[1:] - 1)) * drk
+        Bv = np.sum(β * (-rk) ** pw)
+        dB = dβ.T @ ((-rk) ** pw) - np.sum(β[1:] * pw[1:] * (-rk) ** (pw[1:] - 1)) * drk
+        den, dden = -2.0 * rk.real + 0j, -2.0 * drk.real + 0j
+        for rj, drj in zip(rα, drα):
+            if rj != rk:
+                f = (rj - rk) * (np.conj(rj) + rk)
+                df = (drj - drk) * (np.conj(rj) + rk) + (rj - rk) * (np.conj(drj) + drk)
+                den, dden = den * f, dden * f + den * df
+        num, dnum = A * Bv, dA * Bv + A * dB
+        frac, dfrac = 2.0 * num / den, 2.0 * (dnum * den - num * dden) / den ** 2
+        if k != J - 1 or p % 2 == 0:
+            a[k], b[k], c[k], d[k] = 2.0 * frac.real, 2.0 * frac.imag, -rk.real, -rk.imag
+            da[k], db[k], dc[k], dd[k] = 2.0 * dfrac.real, 2.0 * dfrac.imag, -drk.real, -drk.imag
+        else:
+            a[k], b[k], c[k], d[k] = frac.real, 0.0, -rk.real, 0.0
+            da[k], dc[k] = dfrac.real, -drk.real
+    sa, dsa = np.sum(a), np.sum(da, axis=0)
+    dvar = eye[p + q]
+    scale, dscale = variance / sa, dvar / sa - variance * dsa / sa ** 2
+    return ((a * scale, b * scale, c, d),
+            (da * scale + a[:, None] * dscale[None, :], db * scale + b[:, None] * dscale[None, :], dc, dd))
+
+
 def celerite_repr(cov):
     """celerite_repr(cov::CARMA) (src/CARMA.jl:55-70) → SumOfCelerite."""
     return SumOfCelerite(*celerite_coefs(cov))
@@ -482,11 +555,18 @@ class BatchedLikelihood:
 
     def __init__(self, t, y, σ2, psd_model="SingleBendingPowerLaw", n_components=20, basis_function="SHO",
                  f_min=None, f_max=None, S_low=20.0, S_high=20.0, is_integrated_power=True, ctx=None, log_shift=False,
-                 n_features=0):
+                 n_features=0, gradient="forward"):
         # n_features: Θ rows end with (S₀, f₀, Q) per QPO feature added to the continuum (docs/src/adding_features.md)
         self.n_features = int(n_features)
         if self.n_features and log_shift:
             raise ValueError("PSD features and the log-shift transform cannot be combined in one fused call")
+        # gradient: "forward" (one K5g direction per Θ column) or "reverse" (one K5r sweep); only the gradient with features has
+        # both — without them c and d are fixed by the spectral grid and the fused approx-path gradient serves every column
+        if gradient not in ("forward", "reverse"):
+            raise ValueError(f"gradient must be 'forward' or 'reverse', not {gradient!r}")
+        if gradient == "reverse" and not self.n_features:
+            raise ValueError("gradient='reverse' needs n_features > 0 (the approx path without features has one gradient kernel)")
+        self.gradient_mode = gradient
         # log_shift: Θ rows carry a 7th column c and the data enter as yn = log(y − c), σ² = ν σ²/(y − c)²
         # (docs/src/ultranest.md:197-217); t, y, σ2 are then the untransformed flux and its measurement variance
         self.log_shift = bool(log_shift)
@@ -515,6 +595,8 @@ class BatchedLikelihood:
         (test/test_likelihood.jl:55, examples/turing_distributed/single_pl.jl), for a whole batch of chains at once."""
         theta = np.atleast_2d(np.asarray(theta, dtype=np.float64))
         if self.n_features:
+            if self.gradient_mode == "reverse":
+                return self.ctx.approx_features_logl_grad_reverse(self.series, self.spec, self.n_features, theta)
             return self.ctx.approx_features_logl_grad(self.series, self.spec, self.n_features, theta)
         if self.log_shift:
             return self.ctx.approx_logl_logshift_grad(self.series, self.spec, theta)
@@ -581,6 +663,46 @@ class BatchedCARMALikelihood:
             out[sel] = self.ctx.celerite_logl(self.series, a[sel], b[sel], c[sel], d[sel], mu=theta[sel, k + 2], nu=theta[sel, k + 1],
                                               y_batch=yb, s2_batch=sb)
         return out
+
+    def value_and_gradient(self, theta):
+        """(logL [B], ∂logL/∂Θ [B × n_par]) in the column order of Θ.  The coefficients' Jacobian with respect to (qa, qb, variance)
+        is formed on the host (carma_celerite_coefs_jacobian), the gradient with respect to the coefficients, ν, μ and, with the
+        log shift, the data row comes from one reverse-mode call (K5r) for the batch, and the chain rule joins them.  Rows outside
+        the root bounds get logL = −Inf and a zero gradient."""
+        theta = np.atleast_2d(np.asarray(theta, dtype=np.float64))
+        if theta.shape[1] != self.n_par:
+            raise ValueError(f"theta must have {self.n_par} columns")
+        B, k = theta.shape[0], self.p + self.q
+        out, grad = np.full(B, -np.inf), np.zeros((B, self.n_par))
+        rows = []
+        for i in range(B):
+            rα = quad2roots(theta[i, :self.p])
+            rβ = quad2roots(theta[i, self.p:k])
+            if self._roots_ok(rα) and (self.q == 0 or self._roots_ok(rβ)):
+                rows.append((i, carma_celerite_coefs_jacobian(self.p, self.q, theta[i, :self.p], theta[i, self.p:k], theta[i, k])))
+        if not rows:
+            return out, grad
+        sel = np.array([i for i, _ in rows])
+        a, b, c, d = (np.array([co[0][j] for _, co in rows]) for j in range(4))
+        jac = [np.array([co[1][j] for _, co in rows]) for j in range(4)]   # [n × J × (k + 1)] each
+        yb = sb = None
+        if self.log_shift:
+            shift = self.y[None, :] - theta[sel, k + 3:k + 4]
+            with np.errstate(invalid="ignore", divide="ignore"):
+                yb, sb = np.log(shift), self.σ2[None, :] / shift ** 2
+        L, g = self.ctx.celerite_logl_vjp(self.series, a, b, c, d, mu=theta[sel, k + 2], nu=theta[sel, k + 1], y_batch=yb,
+                                          s2_batch=sb, data_grad=self.log_shift)
+        out[sel] = L
+        grad[sel, :k + 1] = sum(np.einsum("nj,njp->np", g[x], jac[j]) for j, x in enumerate("abcd"))
+        grad[sel, k + 1], grad[sel, k + 2] = g["nu"], g["mu"]
+        if self.log_shift:
+            # yn = log(y − c): dyn/dc = −1/(y − c);  s2 = σ²/(y − c)²: ds2/dc = 2σ²/(y − c)³ (ν is applied inside the kernel)
+            with np.errstate(invalid="ignore", divide="ignore"):
+                grad[sel, k + 3] = np.sum(-g["y"] / shift + g["s2"] * 2.0 * self.σ2[None, :] / shift ** 3, axis=1)
+        return out, grad
+
+    def gradient(self, theta):
+        return self.value_and_gradient(theta)[1]
 
     def close(self):
         self.series.free()

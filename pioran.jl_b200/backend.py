@@ -304,6 +304,47 @@ class Context:
                                                         _p(grad)))
         return out, grad
 
+    # -- K5r: reverse-mode gradient of the explicit-coefficient likelihood
+    def celerite_logl_vjp(self, series, a, b, c, d, *, mu=None, nu=None, y_batch=None, s2_batch=None, data_grad=False):
+        """logL and its gradient with respect to every input of celerite_logl, from one backward sweep per coefficient set.
+        a, b, c, d [B × Jt].  Returns (logL [B], {"a", "b", "c", "d" [B × Jt], "mu", "nu" [B]}); with data_grad also "y" and
+        "s2" [B × N], the gradient with respect to the data row as it enters (ỹ = y − μ, σ̃² = ν·s2)."""
+        a, b, c, d = (np.atleast_2d(_f64(x)) for x in (a, b, c, d))
+        B, Jt = a.shape
+        for x in (b, c, d):
+            if x.shape != (B, Jt):
+                raise ValueError("a, b, c, d must have the same shape")
+        N = series.N
+        mu = _f64(mu, (B,)) if mu is not None else None
+        nu = _f64(nu, (B,)) if nu is not None else None
+        yb = _f64(y_batch, (B, N)) if y_batch is not None else None
+        sb = _f64(s2_batch, (B, N)) if s2_batch is not None else None
+        out = np.empty(B)
+        g = {k: np.empty((B, Jt)) for k in ("a", "b", "c", "d")}
+        g["mu"], g["nu"] = np.empty(B), np.empty(B)
+        if data_grad:
+            g["y"], g["s2"] = np.empty((B, N)), np.empty((B, N))
+        check(self.lib.pioran_celerite_logl_vjp(self.h, series.id, B, Jt, _p(a), _p(b), _p(c), _p(d), _p(mu), _p(nu), _p(yb), _p(sb),
+                                                _p(out), *[_p(g[k]) for k in ("a", "b", "c", "d", "mu", "nu")],
+                                                _p(g.get("y")), _p(g.get("s2"))))
+        return out, g
+
+    def approx_features_logl_grad_reverse(self, series, spec, n_features, theta):
+        """approx_features_logl_grad computed in reverse mode (one K5r sweep instead of one forward direction per column)."""
+        theta = np.atleast_2d(_f64(theta))
+        ncol = N_PSD_PAR[spec.psd_model] + 3 + 3 * int(n_features)
+        if theta.shape[1] != ncol:
+            raise ValueError(f"theta must have {ncol} columns")
+        B = theta.shape[0]
+        out, grad = np.empty(B), np.empty((B, ncol))
+        check(self.lib.pioran_approx_features_logl_grad_reverse(self.h, series.id, C.byref(spec), int(n_features), B, _p(theta),
+                                                                _p(out), _p(grad)))
+        return out, grad
+
+    def set_vjp_workspace(self, nbytes):
+        """Cap in bytes of the reverse-mode workspace of one θ-chunk (0 = 1 GiB, the default)."""
+        check(self.lib.pioran_ctx_set_vjp_workspace(self.h, int(nbytes)))
+
     def approx_logl_grad_dev(self, series, spec, B, theta_ptr, logl_ptr, grad_ptr):
         """Device-resident variant: raw device pointers (ints); logl_ptr may be 0."""
         check(self.lib.pioran_approx_logl_grad_dev(self.h, series.id, C.byref(spec), int(B), C.c_void_p(theta_ptr),

@@ -33,6 +33,7 @@
 #include "scan_wide.cuh"
 #include "scan_blocked.cuh"
 #include "jvp.cuh"
+#include "vjp.cuh"
 
 using namespace pioran;
 
@@ -64,7 +65,7 @@ static int guard_fail() {
     } while (0)
 
 extern "C" const char* pioran_last_error(void) { return g_err.c_str(); }
-extern "C" int pioran_version(void) { return 301; }   // 0.3.1: pioran_ctx_last_kernel_name
+extern "C" int pioran_version(void) { return 302; }   // 0.3.2: pioran_celerite_logl_vjp, pioran_approx_features_logl_grad_reverse
 
 // ------------------------------------------------------------------------------------------------ context
 namespace {
@@ -104,7 +105,7 @@ using PlanKey = std::tuple<int, int, int, int, double, double, double, double>;
 enum KernelFamily : int {
     KF_NONE = 0, KF_BLOCKED, KF_BLOCKED_WIDE, KF_SHARED, KF_SHARED_PAIR, KF_GENERIC, KF_WIDE_REG, KF_WIDE_REG_STORE, KF_WIDE_REG_SIM,
     KF_WIDE, KF_BLOCKED_GRAD, KF_GRAD, KF_GRAD_PIPE, KF_WIDE_GRAD, KF_JVP, KF_PREDICT, KF_GENERIC_SIM, KF_SCAN_FINISH,
-    KF_SCAN_PARTIAL, KF_DENSE_FINISH
+    KF_SCAN_PARTIAL, KF_DENSE_FINISH, KF_VJP
 };
 struct KernelTag { int family = KF_NONE; int p[4] = {0, 0, 0, 0}; };
 
@@ -121,6 +122,7 @@ struct pioran_ctx {
     std::vector<Series*> series;
     std::map<PlanKey, ApproxPlan*> plans;  // device pointers
     DevBuf theta, amp, suma, out, work, coef, rows, misc, post, gradws, gwork, stab;   // stab: per-θ block table of the K3 fold
+    DevBuf vjpws;   // K5r: per-step values and T checkpoints of one θ-chunk
     // device time of the most recent main-kernel launch (K2/K3/K4), for bench.py's roofline line
     cudaEvent_t ev_beg = nullptr, ev_end = nullptr;
     bool ev_valid = false;
@@ -132,6 +134,7 @@ struct pioran_ctx {
     std::vector<int64_t> gwork_key;   // same for the gradient path's work items
     int gwork_items = 0, gwork_tpi = 0;
     int scan_chunks = 0;   // K3: chunks per parameter vector (0 = automatic)
+    size_t vjp_ws_bytes = 0;   // K5r: workspace cap per θ-chunk (0 = 1 GiB; pioran_ctx_set_vjp_workspace)
     bool auto_scan = true; // route few-evaluation calls on long series to K3 (pioran_ctx_set_auto_scan)
     int sweep_kernel = PIORAN_SWEEP_AUTO;   // pioran_ctx_set_sweep_kernel
     // pioran_ctx_create_multi: a group context owns one child context per device and no CUDA state of its own; the batched
@@ -305,7 +308,7 @@ extern "C" int pioran_ctx_destroy(pioran_ctx* c) try {
     for (Series* s : c->series) free_series(s);
     for (auto& kv : c->plans) cudaFree(kv.second);
     c->theta.release(); c->amp.release(); c->suma.release(); c->out.release(); c->work.release();
-    c->coef.release(); c->rows.release(); c->misc.release(); c->post.release(); c->gradws.release(); c->gwork.release(); c->stab.release();
+    c->coef.release(); c->rows.release(); c->misc.release(); c->post.release(); c->gradws.release(); c->gwork.release(); c->stab.release(); c->vjpws.release();
     if (c->ev_beg) cudaEventDestroy(c->ev_beg);
     if (c->ev_end) cudaEventDestroy(c->ev_end);
     if (c->ev_fact) cudaEventDestroy(c->ev_fact);
@@ -387,6 +390,7 @@ extern "C" int pioran_ctx_last_kernel_name(pioran_ctx* c, char* buf, int len) tr
         case KF_GRAD_PIPE: snprintf(name, sizeof name, "grad_pipe<%d,%d>", p[0], p[1]); break;
         case KF_WIDE_GRAD: snprintf(name, sizeof name, "wide_grad<%d>", p[0]); break;
         case KF_JVP: snprintf(name, sizeof name, "jvp<%d>", p[0]); break;
+        case KF_VJP: snprintf(name, sizeof name, "vjp<%d>", p[0]); break;
         case KF_PREDICT: snprintf(name, sizeof name, "predict<%d>", p[0]); break;
         case KF_GENERIC_SIM: snprintf(name, sizeof name, "generic_sim<%d,%d>", p[0], p[1]); break;
         case KF_SCAN_FINISH: snprintf(name, sizeof name, "scan_finish"); break;
@@ -2160,6 +2164,198 @@ extern "C" int pioran_approx_features_logl_grad(pioran_ctx* c, int series_id, co
     if (logl_out) CUDA_TRY(cudaMemcpyAsync(logl_out, gl, sizeof(double) * (size_t)B, cudaMemcpyDeviceToHost, c->stream));
     CUDA_TRY(cudaMemcpyAsync(grad_out, gg, sizeof(double) * np, cudaMemcpyDeviceToHost, c->stream));
     CUDA_TRY(cudaStreamSynchronize(c->stream));
+    return PIORAN_OK;
+} catch (...) { return guard_fail(); }
+
+// ------------------------------------------------------------------------------------------------ K5r: VJP on explicit coefficients
+// Shared by pioran_celerite_logl_vjp and pioran_approx_features_logl_grad_reverse.  `base` holds the device pointers of the
+// inputs and outputs for all B sets (gy, gs2 ignored); the batch runs in θ-chunks whose workspace stays under the context's cap
+// (1 GiB unless pioran_ctx_set_vjp_workspace says otherwise).  gy_host / gs2_host [B × N] (or NULL) receive the data gradients
+// chunk by chunk.  The context is locked by the caller; R <= VJP_MAX_RANK.
+static int vjp_dev_locked(pioran_ctx* c, Series* s, int B, int Jt, int R, const std::vector<int>& term_row, const VjpArgs& base,
+                          double* gy_host, double* gs2_host) {
+    int rc;
+    const int64_t N = s->N;
+    const int TS = std::max(1, (R + 15) / 16);
+    if (TS > 6) return fail(PIORAN_EUNSUPPORTED, "the VJP is built for ranks <= %d (rank %d)", VJP_MAX_RANK, R);
+    // K ≈ √N steps per checkpoint segment minimises the ⌈N/K⌉ + K tiles kept per set
+    int64_t K = (int64_t)std::ceil(std::sqrt((double)N));
+    K = (K + WIDE_CH - 1) / WIDE_CH * WIDE_CH;
+    const size_t per = sizeof(double) * vjp_ws_doubles(TS, N, (int)K);
+    const size_t cap = c->vjp_ws_bytes ? c->vjp_ws_bytes : ((size_t)1 << 30);
+    const int chunk = (int)std::max<size_t>(1, std::min<size_t>((size_t)B, cap / per));
+    if ((rc = c->vjpws.ensure(per * (size_t)chunk))) return rc;
+    if ((rc = c->rows.ensure(sizeof(int) * (Jt + 1)))) return rc;
+    CUDA_TRY(cudaMemcpyAsync(c->rows.p, term_row.data(), sizeof(int) * Jt, cudaMemcpyHostToDevice, c->stream));
+    const size_t nd = (size_t)chunk * N;
+    if ((gy_host || gs2_host) && (rc = c->post.ensure(sizeof(double) * 2 * nd))) return rc;
+    for (int off = 0; off < B; off += chunk) {
+        const int nb = std::min(chunk, B - off);
+        const size_t o = (size_t)off * Jt, on = (size_t)off * N;
+        VjpArgs va = base;
+        va.t = s->t; va.y = s->y; va.s2 = s->s2; va.N = N;
+        va.term_row = c->rows.as<int>(); va.Jt = Jt; va.K = (int)K; va.ws = c->vjpws.as<double>();
+        va.a = base.a + o; va.b = base.b + o; va.c = base.c + o; va.d = base.d + o;
+        va.mu = base.mu ? base.mu + off : nullptr; va.nu = base.nu ? base.nu + off : nullptr;
+        va.y_batch = base.y_batch ? base.y_batch + on : nullptr; va.s2_batch = base.s2_batch ? base.s2_batch + on : nullptr;
+        va.logl = base.logl ? base.logl + off : nullptr;
+        va.ga = base.ga ? base.ga + o : nullptr; va.gb = base.gb ? base.gb + o : nullptr;
+        va.gc = base.gc ? base.gc + o : nullptr; va.gd = base.gd ? base.gd + o : nullptr;
+        va.gmu = base.gmu ? base.gmu + off : nullptr; va.gnu = base.gnu ? base.gnu + off : nullptr;
+        va.gy = gy_host ? c->post.as<double>() : nullptr;
+        va.gs2 = gs2_host ? c->post.as<double>() + nd : nullptr;
+        cudaEventRecord(c->ev_beg, c->stream);
+        switch (TS) {
+            case 1: celerite_vjp_kernel<1><<<nb, WIDE_THREADS, 0, c->stream>>>(va); break;
+            case 2: celerite_vjp_kernel<2><<<nb, WIDE_THREADS, 0, c->stream>>>(va); break;
+            case 3: celerite_vjp_kernel<3><<<nb, WIDE_THREADS, 0, c->stream>>>(va); break;
+            case 4: celerite_vjp_kernel<4><<<nb, WIDE_THREADS, 0, c->stream>>>(va); break;
+            case 5: celerite_vjp_kernel<5><<<nb, WIDE_THREADS, 0, c->stream>>>(va); break;
+            default: celerite_vjp_kernel<6><<<nb, WIDE_THREADS, 0, c->stream>>>(va); break;
+        }
+        cudaEventRecord(c->ev_end, c->stream);
+        note_kernel(c, KF_VJP, TS);
+        c->launches++;
+        CUDA_TRY(cudaGetLastError());
+        if (gy_host) CUDA_TRY(cudaMemcpyAsync(gy_host + on, va.gy, sizeof(double) * nb * N, cudaMemcpyDeviceToHost, c->stream));
+        if (gs2_host) CUDA_TRY(cudaMemcpyAsync(gs2_host + on, va.gs2, sizeof(double) * nb * N, cudaMemcpyDeviceToHost, c->stream));
+    }
+    // term_row is the caller's host vector: the copy must have left it before the caller may drop it
+    CUDA_TRY(cudaStreamSynchronize(c->stream));
+    return 0;
+}
+
+extern "C" int pioran_celerite_logl_vjp(pioran_ctx* c, int series_id, int B, int Jt, const double* a, const double* b,
+                                        const double* cc, const double* d, const double* mu, const double* nu,
+                                        const double* y_batch, const double* s2_batch, double* logl_out, double* ga, double* gb,
+                                        double* gc, double* gd, double* gmu, double* gnu, double* gy, double* gs2) try {
+    if (!c || !a || !b || !cc || !d) return fail(PIORAN_EINVAL, "NULL argument");
+    if (!ga && !gb && !gc && !gd && !gmu && !gnu && !gy && !gs2) return fail(PIORAN_EINVAL, "no gradient output given");
+    if (B < 1 || Jt < 1) return fail(PIORAN_EINVAL, "B and Jt must be >= 1");
+    if (is_group(c)) {
+        std::vector<int> cid(c->children.size());
+        int64_t Ng = 0;
+        { std::lock_guard<std::mutex> lk(c->mu); for (size_t k = 0; k < cid.size(); k++) { const int rc = group_series_id(c, series_id, k, &cid[k]); if (rc) return rc; } }
+        if (y_batch || s2_batch || gy || gs2) { const int rc = pioran_series_length(c->children[0], cid[0], &Ng); if (rc) return rc; }
+        return group_split(c, B, [&](int k, int beg, int nb) -> int {
+            const size_t o = (size_t)beg * Jt, on = (size_t)beg * Ng;
+            return pioran_celerite_logl_vjp(c->children[k], cid[k], nb, Jt, a + o, b + o, cc + o, d + o, mu ? mu + beg : nullptr,
+                                            nu ? nu + beg : nullptr, y_batch ? y_batch + on : nullptr, s2_batch ? s2_batch + on : nullptr,
+                                            logl_out ? logl_out + beg : nullptr, ga ? ga + o : nullptr, gb ? gb + o : nullptr,
+                                            gc ? gc + o : nullptr, gd ? gd + o : nullptr, gmu ? gmu + beg : nullptr,
+                                            gnu ? gnu + beg : nullptr, gy ? gy + on : nullptr, gs2 ? gs2 + on : nullptr);
+        });
+    }
+    PIORAN_COMPUTE_LOCK(c);
+    CUDA_TRY(cudaSetDevice(c->device));
+    Series* s = get_series(c, series_id);
+    if (!s) return fail(PIORAN_EINVAL, "unknown series id %d", series_id);
+    std::vector<int> term_row;
+    const int R = make_term_rows(B, Jt, b, d, term_row);
+    if (R > VJP_MAX_RANK) return fail(PIORAN_EUNSUPPORTED, "the VJP is built for ranks <= %d (rank %d, Jt = %d)", VJP_MAX_RANK, R, Jt);
+    int rc;
+    GenericInputs gi;
+    if ((rc = upload_generic(c, B, Jt, s->N, a, b, cc, d, mu, nu, y_batch, s2_batch, gi))) return rc;
+    // logL [B], ā … d̄ [B × Jt] each, μ̄, ν̄ [B]
+    const size_t n = (size_t)B * Jt;
+    if ((rc = c->out.ensure(sizeof(double) * (3 * (size_t)B + 4 * n)))) return rc;
+    double* ob = c->out.as<double>();
+    VjpArgs base{};
+    base.a = gi.a; base.b = gi.b; base.c = gi.c; base.d = gi.d; base.mu = gi.mu; base.nu = gi.nu;
+    base.y_batch = gi.yb; base.s2_batch = gi.sb;
+    base.logl = ob; base.ga = ob + B; base.gb = ob + B + n; base.gc = ob + B + 2 * n; base.gd = ob + B + 3 * n;
+    base.gmu = ob + B + 4 * n; base.gnu = ob + 2 * B + 4 * n;
+    if ((rc = vjp_dev_locked(c, s, B, Jt, R, term_row, base, gy, gs2))) return rc;
+    double* hdst[7] = {logl_out, ga, gb, gc, gd, gmu, gnu};
+    const double* dsrc[7] = {base.logl, base.ga, base.gb, base.gc, base.gd, base.gmu, base.gnu};
+    for (int q = 0; q < 7; q++)
+        if (hdst[q]) CUDA_TRY(cudaMemcpyAsync(hdst[q], dsrc[q], sizeof(double) * (q >= 1 && q <= 4 ? n : (size_t)B), cudaMemcpyDeviceToHost, c->stream));
+    CUDA_TRY(cudaStreamSynchronize(c->stream));
+    return PIORAN_OK;
+} catch (...) { return guard_fail(); }
+
+// Gradient with PSD features in reverse mode: the same coefficients and tangents as pioran_approx_features_logl_grad
+// (approx_features_grad_kernel), one K5r sweep for ∂logL with respect to the coefficients, and their contraction with the tangents
+// along every θ column (vjp_contract_kernel).  Nothing returns to the host in between.
+extern "C" int pioran_approx_features_logl_grad_reverse(pioran_ctx* c, int series_id, const pioran_approx_spec* spec, int n_features,
+                                                        int B, const double* theta, double* logl_out, double* grad_out) try {
+    if (!c || !spec || !theta || !grad_out) return fail(PIORAN_EINVAL, "NULL argument");
+    if (B < 1) return fail(PIORAN_EINVAL, "B must be >= 1");
+    const int npar = n_psd_par_of(spec->psd_model);
+    if (npar < 0) return fail(PIORAN_EINVAL, "unknown psd_model %d", spec->psd_model);
+    if (n_features < 1) return fail(PIORAN_EINVAL, "n_features must be >= 1 (got %d)", n_features);
+    if (n_features > MAXFEAT) return fail(PIORAN_EUNSUPPORTED, "at most %d features (got %d)", MAXFEAT, n_features);
+    const int ts = npar + 3 + 3 * n_features;
+    if ((long long)B * ts > 0x7fffffffLL) return fail(PIORAN_EINVAL, "B too large");
+    if (is_group(c)) {
+        std::vector<int> cid(c->children.size());
+        { std::lock_guard<std::mutex> lk(c->mu); for (size_t k = 0; k < cid.size(); k++) { const int rc = group_series_id(c, series_id, k, &cid[k]); if (rc) return rc; } }
+        return group_split(c, B, [&](int k, int beg, int nb) -> int {
+            return pioran_approx_features_logl_grad_reverse(c->children[k], cid[k], spec, n_features, nb, theta + (size_t)beg * ts,
+                                                            logl_out ? logl_out + beg : nullptr, grad_out + (size_t)beg * ts);
+        });
+    }
+    PIORAN_COMPUTE_LOCK(c);
+    CUDA_TRY(cudaSetDevice(c->device));
+    int rc;
+    if ((rc = check_spec(*spec))) return rc;
+    Series* s = get_series(c, series_id);
+    if (!s) return fail(PIORAN_EINVAL, "unknown series id %d", series_id);
+    const int J = spec->n_components, nf = n_features;
+    const int Jc = spec->basis == PIORAN_BASIS_SHO ? J : 2 * J, Jt = Jc + nf;
+    const int Rc = rank_of(spec->basis, J), R = Rc + 2 * nf;
+    if (R > VJP_MAX_RANK) return fail(PIORAN_EUNSUPPORTED, "gradients with features are built for ranks <= %d (rank %d)", VJP_MAX_RANK, R);
+    ApproxPlan* plan;
+    if ((rc = get_plan(c, *spec, &plan))) return rc;
+    // term rows as in pioran_approx_features_logl_grad
+    std::vector<int> term_row(Jt + 1, 0);
+    for (int j = 0; j < J; j++) {
+        term_row[j] = 2 * j;
+        if (spec->basis != PIORAN_BASIS_SHO) term_row[J + j] = -(2 * J + j + 1);
+    }
+    for (int f = 0; f < nf; f++) term_row[Jc + f] = Rc + 2 * f;
+    const int P = ts;
+    const size_t n = (size_t)B * Jt, nt = (size_t)B * P * Jt, np = (size_t)B * P;
+    if ((rc = c->theta.ensure(sizeof(double) * (size_t)B * ts))) return rc;
+    if ((rc = c->coef.ensure(sizeof(double) * (4 * n + 2 * (size_t)B)))) return rc;
+    if ((rc = c->gradws.ensure(sizeof(double) * (4 * nt + 2 * np)))) return rc;
+    // logL [B], ā … d̄ [B × Jt] each, μ̄, ν̄ [B], ∂logL/∂θ [B × P]
+    if ((rc = c->out.ensure(sizeof(double) * (3 * (size_t)B + 4 * n + np)))) return rc;
+    CUDA_TRY(cudaMemcpyAsync(c->theta.p, theta, sizeof(double) * (size_t)B * ts, cudaMemcpyHostToDevice, c->stream));
+    double* co = c->coef.as<double>();
+    double* tg = c->gradws.as<double>();
+    double* ob = c->out.as<double>();
+    approx_features_grad_kernel<<<(unsigned)((np + 127) / 128), 128, 0, c->stream>>>(
+        plan, B, c->theta.as<double>(), ts, nf, npar + 3, co, co + n, co + 2 * n, co + 3 * n, co + 4 * n, co + 4 * n + B,
+        tg, tg + nt, tg + 2 * nt, tg + 3 * nt, tg + 4 * nt, tg + 4 * nt + np);
+    c->launches++;
+    CUDA_TRY(cudaGetLastError());
+    VjpArgs base{};
+    base.a = co; base.b = co + n; base.c = co + 2 * n; base.d = co + 3 * n; base.mu = co + 4 * n; base.nu = co + 4 * n + B;
+    base.logl = ob; base.ga = ob + B; base.gb = ob + B + n; base.gc = ob + B + 2 * n; base.gd = ob + B + 3 * n;
+    base.gmu = ob + B + 4 * n; base.gnu = ob + 2 * B + 4 * n;
+    if ((rc = vjp_dev_locked(c, s, B, Jt, R, term_row, base, nullptr, nullptr))) return rc;
+    double* gg = ob + 3 * (size_t)B + 4 * n;
+    vjp_contract_kernel<<<(unsigned)((np + 127) / 128), 128, 0, c->stream>>>(
+        B, P, Jt, base.ga, base.gb, base.gc, base.gd, base.gmu, base.gnu, tg, tg + nt, tg + 2 * nt, tg + 3 * nt, tg + 4 * nt,
+        tg + 4 * nt + np, gg);
+    c->launches++;
+    CUDA_TRY(cudaGetLastError());
+    if (logl_out) CUDA_TRY(cudaMemcpyAsync(logl_out, ob, sizeof(double) * (size_t)B, cudaMemcpyDeviceToHost, c->stream));
+    CUDA_TRY(cudaMemcpyAsync(grad_out, gg, sizeof(double) * np, cudaMemcpyDeviceToHost, c->stream));
+    CUDA_TRY(cudaStreamSynchronize(c->stream));
+    return PIORAN_OK;
+} catch (...) { return guard_fail(); }
+
+extern "C" int pioran_ctx_set_vjp_workspace(pioran_ctx* c, long long bytes) try {
+    if (is_group(c)) {
+        for (pioran_ctx* ch : c->children) { const int rc = pioran_ctx_set_vjp_workspace(ch, bytes); if (rc) return rc; }
+        return PIORAN_OK;
+    }
+    if (!c) return fail(PIORAN_EINVAL, "ctx is NULL");
+    if (bytes < 0) return fail(PIORAN_EINVAL, "bytes must be >= 0 (0 = 1 GiB)");
+    std::lock_guard<std::mutex> lk(c->mu);
+    c->vjp_ws_bytes = (size_t)bytes;
     return PIORAN_OK;
 } catch (...) { return guard_fail(); }
 
