@@ -337,6 +337,17 @@ int pioran_celerite_predict(pioran_ctx *ctx, int series_id, int B, int Jt,
 int pioran_celerite_simulate(pioran_ctx *ctx, int series_id, int B, int Jt,
                              const double *a, const double *b, const double *c, const double *d,
                              const double *nu, const double *q, double *y_out);
+/* Posterior predictive variance (K6): for each of the B coefficient sets the variance of the latent f at the M ascending
+ * points tau,  var_out[i][m] = k_i(0) − k_i(τ_m, t)ᵀ (K_i(t, t) + diag(nu_i σ²))⁻¹ k_i(τ_m, t)  — the diagonal of
+ * predict_cov (src/direct_solver.jl:28-119) behind var / std of a PosteriorGP, without measurement noise and independent of
+ * mu.  O((N + M)·R²) per set from the factor of pioran_celerite_predict; ranks up to 128 (PIORAN_EUNSUPPORTED above).
+ * mean_out [B × M] (or NULL) is what pioran_celerite_predict returns for the same arguments, bit for bit.  A set whose
+ * factor has a pivot D_n <= 0 gets NaN in every entry of its var_out row.  Arguments are checked as in
+ * pioran_celerite_predict; on a device group the call runs on the first device. */
+int pioran_celerite_predict_var(pioran_ctx *ctx, int series_id, int B, int Jt,
+                                const double *a, const double *b, const double *c, const double *d,
+                                const double *mu, const double *nu, int64_t M, const double *tau,
+                                double *mean_out, double *var_out);
 
 #ifdef __cplusplus
 }

@@ -282,6 +282,28 @@ function pred_b200(a, b, c, d, τ, t, y, σ2)
     return μ
 end
 
+"""
+    predict_var_b200(a, b, c, d, τ, t, y, σ2) -> (μ, v)
+
+Posterior mean (what `pred_b200` returns, bit for bit) and variance of the latent f at ascending τ: the diagonal of
+`predict_cov` (src/direct_solver.jl:28-119) in O((N + M)·R²), without measurement noise.  Ranks up to 128.
+"""
+function predict_var_b200(a, b, c, d, τ, t, y, σ2)
+    s = b200_upload(collect(Float64, t), collect(Float64, y), collect(Float64, σ2))
+    μ = Vector{Float64}(undef, length(τ))
+    v = Vector{Float64}(undef, length(τ))
+    try
+        _b200_check(ccall((:pioran_celerite_predict_var, libpioran_b200), Cint,
+            (Ptr{Cvoid}, Cint, Cint, Cint, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64},
+             Int64, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}),
+            b200_context().h, s.id, 1, length(a), Vector{Float64}(a), Vector{Float64}(b), Vector{Float64}(c), Vector{Float64}(d),
+            C_NULL, C_NULL, length(τ), collect(Float64, τ), μ, v))
+    finally
+        b200_free(s)
+    end
+    return μ, v
+end
+
 "Drop-in for sim(rng, a, b, c, d, τ, σ2) (src/celerite_solver.jl:515-549): the draw q = randn(rng, N) is the reference's first line (:518)."
 function sim_b200(rng, a, b, c, d, τ, σ2)
     q = randn(rng, length(τ))

@@ -71,6 +71,8 @@ SYMBOLS = {
     "pioran_direct_logl": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_int, _dp, _dp, _dp, _dp, _dp, _dp, _dp, _ip]),
     "pioran_celerite_predict": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_int, _dp, _dp, _dp, _dp, _dp, _dp, C.c_int64, _dp, _dp]),
     "pioran_celerite_simulate": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_int, _dp, _dp, _dp, _dp, _dp, _dp, _dp]),
+    "pioran_celerite_predict_var": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_int, _dp, _dp, _dp, _dp, _dp, _dp, C.c_int64,
+                                              _dp, _dp, _dp]),
 }
 
 _lib = None

@@ -487,7 +487,7 @@ def logpdf(fx, Y, *, ctx=None):
 # ----------------------------------------------------------------------------------------------- posterior, draws
 class PosteriorGP:
     """posterior(f(t, σ²), y)  (src/scalable_GP.jl:44-54): holds the finite GP and the data; mean(fp, τ) runs the batched
-    `pred` kernel (src/celerite_solver.jl:376-483)."""
+    `pred` kernel (src/celerite_solver.jl:376-483), var / std / mean_and_var(fp, τ) the posterior-variance sweep K6."""
 
     def __init__(self, fx, y):
         if not isinstance(fx, FiniteScalableGP):
@@ -519,6 +519,49 @@ def mean(fp, τ=None, *, ctx=None):
     m = fx.f.mean
     mτ = m(τ) if callable(m) else np.full(τ.shape, float(m))
     return predict(fx.f.kernel, τ, fx.x, fp.y - fx.mean_vector(), fx.σ2, ctx=ctx) + mτ
+
+
+def predict_var(cov, τ, t, σ2, y=None, *, ctx=None):
+    """Posterior variance of the zero-mean GP's latent f at ascending τ: the diagonal of predict_cov
+    (src/direct_solver.jl:28-119) in O((N + M)·R²), without measurement noise.  With y, (mean, var)."""
+    ctx = ctx or get_context()
+    a, b, c, d = celerite_coefs(cov)
+    τ = np.asarray(τ, dtype=np.float64)
+    ser = ctx.upload_series(t, np.zeros_like(t) if y is None else y, σ2)
+    try:
+        out = ctx.celerite_predict_var(ser, a, b, c, d, τ, return_mean=y is not None)
+    finally:
+        ser.free()
+    return (out[0][0], out[1][0]) if y is not None else out[0]
+
+
+def mean_and_var(fp, τ=None, *, ctx=None):
+    """mean_and_var(fp[, τ])  (AbstractGPs): posterior mean and the variance of the latent f at τ (default: the data
+    times), from one factorisation.  The mean function shifts the mean only."""
+    if not isinstance(fp, PosteriorGP):
+        raise TypeError("mean_and_var expects posterior(f(t, σ²), y)")
+    fx = fp.f
+    τ = fx.x if τ is None else np.asarray(τ, dtype=np.float64)
+    m = fx.f.mean
+    mτ = m(τ) if callable(m) else np.full(τ.shape, float(m))
+    mu, v = predict_var(fx.f.kernel, τ, fx.x, fx.σ2, fp.y - fx.mean_vector(), ctx=ctx)
+    return mu + mτ, v
+
+
+def var(fp, τ=None, *, ctx=None):
+    """var(fp[, τ])  (AbstractGPs; diag of cov(fp, τ), src/scalable_GP.jl:44-155): the posterior variance of the latent
+    f at τ (default: the data times), measurement noise not included."""
+    if not isinstance(fp, PosteriorGP):
+        raise TypeError("var expects posterior(f(t, σ²), y)")
+    fx = fp.f
+    τ = fx.x if τ is None else np.asarray(τ, dtype=np.float64)
+    return predict_var(fx.f.kernel, τ, fx.x, fx.σ2, ctx=ctx)
+
+
+def std(fp, τ=None, *, ctx=None):
+    """std(fp[, τ]) = √max(var, 0): at a data point with a tiny σ² the exact variance is close to 0 and rounding can
+    make the computed one slightly negative; it is clamped to 0 rather than turned into NaN."""
+    return np.sqrt(np.maximum(var(fp, τ, ctx=ctx), 0.0))
 
 
 def simulate(cov, τ, σ2, q, *, ctx=None):

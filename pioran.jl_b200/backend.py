@@ -448,6 +448,21 @@ class Context:
                                                tau.shape[0], _p(tau), _p(out)))
         return out
 
+    def celerite_predict_var(self, series, a, b, c, d, tau, mu=None, nu=None, return_mean=True):
+        """Posterior predictive variance of the latent f at ascending τ (the diagonal of predict_cov,
+        src/direct_solver.jl:28-119), [B × M], by the O((N + M)·R²) sweep K6.  With return_mean, (mean, var), where mean is
+        celerite_predict's result bit for bit.  A set whose covariance is not positive definite gets a NaN row."""
+        a, b, c, d = (np.atleast_2d(_f64(x)) for x in (a, b, c, d))
+        B, Jt = a.shape
+        tau = _f64(tau)
+        mu = _f64(mu, (B,)) if mu is not None else None
+        nu = _f64(nu, (B,)) if nu is not None else None
+        var = np.empty((B, tau.shape[0]))
+        mean = np.empty((B, tau.shape[0])) if return_mean else None
+        check(self.lib.pioran_celerite_predict_var(self.h, series.id, B, Jt, _p(a), _p(b), _p(c), _p(d), _p(mu), _p(nu),
+                                                   tau.shape[0], _p(tau), _p(mean), _p(var)))
+        return (mean, var) if return_mean else var
+
     def celerite_simulate(self, series, a, b, c, d, q, nu=None):
         """Batched sim(rng,a,b,c,d,t,σ²) (src/celerite_solver.jl:515-549) with the normal draws q [B × N] supplied."""
         a, b, c, d = (np.atleast_2d(_f64(x)) for x in (a, b, c, d))

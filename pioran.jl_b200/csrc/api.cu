@@ -22,6 +22,7 @@
 #include "dense.cuh"
 #include "scan.cuh"
 #include "posterior.cuh"
+#include "postvar.cuh"
 #include "table.cuh"
 #include "grad.cuh"
 #include "grad_pipe.cuh"
@@ -65,7 +66,7 @@ static int guard_fail() {
     } while (0)
 
 extern "C" const char* pioran_last_error(void) { return g_err.c_str(); }
-extern "C" int pioran_version(void) { return 302; }   // 0.3.2: pioran_celerite_logl_vjp, pioran_approx_features_logl_grad_reverse
+extern "C" int pioran_version(void) { return 303; }   // 0.3.3: pioran_celerite_predict_var
 
 // ------------------------------------------------------------------------------------------------ context
 namespace {
@@ -105,7 +106,7 @@ using PlanKey = std::tuple<int, int, int, int, double, double, double, double>;
 enum KernelFamily : int {
     KF_NONE = 0, KF_BLOCKED, KF_BLOCKED_WIDE, KF_SHARED, KF_SHARED_PAIR, KF_GENERIC, KF_WIDE_REG, KF_WIDE_REG_STORE, KF_WIDE_REG_SIM,
     KF_WIDE, KF_BLOCKED_GRAD, KF_GRAD, KF_GRAD_PIPE, KF_WIDE_GRAD, KF_JVP, KF_PREDICT, KF_GENERIC_SIM, KF_SCAN_FINISH,
-    KF_SCAN_PARTIAL, KF_DENSE_FINISH, KF_VJP
+    KF_SCAN_PARTIAL, KF_DENSE_FINISH, KF_VJP, KF_POSTVAR
 };
 struct KernelTag { int family = KF_NONE; int p[4] = {0, 0, 0, 0}; };
 
@@ -392,6 +393,7 @@ extern "C" int pioran_ctx_last_kernel_name(pioran_ctx* c, char* buf, int len) tr
         case KF_JVP: snprintf(name, sizeof name, "jvp<%d>", p[0]); break;
         case KF_VJP: snprintf(name, sizeof name, "vjp<%d>", p[0]); break;
         case KF_PREDICT: snprintf(name, sizeof name, "predict<%d>", p[0]); break;
+        case KF_POSTVAR: snprintf(name, sizeof name, "postvar<%d>", p[0]); break;
         case KF_GENERIC_SIM: snprintf(name, sizeof name, "generic_sim<%d,%d>", p[0], p[1]); break;
         case KF_SCAN_FINISH: snprintf(name, sizeof name, "scan_finish"); break;
         case KF_SCAN_PARTIAL: snprintf(name, sizeof name, "scan_partial"); break;
@@ -2360,12 +2362,19 @@ extern "C" int pioran_ctx_set_vjp_workspace(pioran_ctx* c, long long bytes) try 
 } catch (...) { return guard_fail(); }
 
 // ------------------------------------------------------------------------------------------------ posterior mean, draws
-// Common set-up of the two widening entries: coefficient upload, row map, work items for the generic kernel.
+// Common set-up of the widening entries: coefficient upload, row map, work items for the generic kernel.  rows: the row
+// map of a larger batch this call is a θ-chunk of (nullptr: the map of these B sets).
 static int generic_setup(pioran_ctx* c, Series* s, int B, int Jt, const double* a, const double* b, const double* cc,
                          const double* d, const double* mu, const double* nu, const double* y_batch, GenericInputs& gi,
-                         BatchArgs& args, int& BS, int& nitems) {
+                         BatchArgs& args, int& BS, int& nitems, const std::vector<int>* rows = nullptr) {
     std::vector<int> term_row;
-    const int R = make_term_rows(B, Jt, b, d, term_row);
+    int R = 0;
+    if (rows) {
+        term_row = *rows;
+        for (int m = 0; m < Jt; m++) R += term_row[m] < 0 ? 1 : 2;
+    } else {
+        R = make_term_rows(B, Jt, b, d, term_row);
+    }
     BS = bs_for_rank(R);
     if (R > 128 || Jt > 128)
         return fail(PIORAN_EUNSUPPORTED, "rank %d (Jt = %d) exceeds the limit of 128 of the posterior mean and the draws", R, Jt);
@@ -2395,6 +2404,27 @@ static int generic_setup(pioran_ctx* c, Series* s, int B, int Jt, const double* 
     return 0;
 }
 
+// n₀ = searchsortedfirst(t, τ) − 1 (celerite_solver.jl:395): the series lives on the device, fetch its times once
+static int prediction_gaps(pioran_ctx* c, const Series* s, int64_t M, const double* tau, std::vector<int>& n0) {
+    std::vector<double> th(s->N);
+    CUDA_TRY(cudaMemcpyAsync(th.data(), s->t, sizeof(double) * s->N, cudaMemcpyDeviceToHost, c->stream));
+    CUDA_TRY(cudaStreamSynchronize(c->stream));
+    n0.resize(M);
+    for (int64_t m = 0; m < M; m++) n0[m] = (int)(std::lower_bound(th.begin(), th.end(), tau[m]) - th.begin());
+    return 0;
+}
+// backsolve and predict kernels of the posterior mean on a stored factor
+static void launch_posterior_mean(pioran_ctx* c, const PostArgs& pa) {
+    if (pa.Jt <= 64) {
+        celerite_backsolve_kernel<2><<<(pa.B + 3) / 4, 128, 0, c->stream>>>(pa);
+        celerite_predict_kernel<2><<<(pa.B + 3) / 4, 128, 0, c->stream>>>(pa);
+    } else {
+        celerite_backsolve_kernel<4><<<(pa.B + 3) / 4, 128, 0, c->stream>>>(pa);
+        celerite_predict_kernel<4><<<(pa.B + 3) / 4, 128, 0, c->stream>>>(pa);
+    }
+    c->launches += 2;
+}
+
 extern "C" int pioran_celerite_predict(pioran_ctx* c, int series_id, int B, int Jt, const double* a, const double* b,
                                        const double* cc, const double* d, const double* mu, const double* nu, int64_t M,
                                        const double* tau, double* mean_out) try {
@@ -2412,14 +2442,9 @@ extern "C" int pioran_celerite_predict(pioran_ctx* c, int series_id, int B, int 
     Series* s = get_series(c, series_id);
     if (!s) return fail(PIORAN_EINVAL, "unknown series id %d", series_id);
     const int64_t N = s->N;
-    // n₀ = searchsortedfirst(t, τ) − 1 (celerite_solver.jl:395): the series lives on the device, fetch its times once
-    std::vector<double> th(N);
-    CUDA_TRY(cudaMemcpyAsync(th.data(), s->t, sizeof(double) * N, cudaMemcpyDeviceToHost, c->stream));
-    CUDA_TRY(cudaStreamSynchronize(c->stream));
-    std::vector<int> n0(M);
-    for (int64_t m = 0; m < M; m++) n0[m] = (int)(std::lower_bound(th.begin(), th.end(), tau[m]) - th.begin());
-
     int rc, BS, nitems;
+    std::vector<int> n0;
+    if ((rc = prediction_gaps(c, s, M, tau, n0))) return rc;
     GenericInputs gi;
     BatchArgs args;
     if ((rc = generic_setup(c, s, B, Jt, a, b, cc, d, mu, nu, nullptr, gi, args, BS, nitems))) return rc;
@@ -2442,14 +2467,7 @@ extern "C" int pioran_celerite_predict(pioran_ctx* c, int series_id, int B, int 
     pa.t = s->t; pa.tau = tau_dev; pa.n0 = n0_dev; pa.N = N; pa.M = M; pa.B = B; pa.Jt = Jt; pa.RPL = RPL;
     pa.a = gi.a; pa.b = gi.b; pa.c = gi.c; pa.d = gi.d; pa.term_row = c->rows.as<int>(); pa.mu = gi.mu;
     pa.W = W; pa.D = D; pa.z = z; pa.mean = mean;
-    if (Jt <= 64) {
-        celerite_backsolve_kernel<2><<<(B + 3) / 4, 128, 0, c->stream>>>(pa);
-        celerite_predict_kernel<2><<<(B + 3) / 4, 128, 0, c->stream>>>(pa);
-    } else {
-        celerite_backsolve_kernel<4><<<(B + 3) / 4, 128, 0, c->stream>>>(pa);
-        celerite_predict_kernel<4><<<(B + 3) / 4, 128, 0, c->stream>>>(pa);
-    }
-    c->launches += 2;
+    launch_posterior_mean(c, pa);
     cudaEventRecord(c->ev_end, c->stream);
     note_kernel(c, KF_PREDICT, Jt <= 64 ? 2 : 4);
     CUDA_TRY(cudaGetLastError());
@@ -2486,6 +2504,100 @@ extern "C" int pioran_celerite_simulate(pioran_ctx* c, int series_id, int B, int
     else note_kernel(c, KF_GENERIC_SIM, BS, nw_for_bs(BS));
     CUDA_TRY(cudaMemcpyAsync(y_out, c->post.p, sizeof(double) * nBN, cudaMemcpyDeviceToHost, c->stream));
     CUDA_TRY(cudaStreamSynchronize(c->stream));
+    return PIORAN_OK;
+} catch (...) { return guard_fail(); }
+
+// ------------------------------------------------------------------------------------------------ posterior variance (K6)
+static int launch_postvar(pioran_ctx* c, const PostVarArgs& pv, int B) {
+    const int TS = (pv.R + 15) / 16;
+    switch (TS) {
+        case 1: celerite_postvar_kernel<1><<<B, WIDE_THREADS, 0, c->stream>>>(pv); break;
+        case 2: celerite_postvar_kernel<2><<<B, WIDE_THREADS, 0, c->stream>>>(pv); break;
+        case 3: celerite_postvar_kernel<3><<<B, WIDE_THREADS, 0, c->stream>>>(pv); break;
+        case 4: celerite_postvar_kernel<4><<<B, WIDE_THREADS, 0, c->stream>>>(pv); break;
+        case 5: celerite_postvar_kernel<5><<<B, WIDE_THREADS, 0, c->stream>>>(pv); break;
+        case 6: celerite_postvar_kernel<6><<<B, WIDE_THREADS, 0, c->stream>>>(pv); break;
+        case 7: celerite_postvar_kernel<7><<<B, WIDE_THREADS, 0, c->stream>>>(pv); break;
+        case 8: celerite_postvar_kernel<8><<<B, WIDE_THREADS, 0, c->stream>>>(pv); break;
+        default: return fail(PIORAN_EUNSUPPORTED, "rank %d exceeds the limit of 128 of the posterior variance", pv.R);
+    }
+    c->launches++;
+    note_kernel(c, KF_POSTVAR, TS);
+    CUDA_TRY(cudaGetLastError());
+    return 0;
+}
+
+extern "C" int pioran_celerite_predict_var(pioran_ctx* c, int series_id, int B, int Jt, const double* a, const double* b,
+                                           const double* cc, const double* d, const double* mu, const double* nu, int64_t M,
+                                           const double* tau, double* mean_out, double* var_out) try {
+    if (is_group(c)) {   // single-device work of a group runs on its first device
+        int cid;
+        { std::lock_guard<std::mutex> lk(c->mu); const int rc = group_series_id(c, series_id, 0, &cid); if (rc) return rc; }
+        return pioran_celerite_predict_var(c->children[0], cid, B, Jt, a, b, cc, d, mu, nu, M, tau, mean_out, var_out);
+    }
+    if (!c || !a || !b || !cc || !d || !tau || !var_out) return fail(PIORAN_EINVAL, "NULL argument");
+    if (B < 1 || Jt < 1 || M < 1) return fail(PIORAN_EINVAL, "B, Jt and M must be >= 1");
+    for (int64_t m = 1; m < M; m++)
+        if (!(tau[m] >= tau[m - 1])) return fail(PIORAN_EINVAL, "tau must be ascending (tau[%lld] < tau[%lld])", (long long)m, (long long)m - 1);
+    PIORAN_COMPUTE_LOCK(c);
+    CUDA_TRY(cudaSetDevice(c->device));
+    Series* s = get_series(c, series_id);
+    if (!s) return fail(PIORAN_EINVAL, "unknown series id %d", series_id);
+    std::vector<int> term_row;
+    const int R = make_term_rows(B, Jt, b, d, term_row);   // the map of the whole batch, shared by every θ-chunk
+    if (R > 128 || Jt > 128)
+        return fail(PIORAN_EUNSUPPORTED, "rank %d (Jt = %d) exceeds the limit of 128 of the posterior variance", R, Jt);
+    const int64_t N = s->N;
+    int rc;
+    std::vector<int> n0;
+    if ((rc = prediction_gaps(c, s, M, tau, n0))) return rc;
+
+    // θ-chunks of at most 1 GiB: per set W [N·RPL] | D [N] | z [N] | mean [M] | g_τ, D_τ [M·(R + 1)] | var [M]
+    const int RPL = stored_factor_ld(R);
+    const size_t per_set = sizeof(double) * ((size_t)N * RPL + 2 * (size_t)N + (size_t)M * (R + 3));
+    const int Bc = (int)std::max<size_t>(1, std::min<size_t>((size_t)B, ((size_t)1 << 30) / per_set));
+    if ((rc = c->post.ensure(per_set * Bc + sizeof(double) * M + sizeof(int) * (M + 2)))) return rc;
+    double* W = c->post.as<double>();
+    double* D = W + (size_t)Bc * N * RPL;
+    double* z = D + (size_t)Bc * N;
+    double* mean = z + (size_t)Bc * N;
+    double* ws = mean + (size_t)Bc * M;
+    double* var = ws + (size_t)Bc * M * (R + 1);
+    double* tau_dev = var + (size_t)Bc * M;
+    int* n0_dev = reinterpret_cast<int*>(tau_dev + M);
+    CUDA_TRY(cudaMemcpyAsync(tau_dev, tau, sizeof(double) * M, cudaMemcpyHostToDevice, c->stream));
+    CUDA_TRY(cudaMemcpyAsync(n0_dev, n0.data(), sizeof(int) * M, cudaMemcpyHostToDevice, c->stream));
+    cudaEventRecord(c->ev_beg, c->stream);
+    for (int b0 = 0; b0 < B; b0 += Bc) {
+        const int Bk = std::min(Bc, B - b0);
+        const size_t o = (size_t)b0 * Jt;
+        int BS, nitems;
+        GenericInputs gi;
+        BatchArgs args;
+        if ((rc = generic_setup(c, s, Bk, Jt, a + o, b + o, cc + o, d + o, mu ? mu + b0 : nullptr, nu ? nu + b0 : nullptr,
+                                nullptr, gi, args, BS, nitems, &term_row))) return rc;
+        args.W_out = W; args.D_out = D; args.zf_out = z;
+        // the factor of pioran_celerite_predict, and its backsolve and predict kernels: mean_out is predict's, bit for bit
+        if ((rc = BS > 8 ? launch_wide<STEP_STORE>(c, args, nitems) : dispatch_generic_mode<STEP_STORE>(c, BS, args, nitems))) return rc;
+        if (mean_out) {
+            PostArgs pa{};
+            pa.t = s->t; pa.tau = tau_dev; pa.n0 = n0_dev; pa.N = N; pa.M = M; pa.B = Bk; pa.Jt = Jt; pa.RPL = RPL;
+            pa.a = gi.a; pa.b = gi.b; pa.c = gi.c; pa.d = gi.d; pa.term_row = c->rows.as<int>(); pa.mu = gi.mu;
+            pa.W = W; pa.D = D; pa.z = z; pa.mean = mean;
+            launch_posterior_mean(c, pa);
+            CUDA_TRY(cudaGetLastError());
+        }
+        PostVarArgs pv{};
+        pv.t = s->t; pv.tau = tau_dev; pv.n0 = n0_dev; pv.N = N; pv.M = M; pv.Jt = Jt; pv.R = R; pv.RPL = RPL;
+        pv.a = gi.a; pv.b = gi.b; pv.c = gi.c; pv.d = gi.d; pv.term_row = c->rows.as<int>();
+        pv.W = W; pv.D = D; pv.ws = ws; pv.var = var;
+        if ((rc = launch_postvar(c, pv, Bk))) return rc;
+        if (mean_out)
+            CUDA_TRY(cudaMemcpyAsync(mean_out + (size_t)b0 * M, mean, sizeof(double) * (size_t)Bk * M, cudaMemcpyDeviceToHost, c->stream));
+        CUDA_TRY(cudaMemcpyAsync(var_out + (size_t)b0 * M, var, sizeof(double) * (size_t)Bk * M, cudaMemcpyDeviceToHost, c->stream));
+    }
+    cudaEventRecord(c->ev_end, c->stream);
+    CUDA_TRY(cudaStreamSynchronize(c->stream));   // n0 is a local
     return PIORAN_OK;
 } catch (...) { return guard_fail(); }
 
