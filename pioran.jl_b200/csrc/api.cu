@@ -192,9 +192,6 @@ static bool auto_scan(const pioran_ctx* c, int64_t N, int B, int R, bool explici
 }
 static int scan_logl_locked(pioran_ctx* c, Series* s, int series_id, int B, int Jt, const double* a, const double* b,
                             const double* cc, const double* d, const double* mu, const double* nu, double* logl_out);
-static int generic_logl_locked(pioran_ctx* c, Series* s, int B, int Jt, const double* a, const double* b, const double* cc,
-                               const double* d, const double* mu, const double* nu, const double* y_batch,
-                               const double* s2_batch, double* logl_out);
 
 static void scan_forget(pioran_ctx* c);   // drops the range-in-progress record of a context (K3 multi-GPU entries)
 extern "C" int pioran_ctx_destroy(pioran_ctx* c);
@@ -260,6 +257,42 @@ static int group_split(pioran_ctx* g, int B, F fn) {
         if (rcs[k]) return fail(rcs[k], "device %d: %s", g->children[k]->device, errs[k].c_str());
     return 0;
 }
+// The batched host-pointer entries of a group: the S series ids are resolved on every child under the group lock, then
+// fn(child, the child's S ids, N, first row, row count) runs for every slice of B rows.  N is the length of the first series,
+// for slicing per-row data of N steps.
+template <typename F>
+static int group_fanout(pioran_ctx* g, int S, const int* series_ids, int B, F fn) {
+    std::vector<int> cid(g->children.size() * S);
+    {
+        std::lock_guard<std::mutex> lk(g->mu);
+        for (size_t k = 0; k < g->children.size(); k++)
+            for (int q = 0; q < S; q++) { const int rc = group_series_id(g, series_ids[q], k, &cid[k * S + q]); if (rc) return rc; }
+    }
+    int64_t N = 0;
+    const int rc = pioran_series_length(g->children[0], cid[0], &N);
+    if (rc) return rc;
+    return group_split(g, B, [&](int k, int beg, int nb) { return fn(g->children[k], cid.data() + (size_t)k * S, N, beg, nb); });
+}
+template <typename F>
+static int group_fanout(pioran_ctx* g, int series_id, int B, F fn) {
+    return group_fanout(g, 1, &series_id, B, [&](pioran_ctx* ch, const int* cid, int64_t N, int beg, int nb) { return fn(ch, *cid, N, beg, nb); });
+}
+// Single-device work of a group runs on its first device: fn(children[0], the series id on it).
+template <typename F>
+static int group_first(pioran_ctx* g, int series_id, F fn) {
+    int cid;
+    { std::lock_guard<std::mutex> lk(g->mu); const int rc = group_series_id(g, series_id, 0, &cid); if (rc) return rc; }
+    return fn(g->children[0], cid);
+}
+// Settings of a group apply to every child.
+template <typename F>
+static int group_each(pioran_ctx* g, F fn) {
+    for (pioran_ctx* ch : g->children) { const int rc = fn(ch); if (rc) return rc; }
+    return PIORAN_OK;
+}
+// An optional array at an offset: the slices of a group split and the θ-chunks of one call.
+template <typename T>
+static T* at(T* p, size_t off) { return p ? p + off : nullptr; }
 
 extern "C" int pioran_ctx_create_multi(const int* devices, int ndev, pioran_ctx** out) try {
     if (!devices || !out) return fail(PIORAN_EINVAL, "NULL argument");
@@ -339,10 +372,7 @@ extern "C" int pioran_ctx_set_stream(pioran_ctx* c, void* s) try {
 } catch (...) { return guard_fail(); }
 extern "C" int pioran_ctx_synchronize(pioran_ctx* c) try {
     if (!c) return fail(PIORAN_EINVAL, "ctx is NULL");
-    if (is_group(c)) {
-        for (pioran_ctx* ch : c->children) { const int rc = pioran_ctx_synchronize(ch); if (rc) return rc; }
-        return PIORAN_OK;
-    }
+    if (is_group(c)) return group_each(c, [](pioran_ctx* ch) { return pioran_ctx_synchronize(ch); });
     CUDA_TRY(cudaSetDevice(c->device));
     CUDA_TRY(cudaStreamSynchronize(c->stream));
     return PIORAN_OK;
@@ -480,11 +510,7 @@ extern "C" int pioran_series_free(pioran_ctx* c, int id) try {
 
 extern "C" int pioran_series_length(pioran_ctx* c, int id, int64_t* N) try {
     if (!c || !N) return fail(PIORAN_EINVAL, "NULL argument");
-    if (is_group(c)) {
-        int cid;
-        { std::lock_guard<std::mutex> lk(c->mu); const int rc = group_series_id(c, id, 0, &cid); if (rc) return rc; }
-        return pioran_series_length(c->children[0], cid, N);
-    }
+    if (is_group(c)) return group_first(c, id, [&](pioran_ctx* ch, int cid) { return pioran_series_length(ch, cid, N); });
     std::lock_guard<std::mutex> lk(c->mu);
     Series* s = get_series(c, id);
     if (!s) return fail(PIORAN_EINVAL, "unknown series id %d", id);
@@ -683,11 +709,12 @@ static int get_btable(pioran_ctx* c, Series* s, const pioran_approx_spec& sp, Ta
 #ifndef PIORAN_BLK_NW_MID
 #define PIORAN_BLK_NW_MID 12      // 5, 6 row tiles (168 registers)
 #endif
-static int blocked_nw(int NT) {
+static constexpr int blocked_nw_of(int NT) { return NT >= 7 ? PIORAN_BLK_NW_LARGE : NT >= 5 ? PIORAN_BLK_NW_MID : 16; }
+static int blocked_force_nw() {   // PIORAN_BLK_NW=8: eight warps per CTA whatever the row tiles (experiments only)
     static const int force_nw = [] { const char* e = getenv("PIORAN_BLK_NW"); return e ? atoi(e) : 0; }();
-    if (force_nw == 8) return 8;
-    return NT >= 7 ? PIORAN_BLK_NW_LARGE : NT >= 5 ? PIORAN_BLK_NW_MID : 16;
+    return force_nw;
 }
+static int blocked_nw(int NT) { return blocked_force_nw() == 8 ? 8 : blocked_nw_of(NT); }
 template <int NT, int NTR, bool HALF, int NW>
 static int launch_blocked_nw(pioran_ctx* c, const BatchArgs& args, int nitems, int R, int amp_stride) {
     auto kern = celerite_blocked_kernel<NT, NTR, HALF, NW, 1>;
@@ -704,12 +731,10 @@ static int launch_blocked_nw(pioran_ctx* c, const BatchArgs& args, int nitems, i
 }
 template <int NT, int NTR, bool HALF>
 static int launch_blocked(pioran_ctx* c, const BatchArgs& args, int nitems, int tpi, int R, int amp_stride) {
-    constexpr int NWF = NT >= 7 ? PIORAN_BLK_NW_LARGE : NT >= 5 ? PIORAN_BLK_NW_MID : 16;
-    static const int force_nw = [] { const char* e = getenv("PIORAN_BLK_NW"); return e ? atoi(e) : 0; }();   // experiments only
-    if (force_nw == 8 && tpi > 4) return launch_blocked_nw<NT, NTR, HALF, 8>(c, args, nitems, R, amp_stride);
+    if (blocked_force_nw() == 8 && tpi > 4) return launch_blocked_nw<NT, NTR, HALF, 8>(c, args, nitems, R, amp_stride);
     if (tpi <= 4) return launch_blocked_nw<NT, NTR, HALF, 4>(c, args, nitems, R, amp_stride);
     if (tpi <= 8) return launch_blocked_nw<NT, NTR, HALF, 8>(c, args, nitems, R, amp_stride);
-    return launch_blocked_nw<NT, NTR, HALF, NWF>(c, args, nitems, R, amp_stride);
+    return launch_blocked_nw<NT, NTR, HALF, blocked_nw_of(NT)>(c, args, nitems, R, amp_stride);
 }
 static int dispatch_blocked(pioran_ctx* c, const BatchArgs& a, int nitems, int tpi, int R, int amp_stride) {
     const int NT = blk_nt(R);
@@ -730,7 +755,12 @@ static int dispatch_blocked(pioran_ctx* c, const BatchArgs& a, int nitems, int t
     return fail(PIORAN_EUNSUPPORTED, "rank %d not served by the blocked kernel", R);
 }
 
-// K2tw (blocked_wide.cuh): ranks 65 … 128 on the tensor pipe, one CTA of W warps per evaluation.
+// K2tw (blocked_wide.cuh): ranks 65 … 128 on the tensor pipe, one CTA of W warps per evaluation.  Small batches at 4 … 8
+// column tiles run it too, one CTA per evaluation (PIORAN_K2_SMALL_CTA=0: the warp kernel instead).
+static bool small_cta_enabled() {
+    static const bool on = [] { const char* e = getenv("PIORAN_K2_SMALL_CTA"); return !(e && !strcmp(e, "0")); }();
+    return on;
+}
 static bool blocked_wide_enabled(const pioran_ctx* c, int R) {
     static const int mode = [] { const char* e = getenv("PIORAN_K2W"); return (e && (!strcmp(e, "scalar") || !strcmp(e, "0"))) ? 0 : 1; }();
     return mode != 0 && c->sweep_kernel != PIORAN_SWEEP_SCALAR && R > 64 && R <= 128;
@@ -770,24 +800,26 @@ static int dispatch_blocked_wide(pioran_ctx* c, const BatchArgs& a, int nitems, 
 #ifndef PIORAN_NW_LARGE
 #define PIORAN_NW_LARGE 8    // block sizes 7, 8 (register budget 255/thread)
 #endif
-template <int BS> struct KCfg { static constexpr int NW = (BS <= 5) ? PIORAN_NW_SMALL : (BS == 6) ? 10 : PIORAN_NW_LARGE; };
+static constexpr int nw_for_bs(int BS) { return BS <= 5 ? PIORAN_NW_SMALL : BS == 6 ? 10 : PIORAN_NW_LARGE; }
 
-template <int BS>
-static size_t shared_smem_bytes() {
-    constexpr int RPS = rps_of(BS), SD = table_step_doubles(RPS);
-    return sizeof(double) * (2 * (size_t)CHUNK_STEPS * SD + (size_t)KCfg<BS>::NW * 2 * RPS) + 2 * sizeof(uint64_t) + 16;
+// Calls f(std::integral_constant<int, v>{}): a launch site instantiates its kernel for LO … HI, and only for those.
+template <int LO, int HI, class F>
+static int with_int(int v, F f) {
+    if constexpr (LO > HI) return fail(PIORAN_EUNSUPPORTED, "no kernel instantiated for %d", v);
+    else return v == LO ? f(std::integral_constant<int, LO>{}) : with_int<LO + 1, HI>(v, f);
 }
+
 template <int BS>
 static size_t generic_smem_bytes(int Jt) {
     constexpr int RPS = rps_of(BS), SD = table_step_doubles(RPS);
-    return sizeof(double) * (size_t)KCfg<BS>::NW * ((size_t)GCH * SD + 2 * RPS + (size_t)(((GCH + 2) * Jt + 1) & ~1));
+    return sizeof(double) * (size_t)nw_for_bs(BS) * ((size_t)GCH * SD + 2 * RPS + (size_t)(((GCH + 2) * Jt + 1) & ~1));
 }
 
 // Small batches (at most SMALL_NW parameter vectors per CTA, i.e. S·B ≤ 4 × SMs — a nested sampler's few hundred live
 // points): a CTA of 4 warps, one per SM sub-partition.  The full-size CTA would fill its surplus warps with redundant
 // sweeps that share the FP64 pipe of the useful ones and roughly double the latency of the call.
 constexpr int SMALL_NW = 4;
-template <int BS, int NW = KCfg<BS>::NW>
+template <int BS, int NW = nw_for_bs(BS)>
 static int launch_shared(pioran_ctx* c, const BatchArgs& args, int nitems) {
     constexpr int RPS = rps_of(BS), SD = table_step_doubles(RPS);
     auto kern = celerite_shared_kernel<BS, NW>;
@@ -801,7 +833,6 @@ static int launch_shared(pioran_ctx* c, const BatchArgs& args, int nitems) {
     CUDA_TRY(cudaGetLastError());
     return 0;
 }
-static int nw_for_bs_fwd(int BS);
 // Two parameter vectors per warp for block sizes <= 5 (celerite_shared_pair_kernel); PIORAN_PAIR=0 falls back to one.
 #ifndef PIORAN_NW_PAIR
 #define PIORAN_NW_PAIR 8
@@ -810,7 +841,7 @@ static bool pair_enabled(int BS) {
     static const int env = [] { const char* e = getenv("PIORAN_PAIR"); return e ? atoi(e) : 1; }();
     return env != 0 && BS <= 5;
 }
-static int theta_per_item(int BS) { return pair_enabled(BS) ? 2 * PIORAN_NW_PAIR : nw_for_bs_fwd(BS); }
+static int theta_per_item(int BS) { return pair_enabled(BS) ? 2 * PIORAN_NW_PAIR : nw_for_bs(BS); }
 template <int BS>
 static int launch_shared_pair(pioran_ctx* c, const BatchArgs& args, int nitems) {
     constexpr int RPS = rps_of(BS), SD = table_step_doubles(RPS), NW = PIORAN_NW_PAIR;
@@ -825,7 +856,7 @@ static int launch_shared_pair(pioran_ctx* c, const BatchArgs& args, int nitems) 
     CUDA_TRY(cudaGetLastError());
     return 0;
 }
-template <int BS, int NW = KCfg<BS>::NW>
+template <int BS, int NW = nw_for_bs(BS)>
 static int launch_generic(pioran_ctx* c, const BatchArgs& args, int nitems) {
     constexpr int RPS = rps_of(BS), SD = table_step_doubles(RPS);
     auto kern = celerite_generic_kernel<BS, NW>;
@@ -839,8 +870,6 @@ static int launch_generic(pioran_ctx* c, const BatchArgs& args, int nitems) {
     CUDA_TRY(cudaGetLastError());
     return 0;
 }
-static int nw_for_bs(int BS) { return BS <= 5 ? PIORAN_NW_SMALL : BS == 6 ? 10 : PIORAN_NW_LARGE; }
-static int nw_for_bs_fwd(int BS) { return nw_for_bs(BS); }
 
 // K3 pass 3: the generic kernel in its chunked variant, 2 warps per CTA so that a few hundred chunks cover every SM.
 constexpr int CHUNK_NW = 2;
@@ -856,87 +885,35 @@ static int launch_chunked(pioran_ctx* c, const BatchArgs& args, int nctas) {
     return 0;
 }
 static int dispatch_chunked(pioran_ctx* c, int BS, const BatchArgs& a, int nctas) {
-    switch (BS) {
-        case 4: return launch_chunked<4>(c, a, nctas);
-        case 5: return launch_chunked<5>(c, a, nctas);
-        case 6: return launch_chunked<6>(c, a, nctas);
-        case 7: return launch_chunked<7>(c, a, nctas);
-        case 8: return launch_chunked<8>(c, a, nctas);
-    }
-    return fail(PIORAN_EUNSUPPORTED, "block size %d not compiled", BS);
+    return with_int<4, 8>(BS, [&](auto bs) { return launch_chunked<bs>(c, a, nctas); });
 }
 
 static int dispatch_shared(pioran_ctx* c, int BS, const BatchArgs& a, int nitems, int tpi) {
-    if (tpi <= SMALL_NW) {
-        switch (BS) {
-            case 4: return launch_shared<4, SMALL_NW>(c, a, nitems);
-            case 5: return launch_shared<5, SMALL_NW>(c, a, nitems);
-            case 6: return launch_shared<6, SMALL_NW>(c, a, nitems);
-            case 7: return launch_shared<7, SMALL_NW>(c, a, nitems);
-            case 8: return launch_shared<8, SMALL_NW>(c, a, nitems);
-        }
-    }
-    if (tpi <= 8 && BS <= 6) {   // two warps per sub-partition, one parameter vector each
-        switch (BS) {
-            case 4: return launch_shared<4, 8>(c, a, nitems);
-            case 5: return launch_shared<5, 8>(c, a, nitems);
-            case 6: return launch_shared<6, 8>(c, a, nitems);
-        }
-    }
-    if (pair_enabled(BS)) {
-        if (BS == 4) return launch_shared_pair<4>(c, a, nitems);
-        if (BS == 5) return launch_shared_pair<5>(c, a, nitems);
-    }
-    switch (BS) {
-        case 4: return launch_shared<4>(c, a, nitems);
-        case 5: return launch_shared<5>(c, a, nitems);
-        case 6: return launch_shared<6>(c, a, nitems);
-        case 7: return launch_shared<7>(c, a, nitems);
-        case 8: return launch_shared<8>(c, a, nitems);
-    }
-    return fail(PIORAN_EUNSUPPORTED, "block size %d not compiled", BS);
+    if (tpi <= SMALL_NW) return with_int<4, 8>(BS, [&](auto bs) { return launch_shared<bs, SMALL_NW>(c, a, nitems); });
+    if (tpi <= 8 && BS <= 6)    // two warps per sub-partition, one parameter vector each
+        return with_int<4, 6>(BS, [&](auto bs) { return launch_shared<bs, 8>(c, a, nitems); });
+    if (pair_enabled(BS)) return with_int<4, 5>(BS, [&](auto bs) { return launch_shared_pair<bs>(c, a, nitems); });
+    return with_int<4, 8>(BS, [&](auto bs) { return launch_shared<bs>(c, a, nitems); });
 }
 static int dispatch_generic(pioran_ctx* c, int BS, const BatchArgs& a, int nitems, int tpi) {
-    if (tpi <= SMALL_NW) {
-        switch (BS) {
-            case 4: return launch_generic<4, SMALL_NW>(c, a, nitems);
-            case 5: return launch_generic<5, SMALL_NW>(c, a, nitems);
-            case 6: return launch_generic<6, SMALL_NW>(c, a, nitems);
-            case 7: return launch_generic<7, SMALL_NW>(c, a, nitems);
-            case 8: return launch_generic<8, SMALL_NW>(c, a, nitems);
-        }
-    }
-    switch (BS) {
-        case 4: return launch_generic<4>(c, a, nitems);
-        case 5: return launch_generic<5>(c, a, nitems);
-        case 6: return launch_generic<6>(c, a, nitems);
-        case 7: return launch_generic<7>(c, a, nitems);
-        case 8: return launch_generic<8>(c, a, nitems);
-    }
-    return fail(PIORAN_EUNSUPPORTED, "block size %d not compiled", BS);
+    if (tpi <= SMALL_NW) return with_int<4, 8>(BS, [&](auto bs) { return launch_generic<bs, SMALL_NW>(c, a, nitems); });
+    return with_int<4, 8>(BS, [&](auto bs) { return launch_generic<bs>(c, a, nitems); });
 }
 
 // generic kernel in STEP_STORE / STEP_SIM mode (posterior mean and GP draws)
 template <int BS, int MODE>
 static int launch_generic_mode(pioran_ctx* c, const BatchArgs& args, int nitems) {
-    auto kern = celerite_generic_kernel<BS, KCfg<BS>::NW, false, MODE>;
+    auto kern = celerite_generic_kernel<BS, nw_for_bs(BS), false, MODE>;
     const size_t smem = generic_smem_bytes<BS>(args.Jt);
     CUDA_TRY(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    kern<<<nitems, KCfg<BS>::NW * 32, smem, c->stream>>>(args);
+    kern<<<nitems, nw_for_bs(BS) * 32, smem, c->stream>>>(args);
     c->launches++;
     CUDA_TRY(cudaGetLastError());
     return 0;
 }
 template <int MODE>
 static int dispatch_generic_mode(pioran_ctx* c, int BS, const BatchArgs& a, int nitems) {
-    switch (BS) {
-        case 4: return launch_generic_mode<4, MODE>(c, a, nitems);
-        case 5: return launch_generic_mode<5, MODE>(c, a, nitems);
-        case 6: return launch_generic_mode<6, MODE>(c, a, nitems);
-        case 7: return launch_generic_mode<7, MODE>(c, a, nitems);
-        case 8: return launch_generic_mode<8, MODE>(c, a, nitems);
-    }
-    return fail(PIORAN_EUNSUPPORTED, "block size %d not compiled", BS);
+    return with_int<4, 8>(BS, [&](auto bs) { return launch_generic_mode<bs, MODE>(c, a, nitems); });
 }
 
 // Splits S series × B parameter vectors into CTA work items of at most NW vectors, sized so that the number of
@@ -1006,16 +983,11 @@ static int launch_wide(pioran_ctx* c, const BatchArgs& args, int nitems) {
     if (args.R > WIDE_MAX_RANK)
         return fail(PIORAN_EUNSUPPORTED, "rank %d exceeds this build's limit of %d", args.R, WIDE_MAX_RANK);
     if (args.R <= 128) {   // the state fits the register file of one CTA
-        const int TS = (args.R + 15) / 16;
+        const int TS = std::max(5, (args.R + 15) / 16);
         cudaEventRecord(c->ev_beg, c->stream);
-        switch (TS) {
-            case 8: celerite_wide_reg_kernel<8, MODE><<<nitems, WIDE_THREADS, 0, c->stream>>>(args); break;
-            case 7: celerite_wide_reg_kernel<7, MODE><<<nitems, WIDE_THREADS, 0, c->stream>>>(args); break;
-            case 6: celerite_wide_reg_kernel<6, MODE><<<nitems, WIDE_THREADS, 0, c->stream>>>(args); break;
-            default: celerite_wide_reg_kernel<5, MODE><<<nitems, WIDE_THREADS, 0, c->stream>>>(args); break;
-        }
+        with_int<5, 8>(TS, [&](auto ts) { celerite_wide_reg_kernel<ts, MODE><<<nitems, WIDE_THREADS, 0, c->stream>>>(args); return 0; });
         cudaEventRecord(c->ev_end, c->stream);
-        note_kernel(c, MODE == STEP_STORE ? KF_WIDE_REG_STORE : MODE == STEP_SIM ? KF_WIDE_REG_SIM : KF_WIDE_REG, std::max(5, TS));
+        note_kernel(c, MODE == STEP_STORE ? KF_WIDE_REG_STORE : MODE == STEP_SIM ? KF_WIDE_REG_SIM : KF_WIDE_REG, TS);
         c->launches++;
         CUDA_TRY(cudaGetLastError());
         return 0;
@@ -1192,8 +1164,7 @@ static int approx_logl_dev_locked(pioran_ctx* c, int S, const int* series_ids, c
     // Small batches (at most 2 evaluations per SM: a handful of chains, the B = 1 drop-in) at 4 … 8 column tiles: one CTA of four warps
     // per evaluation (blocked_wide.cuh) — a block of 8 steps then costs a quarter of the products per warp: 0.22 instead of 0.48 ms per
     // 1 000 steps at rank 60 (tools/small_batch.py).  Beyond two CTAs per SM the register file holds no more of them and the warp kernel wins.
-    static const bool cta_small_on = [] { const char* e = getenv("PIORAN_K2_SMALL_CTA"); return !(e && !strcmp(e, "0")); }();
-    const bool cta_per_theta = blocked && cta_small_on && blk_nt(R) >= 4 && (long long)S * B <= 2LL * c->num_sms;
+    const bool cta_per_theta = blocked && small_cta_enabled() && blk_nt(R) >= 4 && (long long)S * B <= 2LL * c->num_sms;
     key.push_back(S); key.push_back(B); key.push_back(blocked ? (cta_per_theta ? -2000 - R : -R) : BS); key.push_back(theta_per_series != 0);
     for (int s = 0; s < S; s++) { key.push_back((int64_t)(intptr_t)tabs[s].d); key.push_back((int64_t)(intptr_t)ser[s]->t); key.push_back(ser[s]->N); }
     if (key != c->work_key) {
@@ -1237,33 +1208,19 @@ __global__ void log_shift_kernel(const double* __restrict__ y, const double* __r
     }
 }
 
-extern "C" int pioran_approx_logl_logshift(pioran_ctx* c, int series_id, const pioran_approx_spec* spec, int B, const double* theta,
-                                           double* logl_out) try {
-    if (!c || !spec || !theta || !logl_out) return fail(PIORAN_EINVAL, "NULL argument");
-    if (B < 1) return fail(PIORAN_EINVAL, "B must be >= 1");
-    if (is_group(c)) {
-        const int npar_g = n_psd_par_of(spec->psd_model);
-        if (npar_g < 0) return fail(PIORAN_EINVAL, "unknown psd_model %d", spec->psd_model);
-        std::vector<int> cid(c->children.size());
-        { std::lock_guard<std::mutex> lk(c->mu); for (size_t k = 0; k < cid.size(); k++) { const int rc = group_series_id(c, series_id, k, &cid[k]); if (rc) return rc; } }
-        return group_split(c, B, [&](int k, int beg, int nb) -> int {
-            return pioran_approx_logl_logshift(c->children[k], cid[k], spec, nb, theta + (size_t)beg * (npar_g + 4), logl_out + beg);
-        });
-    }
-    PIORAN_COMPUTE_LOCK(c);
-    CUDA_TRY(cudaSetDevice(c->device));
-    int rc;
-    if ((rc = check_spec(*spec))) return rc;
-    Series* s = get_series(c, series_id);
-    if (!s) return fail(PIORAN_EINVAL, "unknown series id %d", series_id);
-    const int npar = n_psd_par_of(spec->psd_model), ts = npar + 4;
-    if ((rc = c->theta.ensure(sizeof(double) * (size_t)B * ts))) return rc;
-    if ((rc = c->out.ensure(sizeof(double) * (size_t)B))) return rc;
-    CUDA_TRY(cudaMemcpyAsync(c->theta.p, theta, sizeof(double) * (size_t)B * ts, cudaMemcpyHostToDevice, c->stream));
-    // θ-chunks: 16 N bytes of transformed data per parameter vector, at most 1 GiB at a time (written and read once: ≈ 0.3 ms
-    // per 65 536 × 1 000 block against tens of ms of sweep)
+// Parameter vectors per θ-chunk whose workspace of bytes_per_set each stays within cap (at least one).
+static int theta_chunk(int B, size_t bytes_per_set, size_t cap = (size_t)1 << 30) {
+    return (int)std::max<size_t>(1, std::min<size_t>((size_t)B, cap / bytes_per_set));
+}
+
+// The θ-chunk loop of the log-shift entries over the B × ts rows in c->theta: the chunk's transformed data, then
+// fn(first row, row count, the chunk's θ rows, y batch, σ² batch).  16 N bytes of transformed data per parameter vector, at most
+// 1 GiB at a time (written and read once: ≈ 0.3 ms per 65 536 × 1 000 block against tens of ms of sweep).
+template <typename F>
+static int logshift_chunks(pioran_ctx* c, Series* s, int B, int ts, F fn) {
     const int64_t N = s->N;
-    const int chunk = (int)std::max<int64_t>(1, std::min<int64_t>(B, ((int64_t)1 << 30) / (16 * std::max<int64_t>(N, 1))));
+    const int chunk = theta_chunk(B, 16 * (size_t)N);
+    int rc;
     if ((rc = c->post.ensure(sizeof(double) * 2 * (size_t)chunk * N))) return rc;
     double* yb = c->post.as<double>();
     double* sb = yb + (size_t)chunk * N;
@@ -1272,11 +1229,38 @@ extern "C" int pioran_approx_logl_logshift(pioran_ctx* c, int series_id, const p
         const double* th = c->theta.as<double>() + (size_t)off * ts;
         const int64_t total = (int64_t)nb * N;
         const int grid = (int)std::min<int64_t>((total + 255) / 256, (int64_t)c->num_sms * 16);
-        log_shift_kernel<<<grid, 256, 0, c->stream>>>(s->y, s->s2, N, th, ts, npar + 3, nb, yb, sb);
+        log_shift_kernel<<<grid, 256, 0, c->stream>>>(s->y, s->s2, N, th, ts, ts - 1, nb, yb, sb);
         c->launches++;
         CUDA_TRY(cudaGetLastError());
-        if ((rc = approx_logl_dev_locked(c, 1, &series_id, spec, nb, th, 0, c->out.as<double>() + off, ts, yb, sb))) return rc;
+        if ((rc = fn(off, nb, th, yb, sb))) return rc;
     }
+    return 0;
+}
+
+extern "C" int pioran_approx_logl_logshift(pioran_ctx* c, int series_id, const pioran_approx_spec* spec, int B, const double* theta,
+                                           double* logl_out) try {
+    if (!c || !spec || !theta || !logl_out) return fail(PIORAN_EINVAL, "NULL argument");
+    if (B < 1) return fail(PIORAN_EINVAL, "B must be >= 1");
+    const int npar = n_psd_par_of(spec->psd_model);
+    if (npar < 0) return fail(PIORAN_EINVAL, "unknown psd_model %d", spec->psd_model);
+    const int ts = npar + 4;
+    if (is_group(c))
+        return group_fanout(c, series_id, B, [&](pioran_ctx* ch, int id, int64_t, int beg, int nb) {
+            return pioran_approx_logl_logshift(ch, id, spec, nb, theta + (size_t)beg * ts, logl_out + beg);
+        });
+    PIORAN_COMPUTE_LOCK(c);
+    CUDA_TRY(cudaSetDevice(c->device));
+    int rc;
+    if ((rc = check_spec(*spec))) return rc;
+    Series* s = get_series(c, series_id);
+    if (!s) return fail(PIORAN_EINVAL, "unknown series id %d", series_id);
+    if ((rc = c->theta.ensure(sizeof(double) * (size_t)B * ts))) return rc;
+    if ((rc = c->out.ensure(sizeof(double) * (size_t)B))) return rc;
+    CUDA_TRY(cudaMemcpyAsync(c->theta.p, theta, sizeof(double) * (size_t)B * ts, cudaMemcpyHostToDevice, c->stream));
+    if ((rc = logshift_chunks(c, s, B, ts, [&](int off, int nb, const double* th, const double* yb, const double* sb) {
+             return approx_logl_dev_locked(c, 1, &series_id, spec, nb, th, 0, c->out.as<double>() + off, ts, yb, sb);
+         })))
+        return rc;
     CUDA_TRY(cudaMemcpyAsync(logl_out, c->out.p, sizeof(double) * (size_t)B, cudaMemcpyDeviceToHost, c->stream));
     CUDA_TRY(cudaStreamSynchronize(c->stream));
     return PIORAN_OK;
@@ -1295,33 +1279,23 @@ extern "C" int pioran_approx_logl(pioran_ctx* c, int S, const int* series_ids, c
                                   const double* theta, int theta_per_series, double* logl_out) try {
     if (!c || !series_ids || !specs || !theta || !logl_out) return fail(PIORAN_EINVAL, "NULL argument");
     if (S < 1 || B < 1) return fail(PIORAN_EINVAL, "S and B must be >= 1");
-    if (is_group(c)) {
-        const int npar_g = n_psd_par_of(specs[0].psd_model);
-        if (npar_g < 0) return fail(PIORAN_EINVAL, "unknown psd_model %d", specs[0].psd_model);
-        const int tsg = npar_g + 3;
-        std::vector<std::vector<int>> cids(c->children.size(), std::vector<int>(S));
-        {
-            std::lock_guard<std::mutex> lk(c->mu);
-            for (size_t k = 0; k < c->children.size(); k++)
-                for (int q = 0; q < S; q++) { const int rc = group_series_id(c, series_ids[q], k, &cids[k][q]); if (rc) return rc; }
-        }
-        return group_split(c, B, [&](int k, int beg, int nb) -> int {
-            if (S == 1) return pioran_approx_logl(c->children[k], 1, cids[k].data(), specs, nb, theta + (size_t)beg * tsg, 0, logl_out + beg);
+    const int npar = n_psd_par_of(specs[0].psd_model);
+    if (npar < 0) return fail(PIORAN_EINVAL, "unknown psd_model %d", specs[0].psd_model);
+    const int ts = npar + 3;
+    if (is_group(c))
+        return group_fanout(c, S, series_ids, B, [&](pioran_ctx* ch, const int* ids, int64_t, int beg, int nb) -> int {
+            if (S == 1) return pioran_approx_logl(ch, 1, ids, specs, nb, theta + (size_t)beg * ts, 0, logl_out + beg);
             // several series: the slice of every series' rows is gathered, evaluated and scattered back
-            std::vector<double> th((size_t)(theta_per_series ? S : 1) * nb * tsg), out((size_t)S * nb);
+            std::vector<double> th((size_t)(theta_per_series ? S : 1) * nb * ts), out((size_t)S * nb);
             for (int q = 0; q < (theta_per_series ? S : 1); q++)
-                std::memcpy(th.data() + (size_t)q * nb * tsg, theta + ((size_t)q * B + beg) * tsg, sizeof(double) * (size_t)nb * tsg);
-            const int rc = pioran_approx_logl(c->children[k], S, cids[k].data(), specs, nb, th.data(), theta_per_series, out.data());
+                std::memcpy(th.data() + (size_t)q * nb * ts, theta + ((size_t)q * B + beg) * ts, sizeof(double) * (size_t)nb * ts);
+            const int rc = pioran_approx_logl(ch, S, ids, specs, nb, th.data(), theta_per_series, out.data());
             if (rc) return rc;
             for (int q = 0; q < S; q++) std::memcpy(logl_out + (size_t)q * B + beg, out.data() + (size_t)q * nb, sizeof(double) * nb);
             return 0;
         });
-    }
     PIORAN_COMPUTE_LOCK(c);
     CUDA_TRY(cudaSetDevice(c->device));
-    const int npar = n_psd_par_of(specs[0].psd_model);
-    if (npar < 0) return fail(PIORAN_EINVAL, "unknown psd_model %d", specs[0].psd_model);
-    const int ts = npar + 3;
     const size_t nth = (size_t)(theta_per_series ? S : 1) * B * ts;
     int rc;
     if (S == 1 && (rc = check_spec(specs[0])) == 0) {
@@ -1406,14 +1380,11 @@ extern "C" int pioran_prior_transform_logl(pioran_ctx* c, int series_id, const p
                                            double* logl_out) try {
     if (!c || !spec || !priors || !cube || !logl_out) return fail(PIORAN_EINVAL, "NULL argument");
     if (B < 1) return fail(PIORAN_EINVAL, "B must be >= 1");
-    if (is_group(c)) {
-        std::vector<int> cid(c->children.size());
-        { std::lock_guard<std::mutex> lk(c->mu); for (size_t k = 0; k < cid.size(); k++) { const int rc = group_series_id(c, series_id, k, &cid[k]); if (rc) return rc; } }
-        return group_split(c, B, [&](int k, int beg, int nb) -> int {
-            return pioran_prior_transform_logl(c->children[k], cid[k], spec, ncol, priors, nb, cube + (size_t)beg * ncol,
-                                               theta_out ? theta_out + (size_t)beg * ncol : nullptr, logl_out + beg);
+    if (is_group(c))
+        return group_fanout(c, series_id, B, [&](pioran_ctx* ch, int id, int64_t, int beg, int nb) {
+            return pioran_prior_transform_logl(ch, id, spec, ncol, priors, nb, cube + (size_t)beg * ncol, at(theta_out, (size_t)beg * ncol),
+                                               logl_out + beg);
         });
-    }
     const int npar = n_psd_par_of(spec->psd_model);
     if (npar < 0) return fail(PIORAN_EINVAL, "unknown psd_model %d", spec->psd_model);
     if (ncol != npar + 3) return fail(PIORAN_EINVAL, "ncol must be %d (psd parameters, norm, nu, mu) for this model, got %d", npar + 3, ncol);
@@ -1663,14 +1634,10 @@ extern "C" int pioran_approx_logl_logshift_grad(pioran_ctx* c, int series_id, co
     const int npar = n_psd_par_of(spec->psd_model);
     if (npar < 0) return fail(PIORAN_EINVAL, "unknown psd_model %d", spec->psd_model);
     const int ts = npar + 4;
-    if (is_group(c)) {
-        std::vector<int> cid(c->children.size());
-        { std::lock_guard<std::mutex> lk(c->mu); for (size_t k = 0; k < cid.size(); k++) { const int rc = group_series_id(c, series_id, k, &cid[k]); if (rc) return rc; } }
-        return group_split(c, B, [&](int k, int beg, int nb) -> int {
-            return pioran_approx_logl_logshift_grad(c->children[k], cid[k], spec, nb, theta + (size_t)beg * ts, logl_out ? logl_out + beg : nullptr,
-                                                    grad_out + (size_t)beg * ts);
+    if (is_group(c))
+        return group_fanout(c, series_id, B, [&](pioran_ctx* ch, int id, int64_t, int beg, int nb) {
+            return pioran_approx_logl_logshift_grad(ch, id, spec, nb, theta + (size_t)beg * ts, at(logl_out, beg), grad_out + (size_t)beg * ts);
         });
-    }
     PIORAN_COMPUTE_LOCK(c);
     CUDA_TRY(cudaSetDevice(c->device));
     int rc;
@@ -1680,23 +1647,12 @@ extern "C" int pioran_approx_logl_logshift_grad(pioran_ctx* c, int series_id, co
     if ((rc = c->theta.ensure(sizeof(double) * (size_t)B * ts))) return rc;
     if ((rc = c->out.ensure(sizeof(double) * (size_t)B * (ts + 1)))) return rc;
     CUDA_TRY(cudaMemcpyAsync(c->theta.p, theta, sizeof(double) * (size_t)B * ts, cudaMemcpyHostToDevice, c->stream));
-    const int64_t N = s->N;
-    const int chunk = (int)std::max<int64_t>(1, std::min<int64_t>(B, ((int64_t)1 << 30) / (16 * std::max<int64_t>(N, 1))));
-    if ((rc = c->post.ensure(sizeof(double) * 2 * (size_t)chunk * N))) return rc;
-    double* yb = c->post.as<double>();
-    double* sb = yb + (size_t)chunk * N;
     double* gl = c->out.as<double>();
     double* gg = gl + B;
-    for (int off = 0; off < B; off += chunk) {
-        const int nb = std::min(chunk, B - off);
-        const double* th = c->theta.as<double>() + (size_t)off * ts;
-        const int64_t total = (int64_t)nb * N;
-        const int grid = (int)std::min<int64_t>((total + 255) / 256, (int64_t)c->num_sms * 16);
-        log_shift_kernel<<<grid, 256, 0, c->stream>>>(s->y, s->s2, N, th, ts, npar + 3, nb, yb, sb);
-        c->launches++;
-        CUDA_TRY(cudaGetLastError());
-        if ((rc = approx_logl_grad_dev_locked(c, series_id, spec, nb, th, gl + off, gg + (size_t)off * ts, true, yb, sb))) return rc;
-    }
+    if ((rc = logshift_chunks(c, s, B, ts, [&](int off, int nb, const double* th, const double* yb, const double* sb) {
+             return approx_logl_grad_dev_locked(c, series_id, spec, nb, th, gl + off, gg + (size_t)off * ts, true, yb, sb);
+         })))
+        return rc;
     if (logl_out) CUDA_TRY(cudaMemcpyAsync(logl_out, gl, sizeof(double) * (size_t)B, cudaMemcpyDeviceToHost, c->stream));
     CUDA_TRY(cudaMemcpyAsync(grad_out, gg, sizeof(double) * (size_t)B * ts, cudaMemcpyDeviceToHost, c->stream));
     CUDA_TRY(cudaStreamSynchronize(c->stream));
@@ -1717,22 +1673,15 @@ extern "C" int pioran_approx_logl_grad(pioran_ctx* c, int series_id, const piora
                                        const double* theta, double* logl_out, double* grad_out) try {
     if (!c || !spec || !theta || !grad_out) return fail(PIORAN_EINVAL, "NULL argument");
     if (B < 1) return fail(PIORAN_EINVAL, "B must be >= 1");
-    if (is_group(c)) {
-        const int npar_g = n_psd_par_of(spec->psd_model);
-        if (npar_g < 0) return fail(PIORAN_EINVAL, "unknown psd_model %d", spec->psd_model);
-        const int Pg = npar_g + 3;
-        std::vector<int> cid(c->children.size());
-        { std::lock_guard<std::mutex> lk(c->mu); for (size_t k = 0; k < cid.size(); k++) { const int rc = group_series_id(c, series_id, k, &cid[k]); if (rc) return rc; } }
-        return group_split(c, B, [&](int k, int beg, int nb) -> int {
-            return pioran_approx_logl_grad(c->children[k], cid[k], spec, nb, theta + (size_t)beg * Pg, logl_out ? logl_out + beg : nullptr,
-                                           grad_out + (size_t)beg * Pg);
-        });
-    }
-    PIORAN_COMPUTE_LOCK(c);
-    CUDA_TRY(cudaSetDevice(c->device));
     const int npar = n_psd_par_of(spec->psd_model);
     if (npar < 0) return fail(PIORAN_EINVAL, "unknown psd_model %d", spec->psd_model);
     const int P = npar + 3;
+    if (is_group(c))
+        return group_fanout(c, series_id, B, [&](pioran_ctx* ch, int id, int64_t, int beg, int nb) {
+            return pioran_approx_logl_grad(ch, id, spec, nb, theta + (size_t)beg * P, at(logl_out, beg), grad_out + (size_t)beg * P);
+        });
+    PIORAN_COMPUTE_LOCK(c);
+    CUDA_TRY(cudaSetDevice(c->device));
     int rc;
     if ((rc = c->theta.ensure(sizeof(double) * (size_t)B * P))) return rc;
     if ((rc = c->out.ensure(sizeof(double) * (size_t)B * (P + 1)))) return rc;
@@ -1781,43 +1730,61 @@ static int upload_generic(pioran_ctx* c, int B, int Jt, int64_t N, const double*
     return 0;
 }
 
-extern "C" int pioran_celerite_logl(pioran_ctx* c, int series_id, int B, int Jt, const double* a, const double* b,
-                                    const double* cc, const double* d, const double* mu, const double* nu,
-                                    const double* y_batch, const double* s2_batch, double* logl_out) try {
-    if (!c || !a || !b || !cc || !d || !logl_out) return fail(PIORAN_EINVAL, "NULL argument");
-    if (B < 1 || Jt < 1) return fail(PIORAN_EINVAL, "B and Jt must be >= 1");
-    if (is_group(c)) {
-        std::vector<int> cid(c->children.size());
-        int64_t Ng = 0;
-        { std::lock_guard<std::mutex> lk(c->mu); for (size_t k = 0; k < cid.size(); k++) { const int rc = group_series_id(c, series_id, k, &cid[k]); if (rc) return rc; } }
-        if (y_batch || s2_batch) { const int rc = pioran_series_length(c->children[0], cid[0], &Ng); if (rc) return rc; }
-        return group_split(c, B, [&](int k, int beg, int nb) -> int {
-            const size_t o = (size_t)beg * Jt;
-            return pioran_celerite_logl(c->children[k], cid[k], nb, Jt, a + o, b + o, cc + o, d + o, mu ? mu + beg : nullptr, nu ? nu + beg : nullptr,
-                                        y_batch ? y_batch + (size_t)beg * Ng : nullptr, s2_batch ? s2_batch + (size_t)beg * Ng : nullptr, logl_out + beg);
-        });
-    }
-    PIORAN_COMPUTE_LOCK(c);
+// The start of every explicit-coefficient entry; the caller holds the context's lock.  Looks the series up, reduces the rank
+// (make_term_rows) and enforces the entry's rank limit: limit_fmt is formatted with the rank, Jt and max_rank as %1$d, %2$d
+// and %3$d.  The caller uploads the coefficients (upload_generic): the likelihood first decides whether the scan path runs,
+// and the posterior variance uploads one θ-chunk at a time.
+struct ExplicitSet { Series* s = nullptr; std::vector<int> term_row; int R = 0; };
+static const char* const LOGL_LIMIT = "rank %1$d (Jt = %2$d) exceeds this build's limit of %3$d";
+static const char* const POSTERIOR_LIMIT = "rank %1$d (Jt = %2$d) exceeds the limit of %3$d of the posterior mean and the draws";
+static int explicit_front(pioran_ctx* c, int series_id, int B, int Jt, const double* b, const double* d, int max_rank,
+                          const char* limit_fmt, ExplicitSet& x) {
     CUDA_TRY(cudaSetDevice(c->device));
-    Series* s = get_series(c, series_id);
-    if (!s) return fail(PIORAN_EINVAL, "unknown series id %d", series_id);
-    std::vector<int> term_row;
-    const int R = make_term_rows(B, Jt, b, d, term_row);
-    if (!y_batch && !s2_batch && auto_scan(c, s->N, B, R, true))
-        return scan_logl_locked(c, s, series_id, B, Jt, a, b, cc, d, mu, nu, logl_out);
-    return generic_logl_locked(c, s, B, Jt, a, b, cc, d, mu, nu, y_batch, s2_batch, logl_out);
-} catch (...) { return guard_fail(); }
+    x.s = get_series(c, series_id);
+    if (!x.s) return fail(PIORAN_EINVAL, "unknown series id %d", series_id);
+    x.R = make_term_rows(B, Jt, b, d, x.term_row);
+    if (x.R > max_rank) return fail(PIORAN_EUNSUPPORTED, limit_fmt, x.R, Jt, max_rank);
+    return 0;
+}
 
-// The sequential sweep on explicit coefficients (generic K2, K2w above rank 64); the context is locked by the caller.
-static int generic_logl_locked(pioran_ctx* c, Series* s, int B, int Jt, const double* a, const double* b, const double* cc,
+// Row map and work items of the generic kernel (one CTA per parameter vector at wide ranks) for uploaded coefficients, and the
+// launch arguments.  term_row may be the map of a larger batch this call is a θ-chunk of.
+static int generic_setup(pioran_ctx* c, Series* s, int B, int Jt, const std::vector<int>& term_row, int R, const GenericInputs& gi,
+                         BatchArgs& args, int& nitems, int& tpi) {
+    int rc;
+    if ((rc = c->rows.ensure(sizeof(int) * (Jt + 1)))) return rc;
+    CUDA_TRY(cudaMemcpyAsync(c->rows.p, term_row.data(), sizeof(int) * Jt, cudaMemcpyHostToDevice, c->stream));
+    if ((rc = c->out.ensure(sizeof(double) * (size_t)B))) return rc;
+    ItemPlan ip;
+    const int BS = bs_for_rank(R);
+    plan_items(c, 1, &s, nullptr, B, BS > 8 ? 1 : nw_for_bs(BS), false, ip);
+    c->work_key.clear();  // the work buffer is shared with the fused path's cached plan
+    if ((rc = c->work.ensure(sizeof(WorkItem) * ip.items.size()))) return rc;
+    CUDA_TRY(cudaMemcpyAsync(c->work.p, ip.items.data(), sizeof(WorkItem) * ip.items.size(), cudaMemcpyHostToDevice,
+                             c->stream));
+    CUDA_TRY(cudaStreamSynchronize(c->stream));   // term_row and ip are host sources
+    nitems = (int)ip.items.size();
+    tpi = ip.tpi;
+    args = BatchArgs{};
+    args.work = c->work.as<WorkItem>();
+    args.a = gi.a; args.b = gi.b; args.c = gi.c; args.d = gi.d;
+    args.Jt = Jt;
+    args.term_row = c->rows.as<int>();
+    args.R = R;
+    args.mu = gi.mu; args.nu = gi.nu; args.pstride = 1;
+    args.y_batch = gi.yb; args.s2_batch = gi.sb; args.ystride = s->N;
+    args.out = c->out.as<double>();
+    return 0;
+}
+
+// The sequential sweep on explicit coefficients (generic K2, K2w above rank 64) for the set-up of explicit_front; the context
+// is locked by the caller.
+static int generic_logl_locked(pioran_ctx* c, const ExplicitSet& x, int B, int Jt, const double* a, const double* b, const double* cc,
                                const double* d, const double* mu, const double* nu, const double* y_batch,
                                const double* s2_batch, double* logl_out) {
-    std::vector<int> term_row;
-    const int R = make_term_rows(B, Jt, b, d, term_row);
-    const int BS = bs_for_rank(R);
-    const bool wide = BS > 8;
-    if (wide && R > WIDE_MAX_RANK)
-        return fail(PIORAN_EUNSUPPORTED, "rank %d (Jt = %d) exceeds this build's limit of %d", R, Jt, WIDE_MAX_RANK);
+    Series* s = x.s;
+    const int R = x.R;
+    const std::vector<int>& term_row = x.term_row;
     int rc;
     GenericInputs gi;
     if ((rc = upload_generic(c, B, Jt, s->N, a, b, cc, d, mu, nu, y_batch, s2_batch, gi))) return rc;
@@ -1882,38 +1849,41 @@ static int generic_logl_locked(pioran_ctx* c, Series* s, int B, int Jt, const do
             args.mu = gi.mu; args.nu = gi.nu; args.pstride = 1;
             args.y_batch = gi.yb; args.s2_batch = gi.sb; args.ystride = s->N;
             args.out = c->out.as<double>();
-            static const bool cta_small_on = [] { const char* e = getenv("PIORAN_K2_SMALL_CTA"); return !(e && !strcmp(e, "0")); }();
-            if ((rc = (R > 64 || (cta_small_on && blk_nt(R) >= 4)) ? dispatch_blocked_wide(c, args, B, R, RPA) : dispatch_blocked(c, args, B, 1, R, RPA))) return rc;
+            if ((rc = (R > 64 || (small_cta_enabled() && blk_nt(R) >= 4)) ? dispatch_blocked_wide(c, args, B, R, RPA) : dispatch_blocked(c, args, B, 1, R, RPA))) return rc;
             CUDA_TRY(cudaMemcpyAsync(logl_out, c->out.p, sizeof(double) * (size_t)B, cudaMemcpyDeviceToHost, c->stream));
             CUDA_TRY(cudaStreamSynchronize(c->stream));
             return PIORAN_OK;
         }
     }
-    if ((rc = c->rows.ensure(sizeof(int) * (Jt + 1)))) return rc;
-    CUDA_TRY(cudaMemcpyAsync(c->rows.p, term_row.data(), sizeof(int) * Jt, cudaMemcpyHostToDevice, c->stream));
-    if ((rc = c->out.ensure(sizeof(double) * (size_t)B))) return rc;
-    ItemPlan ip;
-    Series* sp = s;
-    plan_items(c, 1, &sp, nullptr, B, wide ? 1 : nw_for_bs(BS), false, ip);
-    c->work_key.clear();  // the work buffer is shared with the fused path's cached plan
-    if ((rc = c->work.ensure(sizeof(WorkItem) * ip.items.size()))) return rc;
-    CUDA_TRY(cudaMemcpyAsync(c->work.p, ip.items.data(), sizeof(WorkItem) * ip.items.size(), cudaMemcpyHostToDevice,
-                             c->stream));
-    CUDA_TRY(cudaStreamSynchronize(c->stream));
-    BatchArgs args{};
-    args.work = c->work.as<WorkItem>();
-    args.a = gi.a; args.b = gi.b; args.c = gi.c; args.d = gi.d;
-    args.Jt = Jt;
-    args.term_row = c->rows.as<int>();
-    args.R = R;
-    args.mu = gi.mu; args.nu = gi.nu; args.pstride = 1;
-    args.y_batch = gi.yb; args.s2_batch = gi.sb; args.ystride = s->N;
-    args.out = c->out.as<double>();
-    if ((rc = wide ? launch_wide(c, args, (int)ip.items.size()) : dispatch_generic(c, BS, args, (int)ip.items.size(), ip.tpi))) return rc;
+    BatchArgs args;
+    int nitems, tpi;
+    if ((rc = generic_setup(c, s, B, Jt, term_row, R, gi, args, nitems, tpi))) return rc;
+    const int BS = bs_for_rank(R);
+    if ((rc = BS > 8 ? launch_wide(c, args, nitems) : dispatch_generic(c, BS, args, nitems, tpi))) return rc;
     CUDA_TRY(cudaMemcpyAsync(logl_out, c->out.p, sizeof(double) * (size_t)B, cudaMemcpyDeviceToHost, c->stream));
     CUDA_TRY(cudaStreamSynchronize(c->stream));
     return PIORAN_OK;
 }
+
+extern "C" int pioran_celerite_logl(pioran_ctx* c, int series_id, int B, int Jt, const double* a, const double* b,
+                                    const double* cc, const double* d, const double* mu, const double* nu,
+                                    const double* y_batch, const double* s2_batch, double* logl_out) try {
+    if (!c || !a || !b || !cc || !d || !logl_out) return fail(PIORAN_EINVAL, "NULL argument");
+    if (B < 1 || Jt < 1) return fail(PIORAN_EINVAL, "B and Jt must be >= 1");
+    if (is_group(c))
+        return group_fanout(c, series_id, B, [&](pioran_ctx* ch, int id, int64_t N, int beg, int nb) {
+            const size_t o = (size_t)beg * Jt;
+            return pioran_celerite_logl(ch, id, nb, Jt, a + o, b + o, cc + o, d + o, at(mu, beg), at(nu, beg), at(y_batch, beg * N),
+                                        at(s2_batch, beg * N), logl_out + beg);
+        });
+    PIORAN_COMPUTE_LOCK(c);
+    ExplicitSet x;
+    int rc;
+    if ((rc = explicit_front(c, series_id, B, Jt, b, d, WIDE_MAX_RANK, LOGL_LIMIT, x))) return rc;
+    if (!y_batch && !s2_batch && auto_scan(c, x.s->N, B, x.R, true))
+        return scan_logl_locked(c, x.s, series_id, B, Jt, a, b, cc, d, mu, nu, logl_out);
+    return generic_logl_locked(c, x, B, Jt, a, b, cc, d, mu, nu, y_batch, s2_batch, logl_out);
+} catch (...) { return guard_fail(); }
 
 
 // ------------------------------------------------------------------------------------------------ PSD features (QPO)
@@ -1968,13 +1938,10 @@ extern "C" int pioran_approx_features_logl(pioran_ctx* c, int series_id, const p
     const int npar = n_psd_par_of(spec->psd_model);
     if (npar < 0) return fail(PIORAN_EINVAL, "unknown psd_model %d", spec->psd_model);
     const int ts = npar + 3 + 3 * n_features;
-    if (is_group(c)) {
-        std::vector<int> cid(c->children.size());
-        { std::lock_guard<std::mutex> lk(c->mu); for (size_t k = 0; k < cid.size(); k++) { const int rc = group_series_id(c, series_id, k, &cid[k]); if (rc) return rc; } }
-        return group_split(c, B, [&](int k, int beg, int nb) -> int {
-            return pioran_approx_features_logl(c->children[k], cid[k], spec, n_features, nb, theta + (size_t)beg * ts, logl_out + beg);
+    if (is_group(c))
+        return group_fanout(c, series_id, B, [&](pioran_ctx* ch, int id, int64_t, int beg, int nb) {
+            return pioran_approx_features_logl(ch, id, spec, n_features, nb, theta + (size_t)beg * ts, logl_out + beg);
         });
-    }
     PIORAN_COMPUTE_LOCK(c);
     CUDA_TRY(cudaSetDevice(c->device));
     Series* s = get_series(c, series_id);
@@ -1987,7 +1954,9 @@ extern "C" int pioran_approx_features_logl(pioran_ctx* c, int series_id, const p
     CUDA_TRY(cudaMemcpyAsync(co.data(), c->coef.p, sizeof(double) * 4 * n, cudaMemcpyDeviceToHost, c->stream));
     CUDA_TRY(cudaStreamSynchronize(c->stream));
     for (int i = 0; i < B; i++) { nu[i] = theta[(size_t)i * ts + npar + 1]; mu[i] = theta[(size_t)i * ts + npar + 2]; }
-    return generic_logl_locked(c, s, B, Jt, co.data(), co.data() + n, co.data() + 2 * n, co.data() + 3 * n, mu.data(), nu.data(),
+    ExplicitSet x;
+    if ((rc = explicit_front(c, series_id, B, Jt, co.data() + n, co.data() + 3 * n, WIDE_MAX_RANK, LOGL_LIMIT, x))) return rc;
+    return generic_logl_locked(c, x, B, Jt, co.data(), co.data() + n, co.data() + 2 * n, co.data() + 3 * n, mu.data(), nu.data(),
                                nullptr, nullptr, logl_out);
 } catch (...) { return guard_fail(); }
 
@@ -2005,15 +1974,7 @@ static int jvp_dev_locked(pioran_ctx* c, Series* s, int B, int Jt, int P, int R,
     const int TS = std::max(1, (R + 15) / 16);
     const unsigned grid = (unsigned)B * (unsigned)P;
     cudaEventRecord(c->ev_beg, c->stream);
-    switch (TS) {
-        case 1: celerite_jvp_kernel<1><<<grid, WIDE_THREADS, 0, c->stream>>>(ja); break;
-        case 2: celerite_jvp_kernel<2><<<grid, WIDE_THREADS, 0, c->stream>>>(ja); break;
-        case 3: celerite_jvp_kernel<3><<<grid, WIDE_THREADS, 0, c->stream>>>(ja); break;
-        case 4: celerite_jvp_kernel<4><<<grid, WIDE_THREADS, 0, c->stream>>>(ja); break;
-        case 5: celerite_jvp_kernel<5><<<grid, WIDE_THREADS, 0, c->stream>>>(ja); break;
-        case 6: celerite_jvp_kernel<6><<<grid, WIDE_THREADS, 0, c->stream>>>(ja); break;
-        default: return fail(PIORAN_EUNSUPPORTED, "the JVP is built for ranks <= %d (rank %d)", JVP_MAX_RANK, R);
-    }
+    if ((rc = with_int<1, 6>(TS, [&](auto ts) { celerite_jvp_kernel<ts><<<grid, WIDE_THREADS, 0, c->stream>>>(ja); return 0; }))) return rc;
     cudaEventRecord(c->ev_end, c->stream);
     note_kernel(c, KF_JVP, TS);
     c->launches++;
@@ -2032,31 +1993,19 @@ extern "C" int pioran_celerite_logl_jvp(pioran_ctx* c, int series_id, int B, int
     if (B < 1 || Jt < 1) return fail(PIORAN_EINVAL, "B and Jt must be >= 1");
     if (P < 1) return fail(PIORAN_EINVAL, "P must be >= 1 (got %d)", P);
     if ((long long)B * P > 0x7fffffffLL) return fail(PIORAN_EINVAL, "B * P too large");
-    if (is_group(c)) {
-        std::vector<int> cid(c->children.size());
-        int64_t Ng = 0;
-        { std::lock_guard<std::mutex> lk(c->mu); for (size_t k = 0; k < cid.size(); k++) { const int rc = group_series_id(c, series_id, k, &cid[k]); if (rc) return rc; } }
-        if (y_batch || s2_batch || dy || ds2) { const int rc = pioran_series_length(c->children[0], cid[0], &Ng); if (rc) return rc; }
-        return group_split(c, B, [&](int k, int beg, int nb) -> int {
+    if (is_group(c))
+        return group_fanout(c, series_id, B, [&](pioran_ctx* ch, int id, int64_t N, int beg, int nb) {
             const size_t o = (size_t)beg * Jt, op = (size_t)beg * P;
-            return pioran_celerite_logl_jvp(c->children[k], cid[k], nb, Jt, P, a + o, b + o, cc + o, d + o, mu ? mu + beg : nullptr,
-                                            nu ? nu + beg : nullptr, y_batch ? y_batch + (size_t)beg * Ng : nullptr,
-                                            s2_batch ? s2_batch + (size_t)beg * Ng : nullptr, da ? da + op * Jt : nullptr,
-                                            db ? db + op * Jt : nullptr, dc ? dc + op * Jt : nullptr, dd ? dd + op * Jt : nullptr,
-                                            dmu ? dmu + op : nullptr, dnu ? dnu + op : nullptr, dy ? dy + op * Ng : nullptr,
-                                            ds2 ? ds2 + op * Ng : nullptr, logl_out ? logl_out + beg : nullptr, dlogl_out + op);
+            return pioran_celerite_logl_jvp(ch, id, nb, Jt, P, a + o, b + o, cc + o, d + o, at(mu, beg), at(nu, beg), at(y_batch, beg * N),
+                                            at(s2_batch, beg * N), at(da, op * Jt), at(db, op * Jt), at(dc, op * Jt), at(dd, op * Jt),
+                                            at(dmu, op), at(dnu, op), at(dy, op * N), at(ds2, op * N), at(logl_out, beg), dlogl_out + op);
         });
-    }
     PIORAN_COMPUTE_LOCK(c);
-    CUDA_TRY(cudaSetDevice(c->device));
-    Series* s = get_series(c, series_id);
-    if (!s) return fail(PIORAN_EINVAL, "unknown series id %d", series_id);
-    std::vector<int> term_row;
-    const int R = make_term_rows(B, Jt, b, d, term_row);
-    if (R > JVP_MAX_RANK) return fail(PIORAN_EUNSUPPORTED, "the JVP is built for ranks <= %d (rank %d, Jt = %d)", JVP_MAX_RANK, R, Jt);
+    ExplicitSet x;
     int rc;
+    if ((rc = explicit_front(c, series_id, B, Jt, b, d, JVP_MAX_RANK, "the JVP is built for ranks <= %3$d (rank %1$d, Jt = %2$d)", x))) return rc;
     GenericInputs gi;
-    const int64_t N = s->N;
+    const int64_t N = x.s->N;
     if ((rc = upload_generic(c, B, Jt, N, a, b, cc, d, mu, nu, y_batch, s2_batch, gi))) return rc;
     // coefficient tangents [B × P × Jt] each, then dμ, dν [B × P]
     const size_t nt = (size_t)B * P * Jt, np = (size_t)B * P;
@@ -2073,7 +2022,7 @@ extern "C" int pioran_celerite_logl_jvp(pioran_ctx* c, int series_id, int B, int
     double* gg = gl + B;
     // data tangents [B × P × N]: θ-chunks of at most 1 GiB for dy and ds2 together
     const bool dt = dy || ds2;
-    const int chunk = dt ? (int)std::max<int64_t>(1, std::min<int64_t>(B, ((int64_t)1 << 30) / (16 * (int64_t)P * std::max<int64_t>(N, 1)))) : B;
+    const int chunk = dt ? theta_chunk(B, 16 * (size_t)P * N) : B;
     const size_t nc = (size_t)chunk * P * N;
     if (dt && (rc = c->post.ensure(sizeof(double) * 2 * nc))) return rc;
     for (int off = 0; off < B; off += chunk) {
@@ -2081,11 +2030,10 @@ extern "C" int pioran_celerite_logl_jvp(pioran_ctx* c, int series_id, int B, int
         const size_t o = (size_t)off * Jt, op = (size_t)off * P, nd = (size_t)nb * P * N;
         JvpArgs ja{};
         ja.a = gi.a + o; ja.b = gi.b + o; ja.c = gi.c + o; ja.d = gi.d + o;
-        ja.mu = gi.mu ? gi.mu + off : nullptr; ja.nu = gi.nu ? gi.nu + off : nullptr;
-        ja.y_batch = gi.yb ? gi.yb + (size_t)off * N : nullptr; ja.s2_batch = gi.sb ? gi.sb + (size_t)off * N : nullptr;
-        ja.da = dsrc[0] ? dsrc[0] + op * Jt : nullptr; ja.db = dsrc[1] ? dsrc[1] + op * Jt : nullptr;
-        ja.dc = dsrc[2] ? dsrc[2] + op * Jt : nullptr; ja.dd = dsrc[3] ? dsrc[3] + op * Jt : nullptr;
-        ja.dmu = dsrc[4] ? dsrc[4] + op : nullptr; ja.dnu = dsrc[5] ? dsrc[5] + op : nullptr;
+        ja.mu = at(gi.mu, off); ja.nu = at(gi.nu, off);
+        ja.y_batch = at(gi.yb, (size_t)off * N); ja.s2_batch = at(gi.sb, (size_t)off * N);
+        ja.da = at(dsrc[0], op * Jt); ja.db = at(dsrc[1], op * Jt); ja.dc = at(dsrc[2], op * Jt); ja.dd = at(dsrc[3], op * Jt);
+        ja.dmu = at(dsrc[4], op); ja.dnu = at(dsrc[5], op);
         if (dy) {
             ja.dy = c->post.as<double>();
             CUDA_TRY(cudaMemcpyAsync(c->post.p, dy + op * N, sizeof(double) * nd, cudaMemcpyHostToDevice, c->stream));
@@ -2095,7 +2043,7 @@ extern "C" int pioran_celerite_logl_jvp(pioran_ctx* c, int series_id, int B, int
             CUDA_TRY(cudaMemcpyAsync(c->post.as<double>() + nc, ds2 + op * N, sizeof(double) * nd, cudaMemcpyHostToDevice, c->stream));
         }
         ja.logl = gl + off; ja.dlogl = gg + op;
-        if ((rc = jvp_dev_locked(c, s, nb, Jt, P, R, term_row, ja))) return rc;
+        if ((rc = jvp_dev_locked(c, x.s, nb, Jt, P, x.R, x.term_row, ja))) return rc;
     }
     if (logl_out) CUDA_TRY(cudaMemcpyAsync(logl_out, gl, sizeof(double) * (size_t)B, cudaMemcpyDeviceToHost, c->stream));
     CUDA_TRY(cudaMemcpyAsync(dlogl_out, gg, sizeof(double) * np, cudaMemcpyDeviceToHost, c->stream));
@@ -2103,66 +2051,82 @@ extern "C" int pioran_celerite_logl_jvp(pioran_ctx* c, int series_id, int B, int
     return PIORAN_OK;
 } catch (...) { return guard_fail(); }
 
-// Gradient with PSD features: K1 on pairs (approx_features_grad_kernel) writes the coefficients and their tangents along every θ
-// column into the JVP's device layout, then one K5g sweep with P = θ columns.  Nothing returns to the host in between.
-extern "C" int pioran_approx_features_logl_grad(pioran_ctx* c, int series_id, const pioran_approx_spec* spec, int n_features,
-                                                int B, const double* theta, double* logl_out, double* grad_out) try {
+// Gradients with PSD features, in forward mode (one K5g sweep with P = θ columns) and in reverse mode (one K5r sweep and the
+// contraction kernel): K1 on pairs (approx_features_grad_kernel) writes the coefficients (co: a, b, c, d [B × Jt], μ, ν [B]) and
+// their tangents along every θ column (tg: [B × P × Jt] each, then [B × P] each) in the JVP's device layout.  Nothing returns
+// to the host in between.  features_grad_check validates what the group split needs; features_grad_setup runs under the
+// caller's lock.
+struct FeatureGrad { Series* s = nullptr; int Jt = 0, R = 0, P = 0; std::vector<int> term_row; double *co = nullptr, *tg = nullptr; };
+static int features_grad_check(pioran_ctx* c, const pioran_approx_spec* spec, int n_features, int B, const double* theta,
+                               const double* grad_out, int& ts) {
     if (!c || !spec || !theta || !grad_out) return fail(PIORAN_EINVAL, "NULL argument");
     if (B < 1) return fail(PIORAN_EINVAL, "B must be >= 1");
     const int npar = n_psd_par_of(spec->psd_model);
     if (npar < 0) return fail(PIORAN_EINVAL, "unknown psd_model %d", spec->psd_model);
     if (n_features < 1) return fail(PIORAN_EINVAL, "n_features must be >= 1 (got %d)", n_features);
     if (n_features > MAXFEAT) return fail(PIORAN_EUNSUPPORTED, "at most %d features (got %d)", MAXFEAT, n_features);
-    const int ts = npar + 3 + 3 * n_features;
+    ts = npar + 3 + 3 * n_features;
     if ((long long)B * ts > 0x7fffffffLL) return fail(PIORAN_EINVAL, "B too large");
-    if (is_group(c)) {
-        std::vector<int> cid(c->children.size());
-        { std::lock_guard<std::mutex> lk(c->mu); for (size_t k = 0; k < cid.size(); k++) { const int rc = group_series_id(c, series_id, k, &cid[k]); if (rc) return rc; } }
-        return group_split(c, B, [&](int k, int beg, int nb) -> int {
-            return pioran_approx_features_logl_grad(c->children[k], cid[k], spec, n_features, nb, theta + (size_t)beg * ts,
-                                                    logl_out ? logl_out + beg : nullptr, grad_out + (size_t)beg * ts);
-        });
-    }
-    PIORAN_COMPUTE_LOCK(c);
+    return 0;
+}
+static int features_grad_setup(pioran_ctx* c, int series_id, const pioran_approx_spec* spec, int nf, int B, const double* theta,
+                               int ts, int max_rank, FeatureGrad& f) {
     CUDA_TRY(cudaSetDevice(c->device));
     int rc;
     if ((rc = check_spec(*spec))) return rc;
-    Series* s = get_series(c, series_id);
-    if (!s) return fail(PIORAN_EINVAL, "unknown series id %d", series_id);
-    const int J = spec->n_components, nf = n_features;
-    const int Jc = spec->basis == PIORAN_BASIS_SHO ? J : 2 * J, Jt = Jc + nf;
-    const int Rc = rank_of(spec->basis, J), R = Rc + 2 * nf;
-    if (R > JVP_MAX_RANK) return fail(PIORAN_EUNSUPPORTED, "gradients with features are built for ranks <= %d (rank %d)", JVP_MAX_RANK, R);
+    f.s = get_series(c, series_id);
+    if (!f.s) return fail(PIORAN_EINVAL, "unknown series id %d", series_id);
+    const int J = spec->n_components;
+    const int Jc = spec->basis == PIORAN_BASIS_SHO ? J : 2 * J, Rc = rank_of(spec->basis, J);
+    f.Jt = Jc + nf; f.R = Rc + 2 * nf; f.P = ts;
+    if (f.R > max_rank) return fail(PIORAN_EUNSUPPORTED, "gradients with features are built for ranks <= %d (rank %d)", max_rank, f.R);
     ApproxPlan* plan;
     if ((rc = get_plan(c, *spec, &plan))) return rc;
     // term rows: continuum as in the approx path (SHO complex; DRWCelerite complex ++ real), features complex
-    std::vector<int> term_row(Jt + 1, 0);
+    f.term_row.assign(f.Jt + 1, 0);
     for (int j = 0; j < J; j++) {
-        term_row[j] = 2 * j;
-        if (spec->basis != PIORAN_BASIS_SHO) term_row[J + j] = -(2 * J + j + 1);
+        f.term_row[j] = 2 * j;
+        if (spec->basis != PIORAN_BASIS_SHO) f.term_row[J + j] = -(2 * J + j + 1);
     }
-    for (int f = 0; f < nf; f++) term_row[Jc + f] = Rc + 2 * f;
-    const int P = ts;
-    const size_t n = (size_t)B * Jt, nt = (size_t)B * P * Jt, np = (size_t)B * P;
+    for (int q = 0; q < nf; q++) f.term_row[Jc + q] = Rc + 2 * q;
+    const size_t n = (size_t)B * f.Jt, nt = (size_t)B * f.P * f.Jt, np = (size_t)B * f.P;
     if ((rc = c->theta.ensure(sizeof(double) * (size_t)B * ts))) return rc;
     if ((rc = c->coef.ensure(sizeof(double) * (4 * n + 2 * (size_t)B)))) return rc;
     if ((rc = c->gradws.ensure(sizeof(double) * (4 * nt + 2 * np)))) return rc;
-    if ((rc = c->out.ensure(sizeof(double) * (size_t)B * (P + 1)))) return rc;
     CUDA_TRY(cudaMemcpyAsync(c->theta.p, theta, sizeof(double) * (size_t)B * ts, cudaMemcpyHostToDevice, c->stream));
-    double* co = c->coef.as<double>();
-    double* tg = c->gradws.as<double>();
-    double* gl = c->out.as<double>();
-    double* gg = gl + B;
+    double* co = f.co = c->coef.as<double>();
+    double* tg = f.tg = c->gradws.as<double>();
     approx_features_grad_kernel<<<(unsigned)((np + 127) / 128), 128, 0, c->stream>>>(
-        plan, B, c->theta.as<double>(), ts, nf, npar + 3, co, co + n, co + 2 * n, co + 3 * n, co + 4 * n, co + 4 * n + B,
+        plan, B, c->theta.as<double>(), ts, nf, ts - 3 * nf, co, co + n, co + 2 * n, co + 3 * n, co + 4 * n, co + 4 * n + B,
         tg, tg + nt, tg + 2 * nt, tg + 3 * nt, tg + 4 * nt, tg + 4 * nt + np);
     c->launches++;
     CUDA_TRY(cudaGetLastError());
+    return 0;
+}
+
+extern "C" int pioran_approx_features_logl_grad(pioran_ctx* c, int series_id, const pioran_approx_spec* spec, int n_features,
+                                                int B, const double* theta, double* logl_out, double* grad_out) try {
+    int ts, rc;
+    if ((rc = features_grad_check(c, spec, n_features, B, theta, grad_out, ts))) return rc;
+    if (is_group(c))
+        return group_fanout(c, series_id, B, [&](pioran_ctx* ch, int id, int64_t, int beg, int nb) {
+            return pioran_approx_features_logl_grad(ch, id, spec, n_features, nb, theta + (size_t)beg * ts, at(logl_out, beg),
+                                                    grad_out + (size_t)beg * ts);
+        });
+    PIORAN_COMPUTE_LOCK(c);
+    FeatureGrad f;
+    if ((rc = features_grad_setup(c, series_id, spec, n_features, B, theta, ts, JVP_MAX_RANK, f))) return rc;
+    const int Jt = f.Jt, P = f.P;
+    const size_t n = (size_t)B * Jt, nt = (size_t)B * P * Jt, np = (size_t)B * P;
+    if ((rc = c->out.ensure(sizeof(double) * (size_t)B * (P + 1)))) return rc;
+    double* gl = c->out.as<double>();
+    double* gg = gl + B;
+    const double *co = f.co, *tg = f.tg;
     JvpArgs ja{};
     ja.a = co; ja.b = co + n; ja.c = co + 2 * n; ja.d = co + 3 * n; ja.mu = co + 4 * n; ja.nu = co + 4 * n + B;
     ja.da = tg; ja.db = tg + nt; ja.dc = tg + 2 * nt; ja.dd = tg + 3 * nt; ja.dmu = tg + 4 * nt; ja.dnu = tg + 4 * nt + np;
     ja.logl = gl; ja.dlogl = gg;
-    if ((rc = jvp_dev_locked(c, s, B, Jt, P, R, term_row, ja))) return rc;
+    if ((rc = jvp_dev_locked(c, f.s, B, Jt, P, f.R, f.term_row, ja))) return rc;
     if (logl_out) CUDA_TRY(cudaMemcpyAsync(logl_out, gl, sizeof(double) * (size_t)B, cudaMemcpyDeviceToHost, c->stream));
     CUDA_TRY(cudaMemcpyAsync(grad_out, gg, sizeof(double) * np, cudaMemcpyDeviceToHost, c->stream));
     CUDA_TRY(cudaStreamSynchronize(c->stream));
@@ -2184,8 +2148,7 @@ static int vjp_dev_locked(pioran_ctx* c, Series* s, int B, int Jt, int R, const 
     int64_t K = (int64_t)std::ceil(std::sqrt((double)N));
     K = (K + WIDE_CH - 1) / WIDE_CH * WIDE_CH;
     const size_t per = sizeof(double) * vjp_ws_doubles(TS, N, (int)K);
-    const size_t cap = c->vjp_ws_bytes ? c->vjp_ws_bytes : ((size_t)1 << 30);
-    const int chunk = (int)std::max<size_t>(1, std::min<size_t>((size_t)B, cap / per));
+    const int chunk = c->vjp_ws_bytes ? theta_chunk(B, per, c->vjp_ws_bytes) : theta_chunk(B, per);
     if ((rc = c->vjpws.ensure(per * (size_t)chunk))) return rc;
     if ((rc = c->rows.ensure(sizeof(int) * (Jt + 1)))) return rc;
     CUDA_TRY(cudaMemcpyAsync(c->rows.p, term_row.data(), sizeof(int) * Jt, cudaMemcpyHostToDevice, c->stream));
@@ -2198,23 +2161,15 @@ static int vjp_dev_locked(pioran_ctx* c, Series* s, int B, int Jt, int R, const 
         va.t = s->t; va.y = s->y; va.s2 = s->s2; va.N = N;
         va.term_row = c->rows.as<int>(); va.Jt = Jt; va.K = (int)K; va.ws = c->vjpws.as<double>();
         va.a = base.a + o; va.b = base.b + o; va.c = base.c + o; va.d = base.d + o;
-        va.mu = base.mu ? base.mu + off : nullptr; va.nu = base.nu ? base.nu + off : nullptr;
-        va.y_batch = base.y_batch ? base.y_batch + on : nullptr; va.s2_batch = base.s2_batch ? base.s2_batch + on : nullptr;
-        va.logl = base.logl ? base.logl + off : nullptr;
-        va.ga = base.ga ? base.ga + o : nullptr; va.gb = base.gb ? base.gb + o : nullptr;
-        va.gc = base.gc ? base.gc + o : nullptr; va.gd = base.gd ? base.gd + o : nullptr;
-        va.gmu = base.gmu ? base.gmu + off : nullptr; va.gnu = base.gnu ? base.gnu + off : nullptr;
+        va.mu = at(base.mu, off); va.nu = at(base.nu, off);
+        va.y_batch = at(base.y_batch, on); va.s2_batch = at(base.s2_batch, on);
+        va.logl = at(base.logl, off);
+        va.ga = at(base.ga, o); va.gb = at(base.gb, o); va.gc = at(base.gc, o); va.gd = at(base.gd, o);
+        va.gmu = at(base.gmu, off); va.gnu = at(base.gnu, off);
         va.gy = gy_host ? c->post.as<double>() : nullptr;
         va.gs2 = gs2_host ? c->post.as<double>() + nd : nullptr;
         cudaEventRecord(c->ev_beg, c->stream);
-        switch (TS) {
-            case 1: celerite_vjp_kernel<1><<<nb, WIDE_THREADS, 0, c->stream>>>(va); break;
-            case 2: celerite_vjp_kernel<2><<<nb, WIDE_THREADS, 0, c->stream>>>(va); break;
-            case 3: celerite_vjp_kernel<3><<<nb, WIDE_THREADS, 0, c->stream>>>(va); break;
-            case 4: celerite_vjp_kernel<4><<<nb, WIDE_THREADS, 0, c->stream>>>(va); break;
-            case 5: celerite_vjp_kernel<5><<<nb, WIDE_THREADS, 0, c->stream>>>(va); break;
-            default: celerite_vjp_kernel<6><<<nb, WIDE_THREADS, 0, c->stream>>>(va); break;
-        }
+        with_int<1, 6>(TS, [&](auto ts) { celerite_vjp_kernel<ts><<<nb, WIDE_THREADS, 0, c->stream>>>(va); return 0; });
         cudaEventRecord(c->ev_end, c->stream);
         note_kernel(c, KF_VJP, TS);
         c->launches++;
@@ -2234,30 +2189,19 @@ extern "C" int pioran_celerite_logl_vjp(pioran_ctx* c, int series_id, int B, int
     if (!c || !a || !b || !cc || !d) return fail(PIORAN_EINVAL, "NULL argument");
     if (!ga && !gb && !gc && !gd && !gmu && !gnu && !gy && !gs2) return fail(PIORAN_EINVAL, "no gradient output given");
     if (B < 1 || Jt < 1) return fail(PIORAN_EINVAL, "B and Jt must be >= 1");
-    if (is_group(c)) {
-        std::vector<int> cid(c->children.size());
-        int64_t Ng = 0;
-        { std::lock_guard<std::mutex> lk(c->mu); for (size_t k = 0; k < cid.size(); k++) { const int rc = group_series_id(c, series_id, k, &cid[k]); if (rc) return rc; } }
-        if (y_batch || s2_batch || gy || gs2) { const int rc = pioran_series_length(c->children[0], cid[0], &Ng); if (rc) return rc; }
-        return group_split(c, B, [&](int k, int beg, int nb) -> int {
-            const size_t o = (size_t)beg * Jt, on = (size_t)beg * Ng;
-            return pioran_celerite_logl_vjp(c->children[k], cid[k], nb, Jt, a + o, b + o, cc + o, d + o, mu ? mu + beg : nullptr,
-                                            nu ? nu + beg : nullptr, y_batch ? y_batch + on : nullptr, s2_batch ? s2_batch + on : nullptr,
-                                            logl_out ? logl_out + beg : nullptr, ga ? ga + o : nullptr, gb ? gb + o : nullptr,
-                                            gc ? gc + o : nullptr, gd ? gd + o : nullptr, gmu ? gmu + beg : nullptr,
-                                            gnu ? gnu + beg : nullptr, gy ? gy + on : nullptr, gs2 ? gs2 + on : nullptr);
+    if (is_group(c))
+        return group_fanout(c, series_id, B, [&](pioran_ctx* ch, int id, int64_t N, int beg, int nb) {
+            const size_t o = (size_t)beg * Jt, on = (size_t)beg * N;
+            return pioran_celerite_logl_vjp(ch, id, nb, Jt, a + o, b + o, cc + o, d + o, at(mu, beg), at(nu, beg), at(y_batch, on),
+                                            at(s2_batch, on), at(logl_out, beg), at(ga, o), at(gb, o), at(gc, o), at(gd, o), at(gmu, beg),
+                                            at(gnu, beg), at(gy, on), at(gs2, on));
         });
-    }
     PIORAN_COMPUTE_LOCK(c);
-    CUDA_TRY(cudaSetDevice(c->device));
-    Series* s = get_series(c, series_id);
-    if (!s) return fail(PIORAN_EINVAL, "unknown series id %d", series_id);
-    std::vector<int> term_row;
-    const int R = make_term_rows(B, Jt, b, d, term_row);
-    if (R > VJP_MAX_RANK) return fail(PIORAN_EUNSUPPORTED, "the VJP is built for ranks <= %d (rank %d, Jt = %d)", VJP_MAX_RANK, R, Jt);
+    ExplicitSet x;
     int rc;
+    if ((rc = explicit_front(c, series_id, B, Jt, b, d, VJP_MAX_RANK, "the VJP is built for ranks <= %3$d (rank %1$d, Jt = %2$d)", x))) return rc;
     GenericInputs gi;
-    if ((rc = upload_generic(c, B, Jt, s->N, a, b, cc, d, mu, nu, y_batch, s2_batch, gi))) return rc;
+    if ((rc = upload_generic(c, B, Jt, x.s->N, a, b, cc, d, mu, nu, y_batch, s2_batch, gi))) return rc;
     // logL [B], ā … d̄ [B × Jt] each, μ̄, ν̄ [B]
     const size_t n = (size_t)B * Jt;
     if ((rc = c->out.ensure(sizeof(double) * (3 * (size_t)B + 4 * n)))) return rc;
@@ -2267,7 +2211,7 @@ extern "C" int pioran_celerite_logl_vjp(pioran_ctx* c, int series_id, int B, int
     base.y_batch = gi.yb; base.s2_batch = gi.sb;
     base.logl = ob; base.ga = ob + B; base.gb = ob + B + n; base.gc = ob + B + 2 * n; base.gd = ob + B + 3 * n;
     base.gmu = ob + B + 4 * n; base.gnu = ob + 2 * B + 4 * n;
-    if ((rc = vjp_dev_locked(c, s, B, Jt, R, term_row, base, gy, gs2))) return rc;
+    if ((rc = vjp_dev_locked(c, x.s, B, Jt, x.R, x.term_row, base, gy, gs2))) return rc;
     double* hdst[7] = {logl_out, ga, gb, gc, gd, gmu, gnu};
     const double* dsrc[7] = {base.logl, base.ga, base.gb, base.gc, base.gd, base.gmu, base.gnu};
     for (int q = 0; q < 7; q++)
@@ -2276,67 +2220,29 @@ extern "C" int pioran_celerite_logl_vjp(pioran_ctx* c, int series_id, int B, int
     return PIORAN_OK;
 } catch (...) { return guard_fail(); }
 
-// Gradient with PSD features in reverse mode: the same coefficients and tangents as pioran_approx_features_logl_grad
-// (approx_features_grad_kernel), one K5r sweep for ∂logL with respect to the coefficients, and their contraction with the tangents
-// along every θ column (vjp_contract_kernel).  Nothing returns to the host in between.
 extern "C" int pioran_approx_features_logl_grad_reverse(pioran_ctx* c, int series_id, const pioran_approx_spec* spec, int n_features,
                                                         int B, const double* theta, double* logl_out, double* grad_out) try {
-    if (!c || !spec || !theta || !grad_out) return fail(PIORAN_EINVAL, "NULL argument");
-    if (B < 1) return fail(PIORAN_EINVAL, "B must be >= 1");
-    const int npar = n_psd_par_of(spec->psd_model);
-    if (npar < 0) return fail(PIORAN_EINVAL, "unknown psd_model %d", spec->psd_model);
-    if (n_features < 1) return fail(PIORAN_EINVAL, "n_features must be >= 1 (got %d)", n_features);
-    if (n_features > MAXFEAT) return fail(PIORAN_EUNSUPPORTED, "at most %d features (got %d)", MAXFEAT, n_features);
-    const int ts = npar + 3 + 3 * n_features;
-    if ((long long)B * ts > 0x7fffffffLL) return fail(PIORAN_EINVAL, "B too large");
-    if (is_group(c)) {
-        std::vector<int> cid(c->children.size());
-        { std::lock_guard<std::mutex> lk(c->mu); for (size_t k = 0; k < cid.size(); k++) { const int rc = group_series_id(c, series_id, k, &cid[k]); if (rc) return rc; } }
-        return group_split(c, B, [&](int k, int beg, int nb) -> int {
-            return pioran_approx_features_logl_grad_reverse(c->children[k], cid[k], spec, n_features, nb, theta + (size_t)beg * ts,
-                                                            logl_out ? logl_out + beg : nullptr, grad_out + (size_t)beg * ts);
+    int ts, rc;
+    if ((rc = features_grad_check(c, spec, n_features, B, theta, grad_out, ts))) return rc;
+    if (is_group(c))
+        return group_fanout(c, series_id, B, [&](pioran_ctx* ch, int id, int64_t, int beg, int nb) {
+            return pioran_approx_features_logl_grad_reverse(ch, id, spec, n_features, nb, theta + (size_t)beg * ts, at(logl_out, beg),
+                                                            grad_out + (size_t)beg * ts);
         });
-    }
     PIORAN_COMPUTE_LOCK(c);
-    CUDA_TRY(cudaSetDevice(c->device));
-    int rc;
-    if ((rc = check_spec(*spec))) return rc;
-    Series* s = get_series(c, series_id);
-    if (!s) return fail(PIORAN_EINVAL, "unknown series id %d", series_id);
-    const int J = spec->n_components, nf = n_features;
-    const int Jc = spec->basis == PIORAN_BASIS_SHO ? J : 2 * J, Jt = Jc + nf;
-    const int Rc = rank_of(spec->basis, J), R = Rc + 2 * nf;
-    if (R > VJP_MAX_RANK) return fail(PIORAN_EUNSUPPORTED, "gradients with features are built for ranks <= %d (rank %d)", VJP_MAX_RANK, R);
-    ApproxPlan* plan;
-    if ((rc = get_plan(c, *spec, &plan))) return rc;
-    // term rows as in pioran_approx_features_logl_grad
-    std::vector<int> term_row(Jt + 1, 0);
-    for (int j = 0; j < J; j++) {
-        term_row[j] = 2 * j;
-        if (spec->basis != PIORAN_BASIS_SHO) term_row[J + j] = -(2 * J + j + 1);
-    }
-    for (int f = 0; f < nf; f++) term_row[Jc + f] = Rc + 2 * f;
-    const int P = ts;
+    FeatureGrad f;
+    if ((rc = features_grad_setup(c, series_id, spec, n_features, B, theta, ts, VJP_MAX_RANK, f))) return rc;
+    const int Jt = f.Jt, P = f.P;
     const size_t n = (size_t)B * Jt, nt = (size_t)B * P * Jt, np = (size_t)B * P;
-    if ((rc = c->theta.ensure(sizeof(double) * (size_t)B * ts))) return rc;
-    if ((rc = c->coef.ensure(sizeof(double) * (4 * n + 2 * (size_t)B)))) return rc;
-    if ((rc = c->gradws.ensure(sizeof(double) * (4 * nt + 2 * np)))) return rc;
     // logL [B], ā … d̄ [B × Jt] each, μ̄, ν̄ [B], ∂logL/∂θ [B × P]
     if ((rc = c->out.ensure(sizeof(double) * (3 * (size_t)B + 4 * n + np)))) return rc;
-    CUDA_TRY(cudaMemcpyAsync(c->theta.p, theta, sizeof(double) * (size_t)B * ts, cudaMemcpyHostToDevice, c->stream));
-    double* co = c->coef.as<double>();
-    double* tg = c->gradws.as<double>();
     double* ob = c->out.as<double>();
-    approx_features_grad_kernel<<<(unsigned)((np + 127) / 128), 128, 0, c->stream>>>(
-        plan, B, c->theta.as<double>(), ts, nf, npar + 3, co, co + n, co + 2 * n, co + 3 * n, co + 4 * n, co + 4 * n + B,
-        tg, tg + nt, tg + 2 * nt, tg + 3 * nt, tg + 4 * nt, tg + 4 * nt + np);
-    c->launches++;
-    CUDA_TRY(cudaGetLastError());
+    const double *co = f.co, *tg = f.tg;
     VjpArgs base{};
     base.a = co; base.b = co + n; base.c = co + 2 * n; base.d = co + 3 * n; base.mu = co + 4 * n; base.nu = co + 4 * n + B;
     base.logl = ob; base.ga = ob + B; base.gb = ob + B + n; base.gc = ob + B + 2 * n; base.gd = ob + B + 3 * n;
     base.gmu = ob + B + 4 * n; base.gnu = ob + 2 * B + 4 * n;
-    if ((rc = vjp_dev_locked(c, s, B, Jt, R, term_row, base, nullptr, nullptr))) return rc;
+    if ((rc = vjp_dev_locked(c, f.s, B, Jt, f.R, f.term_row, base, nullptr, nullptr))) return rc;
     double* gg = ob + 3 * (size_t)B + 4 * n;
     vjp_contract_kernel<<<(unsigned)((np + 127) / 128), 128, 0, c->stream>>>(
         B, P, Jt, base.ga, base.gb, base.gc, base.gd, base.gmu, base.gnu, tg, tg + nt, tg + 2 * nt, tg + 3 * nt, tg + 4 * nt,
@@ -2350,10 +2256,7 @@ extern "C" int pioran_approx_features_logl_grad_reverse(pioran_ctx* c, int serie
 } catch (...) { return guard_fail(); }
 
 extern "C" int pioran_ctx_set_vjp_workspace(pioran_ctx* c, long long bytes) try {
-    if (is_group(c)) {
-        for (pioran_ctx* ch : c->children) { const int rc = pioran_ctx_set_vjp_workspace(ch, bytes); if (rc) return rc; }
-        return PIORAN_OK;
-    }
+    if (is_group(c)) return group_each(c, [&](pioran_ctx* ch) { return pioran_ctx_set_vjp_workspace(ch, bytes); });
     if (!c) return fail(PIORAN_EINVAL, "ctx is NULL");
     if (bytes < 0) return fail(PIORAN_EINVAL, "bytes must be >= 0 (0 = 1 GiB)");
     std::lock_guard<std::mutex> lk(c->mu);
@@ -2362,48 +2265,6 @@ extern "C" int pioran_ctx_set_vjp_workspace(pioran_ctx* c, long long bytes) try 
 } catch (...) { return guard_fail(); }
 
 // ------------------------------------------------------------------------------------------------ posterior mean, draws
-// Common set-up of the widening entries: coefficient upload, row map, work items for the generic kernel.  rows: the row
-// map of a larger batch this call is a θ-chunk of (nullptr: the map of these B sets).
-static int generic_setup(pioran_ctx* c, Series* s, int B, int Jt, const double* a, const double* b, const double* cc,
-                         const double* d, const double* mu, const double* nu, const double* y_batch, GenericInputs& gi,
-                         BatchArgs& args, int& BS, int& nitems, const std::vector<int>* rows = nullptr) {
-    std::vector<int> term_row;
-    int R = 0;
-    if (rows) {
-        term_row = *rows;
-        for (int m = 0; m < Jt; m++) R += term_row[m] < 0 ? 1 : 2;
-    } else {
-        R = make_term_rows(B, Jt, b, d, term_row);
-    }
-    BS = bs_for_rank(R);
-    if (R > 128 || Jt > 128)
-        return fail(PIORAN_EUNSUPPORTED, "rank %d (Jt = %d) exceeds the limit of 128 of the posterior mean and the draws", R, Jt);
-    int rc;
-    if ((rc = upload_generic(c, B, Jt, s->N, a, b, cc, d, mu, nu, y_batch, nullptr, gi))) return rc;
-    if ((rc = c->rows.ensure(sizeof(int) * (Jt + 1)))) return rc;
-    CUDA_TRY(cudaMemcpyAsync(c->rows.p, term_row.data(), sizeof(int) * Jt, cudaMemcpyHostToDevice, c->stream));
-    if ((rc = c->out.ensure(sizeof(double) * (size_t)B))) return rc;
-    ItemPlan ip;
-    Series* sp = s;
-    plan_items(c, 1, &sp, nullptr, B, BS > 8 ? 1 : nw_for_bs(BS), false, ip);      // wide ranks: one CTA per parameter vector
-    c->work_key.clear();
-    if ((rc = c->work.ensure(sizeof(WorkItem) * ip.items.size()))) return rc;
-    CUDA_TRY(cudaMemcpyAsync(c->work.p, ip.items.data(), sizeof(WorkItem) * ip.items.size(), cudaMemcpyHostToDevice,
-                             c->stream));
-    CUDA_TRY(cudaStreamSynchronize(c->stream));   // term_row and ip are locals
-    nitems = (int)ip.items.size();
-    args = BatchArgs{};
-    args.work = c->work.as<WorkItem>();
-    args.a = gi.a; args.b = gi.b; args.c = gi.c; args.d = gi.d;
-    args.Jt = Jt;
-    args.term_row = c->rows.as<int>();
-    args.R = R;
-    args.mu = gi.mu; args.nu = gi.nu; args.pstride = 1;
-    args.y_batch = gi.yb; args.ystride = s->N;
-    args.out = c->out.as<double>();
-    return 0;
-}
-
 // n₀ = searchsortedfirst(t, τ) − 1 (celerite_solver.jl:395): the series lives on the device, fetch its times once
 static int prediction_gaps(pioran_ctx* c, const Series* s, int64_t M, const double* tau, std::vector<int>& n0) {
     std::vector<double> th(s->N);
@@ -2428,27 +2289,25 @@ static void launch_posterior_mean(pioran_ctx* c, const PostArgs& pa) {
 extern "C" int pioran_celerite_predict(pioran_ctx* c, int series_id, int B, int Jt, const double* a, const double* b,
                                        const double* cc, const double* d, const double* mu, const double* nu, int64_t M,
                                        const double* tau, double* mean_out) try {
-    if (is_group(c)) {   // single-device work of a group runs on its first device
-        int cid;
-        { std::lock_guard<std::mutex> lk(c->mu); const int rc = group_series_id(c, series_id, 0, &cid); if (rc) return rc; }
-        return pioran_celerite_predict(c->children[0], cid, B, Jt, a, b, cc, d, mu, nu, M, tau, mean_out);
-    }
+    if (is_group(c))
+        return group_first(c, series_id, [&](pioran_ctx* ch, int id) { return pioran_celerite_predict(ch, id, B, Jt, a, b, cc, d, mu, nu, M, tau, mean_out); });
     if (!c || !a || !b || !cc || !d || !tau || !mean_out) return fail(PIORAN_EINVAL, "NULL argument");
     if (B < 1 || Jt < 1 || M < 1) return fail(PIORAN_EINVAL, "B, Jt and M must be >= 1");
     for (int64_t m = 1; m < M; m++)
         if (!(tau[m] >= tau[m - 1])) return fail(PIORAN_EINVAL, "tau must be ascending (tau[%lld] < tau[%lld])", (long long)m, (long long)m - 1);
     PIORAN_COMPUTE_LOCK(c);
-    CUDA_TRY(cudaSetDevice(c->device));
-    Series* s = get_series(c, series_id);
-    if (!s) return fail(PIORAN_EINVAL, "unknown series id %d", series_id);
+    ExplicitSet x;
+    int rc, nitems, tpi;
+    if ((rc = explicit_front(c, series_id, B, Jt, b, d, 128, POSTERIOR_LIMIT, x))) return rc;
+    Series* s = x.s;
     const int64_t N = s->N;
-    int rc, BS, nitems;
     std::vector<int> n0;
     if ((rc = prediction_gaps(c, s, M, tau, n0))) return rc;
     GenericInputs gi;
     BatchArgs args;
-    if ((rc = generic_setup(c, s, B, Jt, a, b, cc, d, mu, nu, nullptr, gi, args, BS, nitems))) return rc;
-    const int RPL = stored_factor_ld(args.R);
+    if ((rc = upload_generic(c, B, Jt, N, a, b, cc, d, mu, nu, nullptr, nullptr, gi))) return rc;
+    if ((rc = generic_setup(c, s, B, Jt, x.term_row, x.R, gi, args, nitems, tpi))) return rc;
+    const int BS = bs_for_rank(x.R), RPL = stored_factor_ld(x.R);
     // workspace: W [B·N·RPL] | D [B·N] | z [B·N] | mean [B·M] | tau [M] | n0 [M ints]
     const size_t nW = (size_t)B * N * RPL, nBN = (size_t)B * N, nBM = (size_t)B * M;
     if ((rc = c->post.ensure(sizeof(double) * (nW + 2 * nBN + nBM + M) + sizeof(int) * (M + 2)))) return rc;
@@ -2479,22 +2338,20 @@ extern "C" int pioran_celerite_predict(pioran_ctx* c, int series_id, int B, int 
 extern "C" int pioran_celerite_simulate(pioran_ctx* c, int series_id, int B, int Jt, const double* a, const double* b,
                                         const double* cc, const double* d, const double* nu, const double* q,
                                         double* y_out) try {
-    if (is_group(c)) {   // single-device work of a group runs on its first device
-        int cid;
-        { std::lock_guard<std::mutex> lk(c->mu); const int rc = group_series_id(c, series_id, 0, &cid); if (rc) return rc; }
-        return pioran_celerite_simulate(c->children[0], cid, B, Jt, a, b, cc, d, nu, q, y_out);
-    }
+    if (is_group(c))
+        return group_first(c, series_id, [&](pioran_ctx* ch, int id) { return pioran_celerite_simulate(ch, id, B, Jt, a, b, cc, d, nu, q, y_out); });
     if (!c || !a || !b || !cc || !d || !q || !y_out) return fail(PIORAN_EINVAL, "NULL argument");
     if (B < 1 || Jt < 1) return fail(PIORAN_EINVAL, "B and Jt must be >= 1");
     PIORAN_COMPUTE_LOCK(c);
-    CUDA_TRY(cudaSetDevice(c->device));
-    Series* s = get_series(c, series_id);
-    if (!s) return fail(PIORAN_EINVAL, "unknown series id %d", series_id);
-    int rc, BS, nitems;
+    ExplicitSet x;
+    int rc, nitems, tpi;
+    if ((rc = explicit_front(c, series_id, B, Jt, b, d, 128, POSTERIOR_LIMIT, x))) return rc;
     GenericInputs gi;
     BatchArgs args;
-    if ((rc = generic_setup(c, s, B, Jt, a, b, cc, d, nullptr, nu, q, gi, args, BS, nitems))) return rc;
-    const size_t nBN = (size_t)B * s->N;
+    if ((rc = upload_generic(c, B, Jt, x.s->N, a, b, cc, d, nullptr, nu, q, nullptr, gi))) return rc;
+    if ((rc = generic_setup(c, x.s, B, Jt, x.term_row, x.R, gi, args, nitems, tpi))) return rc;
+    const int BS = bs_for_rank(x.R);
+    const size_t nBN = (size_t)B * x.s->N;
     if ((rc = c->post.ensure(sizeof(double) * nBN))) return rc;
     args.ysim_out = c->post.as<double>();
     cudaEventRecord(c->ev_beg, c->stream);
@@ -2510,17 +2367,8 @@ extern "C" int pioran_celerite_simulate(pioran_ctx* c, int series_id, int B, int
 // ------------------------------------------------------------------------------------------------ posterior variance (K6)
 static int launch_postvar(pioran_ctx* c, const PostVarArgs& pv, int B) {
     const int TS = (pv.R + 15) / 16;
-    switch (TS) {
-        case 1: celerite_postvar_kernel<1><<<B, WIDE_THREADS, 0, c->stream>>>(pv); break;
-        case 2: celerite_postvar_kernel<2><<<B, WIDE_THREADS, 0, c->stream>>>(pv); break;
-        case 3: celerite_postvar_kernel<3><<<B, WIDE_THREADS, 0, c->stream>>>(pv); break;
-        case 4: celerite_postvar_kernel<4><<<B, WIDE_THREADS, 0, c->stream>>>(pv); break;
-        case 5: celerite_postvar_kernel<5><<<B, WIDE_THREADS, 0, c->stream>>>(pv); break;
-        case 6: celerite_postvar_kernel<6><<<B, WIDE_THREADS, 0, c->stream>>>(pv); break;
-        case 7: celerite_postvar_kernel<7><<<B, WIDE_THREADS, 0, c->stream>>>(pv); break;
-        case 8: celerite_postvar_kernel<8><<<B, WIDE_THREADS, 0, c->stream>>>(pv); break;
-        default: return fail(PIORAN_EUNSUPPORTED, "rank %d exceeds the limit of 128 of the posterior variance", pv.R);
-    }
+    int rc;
+    if ((rc = with_int<1, 8>(TS, [&](auto ts) { celerite_postvar_kernel<ts><<<B, WIDE_THREADS, 0, c->stream>>>(pv); return 0; }))) return rc;
     c->launches++;
     note_kernel(c, KF_POSTVAR, TS);
     CUDA_TRY(cudaGetLastError());
@@ -2530,32 +2378,29 @@ static int launch_postvar(pioran_ctx* c, const PostVarArgs& pv, int B) {
 extern "C" int pioran_celerite_predict_var(pioran_ctx* c, int series_id, int B, int Jt, const double* a, const double* b,
                                            const double* cc, const double* d, const double* mu, const double* nu, int64_t M,
                                            const double* tau, double* mean_out, double* var_out) try {
-    if (is_group(c)) {   // single-device work of a group runs on its first device
-        int cid;
-        { std::lock_guard<std::mutex> lk(c->mu); const int rc = group_series_id(c, series_id, 0, &cid); if (rc) return rc; }
-        return pioran_celerite_predict_var(c->children[0], cid, B, Jt, a, b, cc, d, mu, nu, M, tau, mean_out, var_out);
-    }
+    if (is_group(c))
+        return group_first(c, series_id, [&](pioran_ctx* ch, int id) {
+            return pioran_celerite_predict_var(ch, id, B, Jt, a, b, cc, d, mu, nu, M, tau, mean_out, var_out);
+        });
     if (!c || !a || !b || !cc || !d || !tau || !var_out) return fail(PIORAN_EINVAL, "NULL argument");
     if (B < 1 || Jt < 1 || M < 1) return fail(PIORAN_EINVAL, "B, Jt and M must be >= 1");
     for (int64_t m = 1; m < M; m++)
         if (!(tau[m] >= tau[m - 1])) return fail(PIORAN_EINVAL, "tau must be ascending (tau[%lld] < tau[%lld])", (long long)m, (long long)m - 1);
     PIORAN_COMPUTE_LOCK(c);
-    CUDA_TRY(cudaSetDevice(c->device));
-    Series* s = get_series(c, series_id);
-    if (!s) return fail(PIORAN_EINVAL, "unknown series id %d", series_id);
-    std::vector<int> term_row;
-    const int R = make_term_rows(B, Jt, b, d, term_row);   // the map of the whole batch, shared by every θ-chunk
-    if (R > 128 || Jt > 128)
-        return fail(PIORAN_EUNSUPPORTED, "rank %d (Jt = %d) exceeds the limit of 128 of the posterior variance", R, Jt);
-    const int64_t N = s->N;
+    ExplicitSet x;   // the row map of the whole batch, shared by every θ-chunk
     int rc;
+    if ((rc = explicit_front(c, series_id, B, Jt, b, d, 128, "rank %1$d (Jt = %2$d) exceeds the limit of %3$d of the posterior variance", x)))
+        return rc;
+    Series* s = x.s;
+    const int R = x.R;
+    const int64_t N = s->N;
     std::vector<int> n0;
     if ((rc = prediction_gaps(c, s, M, tau, n0))) return rc;
 
     // θ-chunks of at most 1 GiB: per set W [N·RPL] | D [N] | z [N] | mean [M] | g_τ, D_τ [M·(R + 1)] | var [M]
     const int RPL = stored_factor_ld(R);
     const size_t per_set = sizeof(double) * ((size_t)N * RPL + 2 * (size_t)N + (size_t)M * (R + 3));
-    const int Bc = (int)std::max<size_t>(1, std::min<size_t>((size_t)B, ((size_t)1 << 30) / per_set));
+    const int Bc = theta_chunk(B, per_set);
     if ((rc = c->post.ensure(per_set * Bc + sizeof(double) * M + sizeof(int) * (M + 2)))) return rc;
     double* W = c->post.as<double>();
     double* D = W + (size_t)Bc * N * RPL;
@@ -2571,11 +2416,12 @@ extern "C" int pioran_celerite_predict_var(pioran_ctx* c, int series_id, int B, 
     for (int b0 = 0; b0 < B; b0 += Bc) {
         const int Bk = std::min(Bc, B - b0);
         const size_t o = (size_t)b0 * Jt;
-        int BS, nitems;
+        int nitems, tpi;
         GenericInputs gi;
         BatchArgs args;
-        if ((rc = generic_setup(c, s, Bk, Jt, a + o, b + o, cc + o, d + o, mu ? mu + b0 : nullptr, nu ? nu + b0 : nullptr,
-                                nullptr, gi, args, BS, nitems, &term_row))) return rc;
+        if ((rc = upload_generic(c, Bk, Jt, N, a + o, b + o, cc + o, d + o, at(mu, b0), at(nu, b0), nullptr, nullptr, gi))) return rc;
+        if ((rc = generic_setup(c, s, Bk, Jt, x.term_row, R, gi, args, nitems, tpi))) return rc;
+        const int BS = bs_for_rank(R);
         args.W_out = W; args.D_out = D; args.zf_out = z;
         // the factor of pioran_celerite_predict, and its backsolve and predict kernels: mean_out is predict's, bit for bit
         if ((rc = BS > 8 ? launch_wide<STEP_STORE>(c, args, nitems) : dispatch_generic_mode<STEP_STORE>(c, BS, args, nitems))) return rc;
@@ -2617,10 +2463,7 @@ static int make_term_rows(int B, int Jt, const double* b, const double* d, std::
 }
 
 extern "C" int pioran_ctx_set_auto_scan(pioran_ctx* c, int enabled) try {
-    if (is_group(c)) {
-        for (pioran_ctx* ch : c->children) { const int rc = pioran_ctx_set_auto_scan(ch, enabled); if (rc) return rc; }
-        return PIORAN_OK;
-    }
+    if (is_group(c)) return group_each(c, [&](pioran_ctx* ch) { return pioran_ctx_set_auto_scan(ch, enabled); });
     if (!c) return fail(PIORAN_EINVAL, "ctx is NULL");
     std::lock_guard<std::mutex> lk(c->mu);
     c->auto_scan = enabled != 0;
@@ -2628,10 +2471,7 @@ extern "C" int pioran_ctx_set_auto_scan(pioran_ctx* c, int enabled) try {
 } catch (...) { return guard_fail(); }
 
 extern "C" int pioran_ctx_set_sweep_kernel(pioran_ctx* c, int which) try {
-    if (is_group(c)) {
-        for (pioran_ctx* ch : c->children) { const int rc = pioran_ctx_set_sweep_kernel(ch, which); if (rc) return rc; }
-        return PIORAN_OK;
-    }
+    if (is_group(c)) return group_each(c, [&](pioran_ctx* ch) { return pioran_ctx_set_sweep_kernel(ch, which); });
     if (!c) return fail(PIORAN_EINVAL, "ctx is NULL");
     if (which != PIORAN_SWEEP_AUTO && which != PIORAN_SWEEP_SCALAR) return fail(PIORAN_EINVAL, "unknown sweep kernel %d", which);
     std::lock_guard<std::mutex> lk(c->mu);
@@ -2640,10 +2480,7 @@ extern "C" int pioran_ctx_set_sweep_kernel(pioran_ctx* c, int which) try {
 } catch (...) { return guard_fail(); }
 
 extern "C" int pioran_ctx_set_scan_tolerance(pioran_ctx* c, double tol) try {
-    if (is_group(c)) {
-        for (pioran_ctx* ch : c->children) { const int rc = pioran_ctx_set_scan_tolerance(ch, tol); if (rc) return rc; }
-        return PIORAN_OK;
-    }
+    if (is_group(c)) return group_each(c, [&](pioran_ctx* ch) { return pioran_ctx_set_scan_tolerance(ch, tol); });
     if (!c) return fail(PIORAN_EINVAL, "ctx is NULL");
     if (tol != tol) return fail(PIORAN_EINVAL, "tol is NaN");
     std::lock_guard<std::mutex> lk(c->mu);
@@ -2660,10 +2497,7 @@ extern "C" int pioran_ctx_last_scan_check(pioran_ctx* c, double* estimate, int* 
     return PIORAN_OK;
 } catch (...) { return guard_fail(); }
 extern "C" int pioran_ctx_set_scan_floor_cap(pioran_ctx* c, double cap) try {
-    if (is_group(c)) {
-        for (pioran_ctx* ch : c->children) { const int rc = pioran_ctx_set_scan_floor_cap(ch, cap); if (rc) return rc; }
-        return PIORAN_OK;
-    }
+    if (is_group(c)) return group_each(c, [&](pioran_ctx* ch) { return pioran_ctx_set_scan_floor_cap(ch, cap); });
     if (!c) return fail(PIORAN_EINVAL, "ctx is NULL");
     if (!(cap == cap)) return fail(PIORAN_EINVAL, "cap is NaN");
     std::lock_guard<std::mutex> lk(c->mu);
@@ -2688,10 +2522,7 @@ extern "C" int pioran_ctx_last_scan_history(pioran_ctx* c, int index, int max_pa
     return PIORAN_OK;
 } catch (...) { return guard_fail(); }
 extern "C" int pioran_ctx_set_scan_chunks(pioran_ctx* c, int chunks) try {
-    if (is_group(c)) {
-        for (pioran_ctx* ch : c->children) { const int rc = pioran_ctx_set_scan_chunks(ch, chunks); if (rc) return rc; }
-        return PIORAN_OK;
-    }
+    if (is_group(c)) return group_each(c, [&](pioran_ctx* ch) { return pioran_ctx_set_scan_chunks(ch, chunks); });
     if (!c) return fail(PIORAN_EINVAL, "ctx is NULL");
     if (chunks < 0) return fail(PIORAN_EINVAL, "chunks must be >= 0 (0 = automatic)");
     std::lock_guard<std::mutex> lk(c->mu);
@@ -3249,7 +3080,9 @@ static int scan_logl_locked(pioran_ctx* c, Series* s, int series_id, int B, int 
                 std::copy(d + i * Jt, d + (i + 1) * Jt, rd.begin() + k * Jt);
                 rmu[k] = mu ? mu[i] : 0.0; rnu[k] = nu ? nu[i] : 1.0;
             }
-            if ((rc = generic_logl_locked(c, s, (int)nr, Jt, ra.data(), rb.data(), rcc.data(), rd.data(), rmu.data(), rnu.data(),
+            ExplicitSet x;
+            if ((rc = explicit_front(c, series_id, (int)nr, Jt, rb.data(), rd.data(), WIDE_MAX_RANK, LOGL_LIMIT, x)) ||
+                (rc = generic_logl_locked(c, x, (int)nr, Jt, ra.data(), rb.data(), rcc.data(), rd.data(), rmu.data(), rnu.data(),
                                           nullptr, nullptr, rout.data())))
                 return rc;
             for (size_t k = 0; k < nr; k++) logl_out[redo[k]] = rout[k];
@@ -3262,11 +3095,8 @@ static int scan_logl_locked(pioran_ctx* c, Series* s, int series_id, int B, int 
 extern "C" int pioran_celerite_logl_scan(pioran_ctx* c, int series_id, int B, int Jt, const double* a, const double* b,
                                          const double* cc, const double* d, const double* mu, const double* nu,
                                          double* logl_out) try {
-    if (is_group(c)) {   // single-device work of a group runs on its first device
-        int cid;
-        { std::lock_guard<std::mutex> lk(c->mu); const int rc = group_series_id(c, series_id, 0, &cid); if (rc) return rc; }
-        return pioran_celerite_logl_scan(c->children[0], cid, B, Jt, a, b, cc, d, mu, nu, logl_out);
-    }
+    if (is_group(c))
+        return group_first(c, series_id, [&](pioran_ctx* ch, int id) { return pioran_celerite_logl_scan(ch, id, B, Jt, a, b, cc, d, mu, nu, logl_out); });
     if (!c || !a || !b || !cc || !d || !logl_out) return fail(PIORAN_EINVAL, "NULL argument");
     if (B < 1 || Jt < 1) return fail(PIORAN_EINVAL, "B and Jt must be >= 1");
     PIORAN_COMPUTE_LOCK(c);
@@ -3283,11 +3113,10 @@ extern "C" int pioran_scan_composite_doubles(void) { return SEL; }
 extern "C" int pioran_celerite_scan_range_begin(pioran_ctx* c, int series_id, int Jt, const double* a, const double* b,
                                                 const double* cc, const double* d, const double* mu, const double* nu,
                                                 int64_t n_lo, int64_t n_hi, int max_prev, double* composite_out) try {
-    if (is_group(c)) {   // single-device work of a group runs on its first device
-        int cid;
-        { std::lock_guard<std::mutex> lk(c->mu); const int rc = group_series_id(c, series_id, 0, &cid); if (rc) return rc; }
-        return pioran_celerite_scan_range_begin(c->children[0], cid, Jt, a, b, cc, d, mu, nu, n_lo, n_hi, max_prev, composite_out);
-    }
+    if (is_group(c))
+        return group_first(c, series_id, [&](pioran_ctx* ch, int id) {
+            return pioran_celerite_scan_range_begin(ch, id, Jt, a, b, cc, d, mu, nu, n_lo, n_hi, max_prev, composite_out);
+        });
     if (!c || !a || !b || !cc || !d || !composite_out) return fail(PIORAN_EINVAL, "NULL argument");
     PIORAN_COMPUTE_LOCK(c);
     CUDA_TRY(cudaSetDevice(c->device));
@@ -3371,15 +3200,11 @@ extern "C" int pioran_direct_logl(pioran_ctx* c, int series_id, int B, int Jt, c
                                   double* nll_out, int* info_out) try {
     if (!c || !a || !b || !cc || !d || !nll_out) return fail(PIORAN_EINVAL, "NULL argument");
     if (B < 1 || Jt < 1) return fail(PIORAN_EINVAL, "B and Jt must be >= 1");
-    if (is_group(c)) {   // the parameter vectors are independent: contiguous slices, one per device
-        std::vector<int> cid(c->children.size());
-        { std::lock_guard<std::mutex> lk(c->mu); for (size_t k = 0; k < cid.size(); k++) { const int rc = group_series_id(c, series_id, k, &cid[k]); if (rc) return rc; } }
-        return group_split(c, B, [&](int k, int beg, int nb) -> int {
+    if (is_group(c))   // the parameter vectors are independent: contiguous slices, one per device
+        return group_fanout(c, series_id, B, [&](pioran_ctx* ch, int id, int64_t, int beg, int nb) {
             const size_t o = (size_t)beg * Jt;
-            return pioran_direct_logl(c->children[k], cid[k], nb, Jt, a + o, b + o, cc + o, d + o, mu ? mu + beg : nullptr,
-                                      nu ? nu + beg : nullptr, nll_out + beg, info_out ? info_out + beg : nullptr);
+            return pioran_direct_logl(ch, id, nb, Jt, a + o, b + o, cc + o, d + o, at(mu, beg), at(nu, beg), nll_out + beg, at(info_out, beg));
         });
-    }
     PIORAN_COMPUTE_LOCK(c);
     CUDA_TRY(cudaSetDevice(c->device));
     Series* s = get_series(c, series_id);
@@ -3442,20 +3267,21 @@ extern "C" int pioran_direct_logl(pioran_ctx* c, int series_id, int B, int Jt, c
         // the first group's block columns are filled first: its panel chain (nothing else could run beside it) then overlaps the
         // fill of the rest (PIORAN_K4_FILL_SPLIT=0: one launch)
         static const bool fill_split = [] { const char* e = getenv("PIORAN_K4_FILL_SPLIT"); return !(e && !strcmp(e, "0")); }();
-        static const int Gf = [] { const char* e = getenv("PIORAN_K4_GROUP"); const int g = e ? atoi(e) : 4; return g >= 1 && g <= 8 ? g : 4; }();
-        const bool split = fill_split && nblk > 2 * Gf;
+        // PIORAN_K4_GROUP: panels per group of the factorisation below (1 … 8, default 4)
+        static const int G = [] { const char* e = getenv("PIORAN_K4_GROUP"); const int g = e ? atoi(e) : 4; return g >= 1 && g <= 8 ? g : 4; }();
+        const bool split = fill_split && nblk > 2 * G;
         const int fdir = fill_direct || !fill_tables;
         if (split) {
-            const int mt = nblk - Gf;
-            dense_fill_kernel<<<dim3(nblk * Gf, nb), 256, fill_smem, c->stream>>>(A, ld, N, s->t, s->y, s->s2, Jt, gi.a, gi.b, gi.c,
-                                                                                  gi.d, gi.mu, gi.nu, th0, tab, nfull, fdir, 1, Gf);
+            const int mt = nblk - G;
+            dense_fill_kernel<<<dim3(nblk * G, nb), 256, fill_smem, c->stream>>>(A, ld, N, s->t, s->y, s->s2, Jt, gi.a, gi.b, gi.c,
+                                                                                 gi.d, gi.mu, gi.nu, th0, tab, nfull, fdir, 1, G);
             CUDA_TRY(cudaEventRecord(c->ev_join, c->stream));
             dense_fill_kernel<<<dim3(mt * (mt + 1) / 2, nb), 256, fill_smem, c->stream>>>(A, ld, N, s->t, s->y, s->s2, Jt, gi.a, gi.b, gi.c,
-                                                                                         gi.d, gi.mu, gi.nu, th0, tab, nfull, fdir, 2, Gf);
+                                                                                         gi.d, gi.mu, gi.nu, th0, tab, nfull, fdir, 2, G);
             c->launches += 2;
         } else {
             dense_fill_kernel<<<dim3(ntri, nb), 256, fill_smem, c->stream>>>(A, ld, N, s->t, s->y, s->s2, Jt, gi.a, gi.b, gi.c,
-                                                                             gi.d, gi.mu, gi.nu, th0, tab, nfull, fdir, 0, Gf);
+                                                                             gi.d, gi.mu, gi.nu, th0, tab, nfull, fdir, 0, G);
             c->launches++;
             CUDA_TRY(cudaEventRecord(c->ev_join, c->stream));
         }
@@ -3474,7 +3300,6 @@ extern "C" int pioran_direct_logl(pioran_ctx* c, int series_id, int B, int Jt, c
         };
         bool bulk_pending = false;
         CUDA_TRY(cudaStreamWaitEvent(S1, c->ev_join, 0));      // the fill of the first group's columns (and everything before it) precedes the chain
-        static const int G = [] { const char* e = getenv("PIORAN_K4_GROUP"); const int g = e ? atoi(e) : 4; return g >= 1 && g <= 8 ? g : 4; }();
         // PIORAN_K4_GROUP0: size of the FIRST group (default: G).  Nothing runs beside its chain, so a shorter first group hands
         // the side stream its first bulk earlier — measured: 8.92 (4) / 8.98 (3) / 9.02 (2) / 9.14 ms (1); the shorter bulk then
         // ends before the second group's chain does.
