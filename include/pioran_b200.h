@@ -348,6 +348,22 @@ int pioran_celerite_predict_var(pioran_ctx *ctx, int series_id, int B, int Jt,
                                 const double *a, const double *b, const double *c, const double *d,
                                 const double *mu, const double *nu, int64_t M, const double *tau,
                                 double *mean_out, double *var_out);
+/* Posterior draws (K7): for each of the B coefficient sets, S draws of  rand(fp(τ, sigma2_tau))  for the posterior
+ * fp = posterior(f(t, nu_i σ²), ỹ_i) — the latent f at the M ascending points tau conditioned on the data, plus independent
+ * noise of variance sigma2_tau (AbstractGPs' σ² of fp(τ, σ²); 1e-18 is its default).  ỹ_i is the resident y, or row i of
+ * y_batch [B × N] when given.  Matheron's rule on the merged grid G of t and τ (a data point first at a tie): a prior draw
+ * u = L^G √D^G q on G, then draw = mu_i + u(τ) + K(τ, t) K̃⁻¹ (ỹ − mu_i − u(t)).  q [B × S × (N + M)] holds standard normals
+ * in merged-grid order (the caller's, as for pioran_celerite_simulate); draws_out is [B × S × M].  For the same q this is
+ * not the draw a dense Cholesky of the posterior covariance gives; its distribution is the same.  O((N + M)·R²) per set
+ * for the two factors, O((N + M)·R) per draw; ranks up to 128 (PIORAN_EUNSUPPORTED above).  PIORAN_EINVAL for NULL
+ * pointers, B, Jt, M or S < 1, descending tau, sigma2_tau < 0 or NaN, and repeated tau with sigma2_tau == 0 (the merged
+ * covariance is then singular).  A set with a pivot <= 0 in either factor gets NaN in all of its S·M draws.  A device
+ * group splits the sets over its devices. */
+int pioran_celerite_posterior_draws(pioran_ctx *ctx, int series_id, int B, int Jt,
+                                    const double *a, const double *b, const double *c, const double *d,
+                                    const double *mu, const double *nu, const double *y_batch,
+                                    int64_t M, const double *tau, double sigma2_tau,
+                                    int S, const double *q, double *draws_out);
 
 #ifdef __cplusplus
 }

@@ -304,6 +304,32 @@ function predict_var_b200(a, b, c, d, τ, t, y, σ2)
     return μ, v
 end
 
+"""
+    posterior_draws_b200(a, b, c, d, τ, t, y, σ2, q; σ2τ = 1e-18) -> Matrix (M × n)
+
+Draws of the posterior fp(τ, σ2τ) of the zero-mean GP conditioned on (t, y, σ2), by Matheron's rule (K7): q is
+`randn(rng, N + M, n)`, standard normals in the order of the merged grid of t and τ (a data point first at a tie).  O((N + M)·R)
+per draw after two O((N + M)·R²) factorisations.  For the same q the draws differ from those of a dense Cholesky of
+cov(fp, τ); their distribution is the same.  Ranks up to 128.  Not run here: no Julia toolchain.
+"""
+function posterior_draws_b200(a, b, c, d, τ, t, y, σ2, q; σ2τ = 1e-18)
+    N, M = length(t), length(τ)
+    size(q, 1) == N + M || throw(DimensionMismatch("q must have N + M = $(N + M) rows"))
+    S = size(q, 2)
+    s = b200_upload(collect(Float64, t), collect(Float64, y), collect(Float64, σ2))
+    out = Matrix{Float64}(undef, M, S)   # column-major M × S is the row-major [S × M] of the C ABI
+    try
+        _b200_check(ccall((:pioran_celerite_posterior_draws, libpioran_b200), Cint,
+            (Ptr{Cvoid}, Cint, Cint, Cint, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64},
+             Ptr{Float64}, Int64, Ptr{Float64}, Float64, Cint, Ptr{Float64}, Ptr{Float64}),
+            b200_context().h, s.id, 1, length(a), Vector{Float64}(a), Vector{Float64}(b), Vector{Float64}(c), Vector{Float64}(d),
+            C_NULL, C_NULL, C_NULL, M, collect(Float64, τ), Float64(σ2τ), S, Matrix{Float64}(q), out))
+    finally
+        b200_free(s)
+    end
+    return out
+end
+
 "Drop-in for sim(rng, a, b, c, d, τ, σ2) (src/celerite_solver.jl:515-549): the draw q = randn(rng, N) is the reference's first line (:518)."
 function sim_b200(rng, a, b, c, d, τ, σ2)
     q = randn(rng, length(τ))

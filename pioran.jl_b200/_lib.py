@@ -73,6 +73,8 @@ SYMBOLS = {
     "pioran_celerite_simulate": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_int, _dp, _dp, _dp, _dp, _dp, _dp, _dp]),
     "pioran_celerite_predict_var": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_int, _dp, _dp, _dp, _dp, _dp, _dp, C.c_int64,
                                               _dp, _dp, _dp]),
+    "pioran_celerite_posterior_draws": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_int, _dp, _dp, _dp, _dp, _dp, _dp, _dp,
+                                                  C.c_int64, _dp, C.c_double, C.c_int, _dp, _dp]),
 }
 
 _lib = None

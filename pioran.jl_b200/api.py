@@ -494,6 +494,17 @@ class PosteriorGP:
             raise TypeError("posterior expects ScalableGP(...)(t, σ²)")
         self.f, self.y = fx, np.asarray(y, dtype=np.float64)
 
+    def __call__(self, τ, σ2=1e-18):
+        """fp(τ, σ²): the posterior at ascending τ plus independent noise of variance σ² (AbstractGPs' default 1e-18)."""
+        return FinitePosteriorGP(self, np.asarray(τ, dtype=np.float64), float(σ2))
+
+
+class FinitePosteriorGP:
+    """fp(τ, σ²) of a posterior: what rand draws from (posterior draws K7)."""
+
+    def __init__(self, fp, τ, σ2):
+        self.fp, self.x, self.σ2 = fp, τ, σ2
+
 
 def posterior(fx, y):
     return PosteriorGP(fx, y)
@@ -577,9 +588,39 @@ def simulate(cov, τ, σ2, q, *, ctx=None):
         ser.free()
 
 
+def posterior_draws(fpx, q, *, ctx=None):
+    """rand(rng, fp(τ, σ²), n) for fpx = posterior(f(t, σ²), y)(τ, σ²): draws of the latent f at τ conditioned on the data,
+    plus noise of variance σ², by Matheron's rule (a prior draw on the merged grid of t and τ, corrected by the posterior
+    mean of its residual at the data).  q [N + M] or [S, N + M] holds standard normals in merged-grid order (a data point
+    first at a tie); the result is [M] or [S, M].  The mean function is handled as in mean: the draws are made for y − m(t)
+    and m(τ) is added.  For the same q the draws differ from those of a dense Cholesky of cov(fp, τ); their distribution
+    is the same."""
+    fp = fpx.fp
+    fx = fp.f
+    τ = fpx.x
+    q = np.asarray(q, dtype=np.float64)
+    one = q.ndim == 1
+    ctx = ctx or get_context()
+    a, b, c, d = celerite_coefs(fx.f.kernel)
+    m = fx.f.mean
+    mτ = m(τ) if callable(m) else np.full(τ.shape, float(m))
+    ser = ctx.upload_series(fx.x, fp.y - fx.mean_vector(), fx.σ2)
+    try:
+        out = ctx.celerite_posterior_draws(ser, a, b, c, d, τ, q.reshape(1, -1, q.shape[-1]), sigma2_tau=fpx.σ2)[0]
+    finally:
+        ser.free()
+    out += mτ
+    return out[0] if one else out
+
+
 def rand(fx, q, t=None, *, ctx=None):
     """rand(rng, f(t, σ²)[, t'])  (src/scalable_GP.jl:133-155): one realisation on the GP's own times with its noise
-    variances, or on other times t' without noise; the mean function is added."""
+    variances, or on other times t' without noise; the mean function is added.  For fx = posterior(...)(τ, σ²), draws of
+    the posterior (posterior_draws)."""
+    if isinstance(fx, FinitePosteriorGP):
+        if t is not None:
+            raise TypeError("rand(fp(τ, σ²), q) takes no second time vector")
+        return posterior_draws(fx, q, ctx=ctx)
     if not isinstance(fx, FiniteScalableGP):
         raise TypeError("rand expects ScalableGP(...)(t, σ²)")
     m = fx.f.mean

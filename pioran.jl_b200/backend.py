@@ -474,6 +474,26 @@ class Context:
                                                 _p(out)))
         return out
 
+    def celerite_posterior_draws(self, series, a, b, c, d, tau, q, mu=None, nu=None, y_batch=None, sigma2_tau=1e-18):
+        """Draws [B × S × M] of rand(fp(τ, σ²_τ)) for the posterior of each coefficient set, by Matheron's rule on the merged
+        grid of t and τ (K7).  q [B × S × (N + M)] holds standard normals in merged-grid order (a data point first at a tie);
+        y_batch [B × N] replaces the resident y per set.  A set whose covariance is not positive definite gets NaN draws."""
+        a, b, c, d = (np.atleast_2d(_f64(x)) for x in (a, b, c, d))
+        B, Jt = a.shape
+        tau = _f64(tau)
+        M = tau.shape[0]
+        q = np.ascontiguousarray(q, dtype=np.float64)
+        if q.ndim != 3 or q.shape[0] != B or q.shape[2] != series.N + M:
+            raise ValueError(f"q must be [B, S, N + M] = [{B}, S, {series.N + M}], got {list(q.shape)}")
+        S = q.shape[1]
+        mu = _f64(mu, (B,)) if mu is not None else None
+        nu = _f64(nu, (B,)) if nu is not None else None
+        y_batch = _f64(y_batch, (B, series.N)) if y_batch is not None else None
+        out = np.empty((B, S, M))
+        check(self.lib.pioran_celerite_posterior_draws(self.h, series.id, B, Jt, _p(a), _p(b), _p(c), _p(d), _p(mu), _p(nu),
+                                                       _p(y_batch), M, _p(tau), float(sigma2_tau), S, _p(q), _p(out)))
+        return out
+
 
 _default = {}
 

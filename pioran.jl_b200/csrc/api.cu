@@ -23,6 +23,7 @@
 #include "scan.cuh"
 #include "posterior.cuh"
 #include "postvar.cuh"
+#include "postdraw.cuh"
 #include "table.cuh"
 #include "grad.cuh"
 #include "grad_pipe.cuh"
@@ -66,7 +67,7 @@ static int guard_fail() {
     } while (0)
 
 extern "C" const char* pioran_last_error(void) { return g_err.c_str(); }
-extern "C" int pioran_version(void) { return 303; }   // 0.3.3: pioran_celerite_predict_var
+extern "C" int pioran_version(void) { return 304; }   // 0.3.4: pioran_celerite_posterior_draws
 
 // ------------------------------------------------------------------------------------------------ context
 namespace {
@@ -106,7 +107,7 @@ using PlanKey = std::tuple<int, int, int, int, double, double, double, double>;
 enum KernelFamily : int {
     KF_NONE = 0, KF_BLOCKED, KF_BLOCKED_WIDE, KF_SHARED, KF_SHARED_PAIR, KF_GENERIC, KF_WIDE_REG, KF_WIDE_REG_STORE, KF_WIDE_REG_SIM,
     KF_WIDE, KF_BLOCKED_GRAD, KF_GRAD, KF_GRAD_PIPE, KF_WIDE_GRAD, KF_JVP, KF_PREDICT, KF_GENERIC_SIM, KF_SCAN_FINISH,
-    KF_SCAN_PARTIAL, KF_DENSE_FINISH, KF_VJP, KF_POSTVAR
+    KF_SCAN_PARTIAL, KF_DENSE_FINISH, KF_VJP, KF_POSTVAR, KF_POSTDRAW
 };
 struct KernelTag { int family = KF_NONE; int p[4] = {0, 0, 0, 0}; };
 
@@ -424,6 +425,7 @@ extern "C" int pioran_ctx_last_kernel_name(pioran_ctx* c, char* buf, int len) tr
         case KF_VJP: snprintf(name, sizeof name, "vjp<%d>", p[0]); break;
         case KF_PREDICT: snprintf(name, sizeof name, "predict<%d>", p[0]); break;
         case KF_POSTVAR: snprintf(name, sizeof name, "postvar<%d>", p[0]); break;
+        case KF_POSTDRAW: snprintf(name, sizeof name, "postdraw<%d>", p[0]); break;
         case KF_GENERIC_SIM: snprintf(name, sizeof name, "generic_sim<%d,%d>", p[0], p[1]); break;
         case KF_SCAN_FINISH: snprintf(name, sizeof name, "scan_finish"); break;
         case KF_SCAN_PARTIAL: snprintf(name, sizeof name, "scan_partial"); break;
@@ -2265,11 +2267,18 @@ extern "C" int pioran_ctx_set_vjp_workspace(pioran_ctx* c, long long bytes) try 
 } catch (...) { return guard_fail(); }
 
 // ------------------------------------------------------------------------------------------------ posterior mean, draws
-// n₀ = searchsortedfirst(t, τ) − 1 (celerite_solver.jl:395): the series lives on the device, fetch its times once
-static int prediction_gaps(pioran_ctx* c, const Series* s, int64_t M, const double* tau, std::vector<int>& n0) {
-    std::vector<double> th(s->N);
+// The times of a series live on the device: fetch them once per call.
+static int series_times(pioran_ctx* c, const Series* s, std::vector<double>& th) {
+    th.resize(s->N);
     CUDA_TRY(cudaMemcpyAsync(th.data(), s->t, sizeof(double) * s->N, cudaMemcpyDeviceToHost, c->stream));
     CUDA_TRY(cudaStreamSynchronize(c->stream));
+    return 0;
+}
+// n₀ = searchsortedfirst(t, τ) − 1 (celerite_solver.jl:395)
+static int prediction_gaps(pioran_ctx* c, const Series* s, int64_t M, const double* tau, std::vector<int>& n0) {
+    std::vector<double> th;
+    int rc;
+    if ((rc = series_times(c, s, th))) return rc;
     n0.resize(M);
     for (int64_t m = 0; m < M; m++) n0[m] = (int)(std::lower_bound(th.begin(), th.end(), tau[m]) - th.begin());
     return 0;
@@ -2444,6 +2453,115 @@ extern "C" int pioran_celerite_predict_var(pioran_ctx* c, int series_id, int B, 
     }
     cudaEventRecord(c->ev_end, c->stream);
     CUDA_TRY(cudaStreamSynchronize(c->stream));   // n0 is a local
+    return PIORAN_OK;
+} catch (...) { return guard_fail(); }
+
+// ------------------------------------------------------------------------------------------------ posterior draws (K7)
+extern "C" int pioran_celerite_posterior_draws(pioran_ctx* c, int series_id, int B, int Jt, const double* a, const double* b,
+                                               const double* cc, const double* d, const double* mu, const double* nu,
+                                               const double* y_batch, int64_t M, const double* tau, double sigma2_tau, int S,
+                                               const double* q, double* draws_out) try {
+    if (!c || !a || !b || !cc || !d || !tau || !q || !draws_out) return fail(PIORAN_EINVAL, "NULL argument");
+    if (B < 1 || Jt < 1 || M < 1 || S < 1) return fail(PIORAN_EINVAL, "B, Jt, M and S must be >= 1");
+    if (!(sigma2_tau >= 0.0)) return fail(PIORAN_EINVAL, "sigma2_tau must be >= 0 (got %g)", sigma2_tau);
+    for (int64_t m = 1; m < M; m++) {
+        if (!(tau[m] >= tau[m - 1])) return fail(PIORAN_EINVAL, "tau must be ascending (tau[%lld] < tau[%lld])", (long long)m, (long long)m - 1);
+        if (tau[m] == tau[m - 1] && sigma2_tau == 0.0)
+            return fail(PIORAN_EINVAL, "tau[%lld] repeats tau[%lld]: with sigma2_tau = 0 the merged covariance is singular", (long long)m, (long long)m - 1);
+    }
+    if (is_group(c))
+        return group_fanout(c, series_id, B, [&](pioran_ctx* ch, int id, int64_t N, int beg, int nb) {
+            const size_t o = (size_t)beg * Jt, NG = (size_t)N + M;
+            return pioran_celerite_posterior_draws(ch, id, nb, Jt, a + o, b + o, cc + o, d + o, at(mu, beg), at(nu, beg),
+                                                   at(y_batch, beg * N), M, tau, sigma2_tau, S, q + (size_t)beg * S * NG,
+                                                   draws_out + (size_t)beg * S * M);
+        });
+    PIORAN_COMPUTE_LOCK(c);
+    ExplicitSet x;   // the row map of the whole batch, shared by every θ-chunk
+    int rc;
+    if ((rc = explicit_front(c, series_id, B, Jt, b, d, 128, "rank %1$d (Jt = %2$d) exceeds the limit of %3$d of the posterior draws", x)))
+        return rc;
+    Series* s = x.s;
+    const int R = x.R;
+    const int64_t N = s->N, NG = N + M;
+    // merged grid: a data point first at a tie, the τ points in their order (θ-independent, built once per call)
+    std::vector<double> th, gt(NG);
+    std::vector<int> gcode(NG);
+    if ((rc = series_times(c, s, th))) return rc;
+    for (int64_t k = 0, n = 0, m = 0; k < NG; k++) {
+        const bool data = m == M || (n < N && th[n] <= tau[m]);
+        gt[k] = data ? th[n] : tau[m];
+        gcode[k] = data ? (int)n++ : -(int)(m++) - 1;
+    }
+
+    // θ-chunks of at most 1 GiB: per set W [N·RPL] | D, zf [N] | W^G [NG·RPL] | D^G, zf^G, noise [NG] | q [S·NG] | z [S·N] | draws [S·M]
+    const int RPL = stored_factor_ld(R);
+    const size_t per_set = sizeof(double) * ((size_t)N * RPL + 2 * (size_t)N + (size_t)NG * RPL + 3 * (size_t)NG +
+                                             (size_t)S * (NG + N + M));
+    const int Bc = theta_chunk(B, per_set);
+    if ((rc = c->post.ensure(per_set * Bc + sizeof(double) * 2 * NG + sizeof(int) * (NG + 2)))) return rc;
+    double* W = c->post.as<double>();
+    double* D = W + (size_t)Bc * N * RPL;
+    double* zf = D + (size_t)Bc * N;
+    double* WG = zf + (size_t)Bc * N;
+    double* DG = WG + (size_t)Bc * NG * RPL;
+    double* zfG = DG + (size_t)Bc * NG;
+    double* noise = zfG + (size_t)Bc * NG;
+    double* qd = noise + (size_t)Bc * NG;
+    double* z = qd + (size_t)Bc * S * NG;
+    double* draws = z + (size_t)Bc * S * N;
+    double* gt_dev = draws + (size_t)Bc * S * M;
+    double* gy_dev = gt_dev + NG;   // the merged series carries no data: its forward substitution is not read
+    int* gcode_dev = reinterpret_cast<int*>(gy_dev + NG);
+    CUDA_TRY(cudaMemcpyAsync(gt_dev, gt.data(), sizeof(double) * NG, cudaMemcpyHostToDevice, c->stream));
+    CUDA_TRY(cudaMemsetAsync(gy_dev, 0, sizeof(double) * NG, c->stream));
+    CUDA_TRY(cudaMemcpyAsync(gcode_dev, gcode.data(), sizeof(int) * NG, cudaMemcpyHostToDevice, c->stream));
+    Series merged;
+    merged.N = NG; merged.t = gt_dev; merged.y = gy_dev; merged.s2 = nullptr;
+    const int BS = bs_for_rank(R);
+    const int PT = R <= 32 ? 1 : R <= 64 ? 2 : 4;
+    const int warps = std::min(S, PD_MAXW);
+    cudaEventRecord(c->ev_beg, c->stream);
+    for (int b0 = 0; b0 < B; b0 += Bc) {
+        const int Bk = std::min(Bc, B - b0);
+        const size_t o = (size_t)b0 * Jt;
+        int nitems, tpi;
+        GenericInputs gi;
+        BatchArgs args;
+        if ((rc = upload_generic(c, Bk, Jt, N, a + o, b + o, cc + o, d + o, at(mu, b0), at(nu, b0), at(y_batch, (size_t)b0 * N),
+                                 nullptr, gi))) return rc;
+        // the factor of the data covariance (that of pioran_celerite_predict)
+        if ((rc = generic_setup(c, s, Bk, Jt, x.term_row, R, gi, args, nitems, tpi))) return rc;
+        args.W_out = W; args.D_out = D; args.zf_out = zf;
+        if ((rc = BS > 8 ? launch_wide<STEP_STORE>(c, args, nitems) : dispatch_generic_mode<STEP_STORE>(c, BS, args, nitems))) return rc;
+        // the factor of the merged covariance: the per-set noise comes in as σ² rows, ν = 1
+        const int64_t total = (int64_t)Bk * NG;
+        merged_noise_kernel<<<(int)std::min<int64_t>((total + 255) / 256, (int64_t)c->num_sms * 16), 256, 0, c->stream>>>(
+            gcode_dev, s->s2, gi.nu, sigma2_tau, NG, Bk, noise);
+        c->launches++;
+        CUDA_TRY(cudaGetLastError());
+        if ((rc = generic_setup(c, &merged, Bk, Jt, x.term_row, R, gi, args, nitems, tpi))) return rc;
+        args.mu = nullptr; args.nu = nullptr; args.y_batch = nullptr; args.s2_batch = noise;
+        args.W_out = WG; args.D_out = DG; args.zf_out = zfG;
+        if ((rc = BS > 8 ? launch_wide<STEP_STORE>(c, args, nitems) : dispatch_generic_mode<STEP_STORE>(c, BS, args, nitems))) return rc;
+        // the draws
+        CUDA_TRY(cudaMemcpyAsync(qd, q + (size_t)b0 * S * NG, sizeof(double) * (size_t)Bk * S * NG, cudaMemcpyHostToDevice, c->stream));
+        PostDrawArgs pd{};
+        pd.gt = gt_dev; pd.gcode = gcode_dev; pd.N = N; pd.M = M; pd.NG = NG;
+        pd.S = S; pd.Jt = Jt; pd.R = R; pd.RPL = RPL;
+        pd.a = gi.a; pd.b = gi.b; pd.c = gi.c; pd.d = gi.d; pd.term_row = c->rows.as<int>(); pd.mu = gi.mu;
+        pd.y = gi.yb ? gi.yb : s->y; pd.y_batch = gi.yb != nullptr;
+        pd.WG = WG; pd.DG = DG; pd.W = W; pd.D = D; pd.q = qd; pd.z = z; pd.out = draws;
+        const dim3 grid((S + warps - 1) / warps, Bk);
+        if ((rc = with_int<0, 2>(PT >> 1, [&](auto lp) { celerite_postdraw_kernel<1 << lp><<<grid, 32 * warps, 0, c->stream>>>(pd); return 0; })))
+            return rc;
+        c->launches++;
+        CUDA_TRY(cudaGetLastError());
+        CUDA_TRY(cudaMemcpyAsync(draws_out + (size_t)b0 * S * M, draws, sizeof(double) * (size_t)Bk * S * M, cudaMemcpyDeviceToHost, c->stream));
+    }
+    cudaEventRecord(c->ev_end, c->stream);
+    note_kernel(c, KF_POSTDRAW, PT);
+    CUDA_TRY(cudaStreamSynchronize(c->stream));   // gt and gcode are locals
     return PIORAN_OK;
 } catch (...) { return guard_fail(); }
 
