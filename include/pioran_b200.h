@@ -364,6 +364,23 @@ int pioran_celerite_posterior_draws(pioran_ctx *ctx, int series_id, int B, int J
                                     const double *mu, const double *nu, const double *y_batch,
                                     int64_t M, const double *tau, double sigma2_tau,
                                     int S, const double *q, double *draws_out);
+/* Posterior covariance (K8): for each of the B coefficient sets the full covariance of the latent f at the M ascending points
+ * tau,  cov_out[i][m][m'] = k_i(τ_m, τ_m') − k_i(τ_m, t)ᵀ (K_i(t, t) + diag(nu_i σ²))⁻¹ k_i(t, τ_m')  — predict_cov
+ * (src/direct_solver.jl:28-119) behind cov / mean_and_cov of a PosteriorGP, without measurement noise and independent of mu.
+ * cov_out is [B × M × M] row-major and exactly symmetric; its diagonal is pioran_celerite_predict_var's variance up to
+ * rounding.  O((N + M)·R² + M·(N + M)·R) per set from the factor of pioran_celerite_predict: K6 adds two vectors per point,
+ * then one walk per column over the merged grid of t and τ.  mean_out [B × M] (or NULL) is what pioran_celerite_predict
+ * returns for the same arguments, bit for bit.  Ranks up to 128 (PIORAN_EUNSUPPORTED above); arguments are checked as in
+ * pioran_celerite_predict_var.  A set whose factor has a pivot D_n <= 0 gets NaN in its whole matrix.  The device workspace
+ * and output of one step is at most 1 GiB (pioran_ctx_set_postcov_workspace): the sets are processed in θ-chunks, and a set
+ * whose matrix alone exceeds the cap in column ranges.  A device group splits the sets over its devices. */
+int pioran_celerite_predict_cov(pioran_ctx *ctx, int series_id, int B, int Jt,
+                                const double *a, const double *b, const double *c, const double *d,
+                                const double *mu, const double *nu, int64_t M, const double *tau,
+                                double *mean_out, double *cov_out);
+/* Cap in bytes of the device workspace plus output of one step of pioran_celerite_predict_cov (0 = 1 GiB, the default).
+ * The result does not depend on it; a small cap splits a batch into many θ-chunks, and a set into column ranges. */
+int pioran_ctx_set_postcov_workspace(pioran_ctx *ctx, long long bytes);
 
 #ifdef __cplusplus
 }

@@ -305,6 +305,31 @@ function predict_var_b200(a, b, c, d, τ, t, y, σ2)
 end
 
 """
+    predict_cov_b200(a, b, c, d, τ, t, y, σ2) -> (μ, C)
+
+Posterior mean (what `pred_b200` returns, bit for bit) and the M × M covariance of the latent f at ascending τ: `predict_cov`
+(src/direct_solver.jl:28-119) without measurement noise, in O((N + M)·R² + M·(N + M)·R) instead of O(N³).  C is exactly
+symmetric (so the row-major matrix of the C ABI reads as itself in Julia's column-major order).  Ranks up to 128.  Not run here:
+no Julia toolchain.
+"""
+function predict_cov_b200(a, b, c, d, τ, t, y, σ2)
+    s = b200_upload(collect(Float64, t), collect(Float64, y), collect(Float64, σ2))
+    M = length(τ)
+    μ = Vector{Float64}(undef, M)
+    C = Matrix{Float64}(undef, M, M)
+    try
+        _b200_check(ccall((:pioran_celerite_predict_cov, libpioran_b200), Cint,
+            (Ptr{Cvoid}, Cint, Cint, Cint, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64},
+             Int64, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}),
+            b200_context().h, s.id, 1, length(a), Vector{Float64}(a), Vector{Float64}(b), Vector{Float64}(c), Vector{Float64}(d),
+            C_NULL, C_NULL, M, collect(Float64, τ), μ, C))
+    finally
+        b200_free(s)
+    end
+    return μ, C
+end
+
+"""
     posterior_draws_b200(a, b, c, d, τ, t, y, σ2, q; σ2τ = 1e-18) -> Matrix (M × n)
 
 Draws of the posterior fp(τ, σ2τ) of the zero-mean GP conditioned on (t, y, σ2), by Matheron's rule (K7): q is

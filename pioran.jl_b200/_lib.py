@@ -75,6 +75,9 @@ SYMBOLS = {
                                               _dp, _dp, _dp]),
     "pioran_celerite_posterior_draws": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_int, _dp, _dp, _dp, _dp, _dp, _dp, _dp,
                                                   C.c_int64, _dp, C.c_double, C.c_int, _dp, _dp]),
+    "pioran_celerite_predict_cov": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_int, _dp, _dp, _dp, _dp, _dp, _dp, C.c_int64,
+                                              _dp, _dp, _dp]),
+    "pioran_ctx_set_postcov_workspace": (C.c_int, [C.c_void_p, C.c_longlong]),
 }
 
 _lib = None

@@ -487,7 +487,8 @@ def logpdf(fx, Y, *, ctx=None):
 # ----------------------------------------------------------------------------------------------- posterior, draws
 class PosteriorGP:
     """posterior(f(t, σ²), y)  (src/scalable_GP.jl:44-54): holds the finite GP and the data; mean(fp, τ) runs the batched
-    `pred` kernel (src/celerite_solver.jl:376-483), var / std / mean_and_var(fp, τ) the posterior-variance sweep K6."""
+    `pred` kernel (src/celerite_solver.jl:376-483), var / std / mean_and_var(fp, τ) the posterior-variance sweep K6,
+    cov / mean_and_cov(fp, τ) the posterior-covariance walk K8."""
 
     def __init__(self, fx, y):
         if not isinstance(fx, FiniteScalableGP):
@@ -573,6 +574,44 @@ def std(fp, τ=None, *, ctx=None):
     """std(fp[, τ]) = √max(var, 0): at a data point with a tiny σ² the exact variance is close to 0 and rounding can
     make the computed one slightly negative; it is clamped to 0 rather than turned into NaN."""
     return np.sqrt(np.maximum(var(fp, τ, ctx=ctx), 0.0))
+
+
+def predict_cov(cov, τ, t, σ2, y=None, *, ctx=None):
+    """predict_cov(cov, τ, t, y, σ²)  (src/direct_solver.jl:28-119): the M × M posterior covariance of the zero-mean GP's
+    latent f at ascending τ, without measurement noise, exactly symmetric; O((N + M)·R² + M·(N + M)·R) instead of the dense
+    O(N³).  With y, (mean, cov)."""
+    ctx = ctx or get_context()
+    a, b, c, d = celerite_coefs(cov)
+    τ = np.asarray(τ, dtype=np.float64)
+    ser = ctx.upload_series(t, np.zeros_like(t) if y is None else y, σ2)
+    try:
+        out = ctx.celerite_predict_cov(ser, a, b, c, d, τ, return_mean=y is not None)
+    finally:
+        ser.free()
+    return (out[0][0], out[1][0]) if y is not None else out[0]
+
+
+def mean_and_cov(fp, τ=None, *, ctx=None):
+    """mean_and_cov(fp[, τ])  (AbstractGPs): posterior mean and the covariance of the latent f at τ (default: the data
+    times), from one factorisation.  The mean function shifts the mean only."""
+    if not isinstance(fp, PosteriorGP):
+        raise TypeError("mean_and_cov expects posterior(f(t, σ²), y)")
+    fx = fp.f
+    τ = fx.x if τ is None else np.asarray(τ, dtype=np.float64)
+    m = fx.f.mean
+    mτ = m(τ) if callable(m) else np.full(τ.shape, float(m))
+    mu, C = predict_cov(fx.f.kernel, τ, fx.x, fx.σ2, fp.y - fx.mean_vector(), ctx=ctx)
+    return mu + mτ, C
+
+
+def cov(fp, τ=None, *, ctx=None):
+    """cov(fp[, τ])  (AbstractGPs; predict_cov, src/direct_solver.jl:28-119): the M × M posterior covariance of the latent
+    f at τ (default: the data times), measurement noise not included."""
+    if not isinstance(fp, PosteriorGP):
+        raise TypeError("cov expects posterior(f(t, σ²), y)")
+    fx = fp.f
+    τ = fx.x if τ is None else np.asarray(τ, dtype=np.float64)
+    return predict_cov(fx.f.kernel, τ, fx.x, fx.σ2, ctx=ctx)
 
 
 def simulate(cov, τ, σ2, q, *, ctx=None):

@@ -345,6 +345,10 @@ class Context:
         """Cap in bytes of the reverse-mode workspace of one θ-chunk (0 = 1 GiB, the default)."""
         check(self.lib.pioran_ctx_set_vjp_workspace(self.h, int(nbytes)))
 
+    def set_postcov_workspace(self, nbytes):
+        """Cap in bytes of the device workspace plus output of one step of celerite_predict_cov (0 = 1 GiB, the default)."""
+        check(self.lib.pioran_ctx_set_postcov_workspace(self.h, int(nbytes)))
+
     def approx_logl_grad_dev(self, series, spec, B, theta_ptr, logl_ptr, grad_ptr):
         """Device-resident variant: raw device pointers (ints); logl_ptr may be 0."""
         check(self.lib.pioran_approx_logl_grad_dev(self.h, series.id, C.byref(spec), int(B), C.c_void_p(theta_ptr),
@@ -462,6 +466,22 @@ class Context:
         check(self.lib.pioran_celerite_predict_var(self.h, series.id, B, Jt, _p(a), _p(b), _p(c), _p(d), _p(mu), _p(nu),
                                                    tau.shape[0], _p(tau), _p(mean), _p(var)))
         return (mean, var) if return_mean else var
+
+    def celerite_predict_cov(self, series, a, b, c, d, tau, mu=None, nu=None, return_mean=True):
+        """Posterior covariance of the latent f at ascending τ (predict_cov, src/direct_solver.jl:28-119), [B × M × M] and
+        exactly symmetric, by K6 and the O(M·(N + M)·R) column walk K8.  With return_mean, (mean, cov), where mean is
+        celerite_predict's result bit for bit.  A set whose covariance is not positive definite gets a NaN matrix."""
+        a, b, c, d = (np.atleast_2d(_f64(x)) for x in (a, b, c, d))
+        B, Jt = a.shape
+        tau = _f64(tau)
+        M = tau.shape[0]
+        mu = _f64(mu, (B,)) if mu is not None else None
+        nu = _f64(nu, (B,)) if nu is not None else None
+        cov = np.empty((B, M, M))
+        mean = np.empty((B, M)) if return_mean else None
+        check(self.lib.pioran_celerite_predict_cov(self.h, series.id, B, Jt, _p(a), _p(b), _p(c), _p(d), _p(mu), _p(nu),
+                                                   M, _p(tau), _p(mean), _p(cov)))
+        return (mean, cov) if return_mean else cov
 
     def celerite_simulate(self, series, a, b, c, d, q, nu=None):
         """Batched sim(rng,a,b,c,d,t,σ²) (src/celerite_solver.jl:515-549) with the normal draws q [B × N] supplied."""

@@ -24,6 +24,7 @@
 #include "posterior.cuh"
 #include "postvar.cuh"
 #include "postdraw.cuh"
+#include "postcov.cuh"
 #include "table.cuh"
 #include "grad.cuh"
 #include "grad_pipe.cuh"
@@ -67,7 +68,7 @@ static int guard_fail() {
     } while (0)
 
 extern "C" const char* pioran_last_error(void) { return g_err.c_str(); }
-extern "C" int pioran_version(void) { return 304; }   // 0.3.4: pioran_celerite_posterior_draws
+extern "C" int pioran_version(void) { return 305; }   // 0.3.5: pioran_celerite_predict_cov
 
 // ------------------------------------------------------------------------------------------------ context
 namespace {
@@ -107,7 +108,7 @@ using PlanKey = std::tuple<int, int, int, int, double, double, double, double>;
 enum KernelFamily : int {
     KF_NONE = 0, KF_BLOCKED, KF_BLOCKED_WIDE, KF_SHARED, KF_SHARED_PAIR, KF_GENERIC, KF_WIDE_REG, KF_WIDE_REG_STORE, KF_WIDE_REG_SIM,
     KF_WIDE, KF_BLOCKED_GRAD, KF_GRAD, KF_GRAD_PIPE, KF_WIDE_GRAD, KF_JVP, KF_PREDICT, KF_GENERIC_SIM, KF_SCAN_FINISH,
-    KF_SCAN_PARTIAL, KF_DENSE_FINISH, KF_VJP, KF_POSTVAR, KF_POSTDRAW
+    KF_SCAN_PARTIAL, KF_DENSE_FINISH, KF_VJP, KF_POSTVAR, KF_POSTDRAW, KF_POSTCOV
 };
 struct KernelTag { int family = KF_NONE; int p[4] = {0, 0, 0, 0}; };
 
@@ -137,6 +138,7 @@ struct pioran_ctx {
     int gwork_items = 0, gwork_tpi = 0;
     int scan_chunks = 0;   // K3: chunks per parameter vector (0 = automatic)
     size_t vjp_ws_bytes = 0;   // K5r: workspace cap per θ-chunk (0 = 1 GiB; pioran_ctx_set_vjp_workspace)
+    size_t postcov_ws_bytes = 0;   // K8: workspace + output cap per step (0 = 1 GiB; pioran_ctx_set_postcov_workspace)
     bool auto_scan = true; // route few-evaluation calls on long series to K3 (pioran_ctx_set_auto_scan)
     int sweep_kernel = PIORAN_SWEEP_AUTO;   // pioran_ctx_set_sweep_kernel
     // pioran_ctx_create_multi: a group context owns one child context per device and no CUDA state of its own; the batched
@@ -426,6 +428,7 @@ extern "C" int pioran_ctx_last_kernel_name(pioran_ctx* c, char* buf, int len) tr
         case KF_PREDICT: snprintf(name, sizeof name, "predict<%d>", p[0]); break;
         case KF_POSTVAR: snprintf(name, sizeof name, "postvar<%d>", p[0]); break;
         case KF_POSTDRAW: snprintf(name, sizeof name, "postdraw<%d>", p[0]); break;
+        case KF_POSTCOV: snprintf(name, sizeof name, "postcov<%d>", p[0]); break;
         case KF_GENERIC_SIM: snprintf(name, sizeof name, "generic_sim<%d,%d>", p[0], p[1]); break;
         case KF_SCAN_FINISH: snprintf(name, sizeof name, "scan_finish"); break;
         case KF_SCAN_PARTIAL: snprintf(name, sizeof name, "scan_partial"); break;
@@ -2374,10 +2377,12 @@ extern "C" int pioran_celerite_simulate(pioran_ctx* c, int series_id, int B, int
 } catch (...) { return guard_fail(); }
 
 // ------------------------------------------------------------------------------------------------ posterior variance (K6)
-static int launch_postvar(pioran_ctx* c, const PostVarArgs& pv, int B) {
+template <bool COV = false>
+static int launch_postvar(pioran_ctx* c, const typename std::conditional<COV, PostVarCovArgs, PostVarArgs>::type& pv, int B) {
     const int TS = (pv.R + 15) / 16;
     int rc;
-    if ((rc = with_int<1, 8>(TS, [&](auto ts) { celerite_postvar_kernel<ts><<<B, WIDE_THREADS, 0, c->stream>>>(pv); return 0; }))) return rc;
+    if ((rc = with_int<1, 8>(TS, [&](auto ts) { celerite_postvar_kernel<ts, COV><<<B, WIDE_THREADS, 0, c->stream>>>(pv); return 0; })))
+        return rc;
     c->launches++;
     note_kernel(c, KF_POSTVAR, TS);
     CUDA_TRY(cudaGetLastError());
@@ -2562,6 +2567,155 @@ extern "C" int pioran_celerite_posterior_draws(pioran_ctx* c, int series_id, int
     cudaEventRecord(c->ev_end, c->stream);
     note_kernel(c, KF_POSTDRAW, PT);
     CUDA_TRY(cudaStreamSynchronize(c->stream));   // gt and gcode are locals
+    return PIORAN_OK;
+} catch (...) { return guard_fail(); }
+
+// ------------------------------------------------------------------------------------------------ posterior covariance (K8)
+extern "C" int pioran_celerite_predict_cov(pioran_ctx* c, int series_id, int B, int Jt, const double* a, const double* b,
+                                           const double* cc, const double* d, const double* mu, const double* nu, int64_t M,
+                                           const double* tau, double* mean_out, double* cov_out) try {
+    if (!c || !a || !b || !cc || !d || !tau || !cov_out) return fail(PIORAN_EINVAL, "NULL argument");
+    if (B < 1 || Jt < 1 || M < 1) return fail(PIORAN_EINVAL, "B, Jt and M must be >= 1");
+    for (int64_t m = 1; m < M; m++)
+        if (!(tau[m] >= tau[m - 1])) return fail(PIORAN_EINVAL, "tau must be ascending (tau[%lld] < tau[%lld])", (long long)m, (long long)m - 1);
+    if (is_group(c))
+        return group_fanout(c, series_id, B, [&](pioran_ctx* ch, int id, int64_t, int beg, int nb) {
+            const size_t o = (size_t)beg * Jt;
+            return pioran_celerite_predict_cov(ch, id, nb, Jt, a + o, b + o, cc + o, d + o, at(mu, beg), at(nu, beg), M, tau,
+                                               at(mean_out, (size_t)beg * M), cov_out + (size_t)beg * M * M);
+        });
+    PIORAN_COMPUTE_LOCK(c);
+    ExplicitSet x;   // the row map of the whole batch, shared by every θ-chunk
+    int rc;
+    if ((rc = explicit_front(c, series_id, B, Jt, b, d, 128, "rank %1$d (Jt = %2$d) exceeds the limit of %3$d of the posterior covariance", x)))
+        return rc;
+    Series* s = x.s;
+    const int R = x.R;
+    const int64_t N = s->N, NG = N + M;
+    std::vector<int> n0;
+    if ((rc = prediction_gaps(c, s, M, tau, n0))) return rc;
+    // merged grid: a τ point first at a tie (n₀ = #{t_n < τ}), the τ points in their order; gpos[m] = position of τ_m
+    std::vector<double> th, gt(NG);
+    std::vector<int> gcode(NG), gpos(M);
+    if ((rc = series_times(c, s, th))) return rc;
+    for (int64_t k = 0, n = 0, m = 0; k < NG; k++) {
+        const bool data = m == M || (n < N && th[n] < tau[m]);
+        gt[k] = data ? th[n] : tau[m];
+        if (!data) gpos[m] = (int)k;
+        gcode[k] = data ? (int)n++ : -(int)(m++) - 1;
+    }
+
+    // per set: W [N·RPL] | D, z [N] | mean, var [M] | g_τ, D_τ [M·(R + 1)] | r, w₀ [M·2R], and the output [M·M] of one θ-chunk,
+    // or, when one set's matrix alone exceeds the cap, a column range of w columns: rows [w·M] and their mirror rows [M·w].
+    // The factor, the mean and K6 run over groups of Bp ≥ Bc sets, as many as the cap holds beside the output of one K8 chunk of
+    // Bc sets: at N = M = 1e4 a matrix is 800 MB and a K8 chunk one set, but the sweeps still see the whole batch.
+    const size_t cap = c->postcov_ws_bytes ? c->postcov_ws_bytes : (size_t)1 << 30;
+    const int RPL = stored_factor_ld(R);
+    const size_t ws_set = sizeof(double) * ((size_t)N * RPL + 2 * (size_t)N + (size_t)M * (3 * R + 3));
+    const size_t full_set = ws_set + sizeof(double) * (size_t)M * M;
+    const int Bc = theta_chunk(B, full_set, cap);
+    int64_t wc = M;   // columns per range
+    if (full_set > cap) {
+        const size_t left = cap > ws_set ? cap - ws_set : 0;
+        wc = std::max<int64_t>(1, std::min<int64_t>(M, (int64_t)(left / (sizeof(double) * 2 * (size_t)M))));
+    }
+    const size_t out_set = wc == M ? (size_t)M * M : 2 * (size_t)wc * M;
+    const size_t out_bytes = sizeof(double) * out_set * Bc;
+    const int Bp = std::max(Bc, theta_chunk(B, ws_set, cap > out_bytes ? cap - out_bytes : 0));
+    if ((rc = c->post.ensure(ws_set * Bp + out_bytes + sizeof(double) * (NG + M) + sizeof(int) * (NG + 2 * M + 2))))
+        return rc;
+    double* W = c->post.as<double>();
+    double* D = W + (size_t)Bp * N * RPL;
+    double* z = D + (size_t)Bp * N;
+    double* mean = z + (size_t)Bp * N;
+    double* var = mean + (size_t)Bp * M;
+    double* ws = var + (size_t)Bp * M;
+    double* pt = ws + (size_t)Bp * M * (R + 1);
+    double* cov = pt + (size_t)Bp * M * 2 * R;
+    double* upm = cov + (size_t)Bc * wc * M;   // mirror rows of a column range
+    double* gt_dev = cov + (size_t)Bc * out_set;
+    double* tau_dev = gt_dev + NG;
+    int* n0_dev = reinterpret_cast<int*>(tau_dev + M);
+    int* gcode_dev = n0_dev + M;
+    int* gpos_dev = gcode_dev + NG;
+    CUDA_TRY(cudaMemcpyAsync(gt_dev, gt.data(), sizeof(double) * NG, cudaMemcpyHostToDevice, c->stream));
+    CUDA_TRY(cudaMemcpyAsync(tau_dev, tau, sizeof(double) * M, cudaMemcpyHostToDevice, c->stream));
+    CUDA_TRY(cudaMemcpyAsync(n0_dev, n0.data(), sizeof(int) * M, cudaMemcpyHostToDevice, c->stream));
+    CUDA_TRY(cudaMemcpyAsync(gcode_dev, gcode.data(), sizeof(int) * NG, cudaMemcpyHostToDevice, c->stream));
+    CUDA_TRY(cudaMemcpyAsync(gpos_dev, gpos.data(), sizeof(int) * M, cudaMemcpyHostToDevice, c->stream));
+    const int PT = R <= 32 ? 1 : R <= 64 ? 2 : 4;
+    cudaEventRecord(c->ev_beg, c->stream);
+    for (int b0 = 0; b0 < B; b0 += Bp) {
+        const int Bk = std::min(Bp, B - b0);
+        const size_t o = (size_t)b0 * Jt;
+        int nitems, tpi;
+        GenericInputs gi;
+        BatchArgs args;
+        if ((rc = upload_generic(c, Bk, Jt, N, a + o, b + o, cc + o, d + o, at(mu, b0), at(nu, b0), nullptr, nullptr, gi))) return rc;
+        if ((rc = generic_setup(c, s, Bk, Jt, x.term_row, R, gi, args, nitems, tpi))) return rc;
+        const int BS = bs_for_rank(R);
+        args.W_out = W; args.D_out = D; args.zf_out = z;
+        // the factor of pioran_celerite_predict, and its backsolve and predict kernels: mean_out is predict's, bit for bit
+        if ((rc = BS > 8 ? launch_wide<STEP_STORE>(c, args, nitems) : dispatch_generic_mode<STEP_STORE>(c, BS, args, nitems))) return rc;
+        if (mean_out) {
+            PostArgs pa{};
+            pa.t = s->t; pa.tau = tau_dev; pa.n0 = n0_dev; pa.N = N; pa.M = M; pa.B = Bk; pa.Jt = Jt; pa.RPL = RPL;
+            pa.a = gi.a; pa.b = gi.b; pa.c = gi.c; pa.d = gi.d; pa.term_row = c->rows.as<int>(); pa.mu = gi.mu;
+            pa.W = W; pa.D = D; pa.z = z; pa.mean = mean;
+            launch_posterior_mean(c, pa);
+            CUDA_TRY(cudaGetLastError());
+            CUDA_TRY(cudaMemcpyAsync(mean_out + (size_t)b0 * M, mean, sizeof(double) * (size_t)Bk * M, cudaMemcpyDeviceToHost, c->stream));
+        }
+        // K6 with the per-point vectors r(τ), w₀(τ)
+        PostVarCovArgs pv{};
+        pv.t = s->t; pv.tau = tau_dev; pv.n0 = n0_dev; pv.N = N; pv.M = M; pv.Jt = Jt; pv.R = R; pv.RPL = RPL;
+        pv.a = gi.a; pv.b = gi.b; pv.c = gi.c; pv.d = gi.d; pv.term_row = c->rows.as<int>();
+        pv.W = W; pv.D = D; pv.ws = ws; pv.var = var; pv.pt = pt;
+        if ((rc = launch_postvar<true>(c, pv, Bk))) return rc;
+        // K8 over chunks of Bc sets of the group, one launch per column range
+        for (int j0 = 0; j0 < Bk; j0 += Bc) {
+            const int Bj = std::min(Bc, Bk - j0);
+            PostCovArgs pc{};
+            pc.gt = gt_dev; pc.gcode = gcode_dev; pc.gpos = gpos_dev; pc.N = N; pc.M = M; pc.NG = NG;
+            pc.Jt = Jt; pc.R = R; pc.RPL = RPL;
+            pc.a = gi.a + (size_t)j0 * Jt; pc.b = gi.b + (size_t)j0 * Jt; pc.c = gi.c + (size_t)j0 * Jt; pc.d = gi.d + (size_t)j0 * Jt;
+            pc.term_row = c->rows.as<int>();
+            pc.W = W + (size_t)j0 * N * RPL; pc.pt = pt + (size_t)j0 * M * 2 * R; pc.out = cov; pc.ldo = M;
+            double* dst = cov_out + (size_t)(b0 + j0) * M * M;
+            for (int64_t c0 = 0; c0 < M; c0 += wc) {
+                const int64_t w = std::min<int64_t>(wc, M - c0);
+                pc.c0 = c0; pc.w = w; pc.up = wc == M ? nullptr : upm;
+                const int warps = (int)std::min<int64_t>(w, PC_MAXW);
+                const dim3 grid((unsigned)((w + warps - 1) / warps), Bj);
+                if ((rc = with_int<0, 2>(PT >> 1, [&](auto lp) { celerite_postcov_kernel<1 << lp><<<grid, 32 * warps, 0, c->stream>>>(pc); return 0; })))
+                    return rc;
+                c->launches++;
+                CUDA_TRY(cudaGetLastError());
+                if (wc == M) {
+                    CUDA_TRY(cudaMemcpyAsync(dst, cov, sizeof(double) * (size_t)Bj * M * M, cudaMemcpyDeviceToHost, c->stream));
+                } else {   // Bj = 1: rows c0 … c0 + w − 1 up to column c0 + w, then the mirror entries of rows 0 … c0 − 1
+                    CUDA_TRY(cudaMemcpy2DAsync(dst + (size_t)c0 * M, sizeof(double) * M, cov, sizeof(double) * M,
+                                               sizeof(double) * (size_t)(c0 + w), (size_t)w, cudaMemcpyDeviceToHost, c->stream));
+                    if (c0 > 0)
+                        CUDA_TRY(cudaMemcpy2DAsync(dst + c0, sizeof(double) * M, upm, sizeof(double) * w, sizeof(double) * w,
+                                                   (size_t)c0, cudaMemcpyDeviceToHost, c->stream));
+                    CUDA_TRY(cudaStreamSynchronize(c->stream));   // the next range reuses the staging rows
+                }
+            }
+        }
+    }
+    cudaEventRecord(c->ev_end, c->stream);
+    note_kernel(c, KF_POSTCOV, PT);
+    CUDA_TRY(cudaStreamSynchronize(c->stream));   // the merged grid and n0 are locals
+    return PIORAN_OK;
+} catch (...) { return guard_fail(); }
+
+extern "C" int pioran_ctx_set_postcov_workspace(pioran_ctx* c, long long bytes) try {
+    if (is_group(c)) return group_each(c, [&](pioran_ctx* ch) { return pioran_ctx_set_postcov_workspace(ch, bytes); });
+    if (!c) return fail(PIORAN_EINVAL, "ctx is NULL");
+    if (bytes < 0) return fail(PIORAN_EINVAL, "bytes must be >= 0 (0 = 1 GiB)");
+    std::lock_guard<std::mutex> lk(c->mu);
+    c->postcov_ws_bytes = (size_t)bytes;
     return PIORAN_OK;
 } catch (...) { return guard_fail(); }
 

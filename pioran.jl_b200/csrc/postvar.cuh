@@ -19,7 +19,13 @@
 // (Q and Ξ are symmetric; keeping both triangles makes every contraction a row sum).  U, W, φ and D of WIDE_PV_CH steps are
 // staged in shared memory; rows R … 16·TS − 1 are zero.  cos/sin are taken at absolute times (sincos_large, common.cuh).
 // A parameter vector whose factor has a pivot D_n ≤ 0 (or NaN) gets NaN in every entry of its row.
+//
+// COV = true (the first launch of the posterior covariance, postcov.cuh) also writes, per prediction point, the two vectors
+// the covariance walk K8 reads:  r(τ) = S_τ U(τ) − V(τ) (pass 1, before the decay to t_{n₀}) and the start vector
+// w₀(τ) = U(τ) + e_{τ→t_{n₀}} ∘ (Ξ_{n₀} g_τ) (U(τ) in pass 1, the Ξ term in pass 2); a bad pivot makes both NaN.
+// COV = false compiles to the variance kernel alone.
 #pragma once
+#include <type_traits>
 #include "common.cuh"
 #include "wide.cuh"
 
@@ -37,6 +43,9 @@ struct PostVarArgs {
     const double* W; const double* D;     // stored factor [B × N × RPL], [B × N]
     double* ws;                           // workspace [B × M × (R + 1)]: g_τ (R entries), then D_τ
     double* var;                          // [B × M]
+};
+struct PostVarCovArgs : PostVarArgs {     // COV = true: the variance kernel's arguments and
+    double* pt;                           // [B × M × 2R], r(τ) (R entries), then w₀(τ)
 };
 
 // Sum over the CTA of one value per thread, into slot `red` (8 doubles); the caller synchronises before reading it.
@@ -70,8 +79,9 @@ __device__ __forceinline__ void pv_row_sums(double (&rs)[8], double* out, int ty
 }
 
 // grid = B (one CTA per parameter vector), block = WIDE_THREADS
-template <int TS>
-__global__ void __launch_bounds__(WIDE_THREADS, TS <= 6 ? 2 : 1) celerite_postvar_kernel(const PostVarArgs pa) {
+template <int TS, bool COV = false>
+__global__ void __launch_bounds__(WIDE_THREADS, TS <= 6 ? 2 : 1)
+celerite_postvar_kernel(const typename std::conditional<COV, PostVarCovArgs, PostVarArgs>::type pa) {
     constexpr int LD = 16 * TS, NWARP = WIDE_THREADS / 32;
     __shared__ __align__(16) double tabU[PV_CH][LD], tabW[PV_CH][LD], tabP[PV_CH][LD];
     __shared__ double tabD[PV_CH];
@@ -99,6 +109,9 @@ __global__ void __launch_bounds__(WIDE_THREADS, TS <= 6 ? 2 : 1) celerite_postva
     for (int64_t n = tid; n < N; n += WIDE_THREADS) bad |= !(Dg[n] > 0.0);
     if (__syncthreads_or(bad)) {
         for (int64_t m = tid; m < M; m += WIDE_THREADS) var[m] = __longlong_as_double(0x7ff8000000000000LL);
+        if constexpr (COV)
+            for (int64_t k = tid; k < M * 2 * R; k += WIDE_THREADS)
+                pa.pt[(size_t)th * M * 2 * R + k] = __longlong_as_double(0x7ff8000000000000LL);
         return;
     }
     for (int r = tid; r < LD; r += WIDE_THREADS) { rterm[r] = 0; rkind[r] = ROW_PAD; }
@@ -139,6 +152,8 @@ __global__ void __launch_bounds__(WIDE_THREADS, TS <= 6 ? 2 : 1) celerite_postva
             if (tid < LD) {
                 double u;
                 row_uv(tid, tm, u, v);
+                if constexpr (COV)
+                    if (tid < R) pa.pt[((size_t)th * M + mp) * 2 * R + R + tid] = u;   // w₀ = U(τ); pass 2 adds the Ξ term
                 const double cr = rkind[tid] == ROW_PAD ? 0.0 : cc[rterm[tid]];
                 e = n > 0 ? exp(-cr * (tm - pa.t[n - 1])) : 0.0;
                 e2 = n < N ? exp(-cr * (pa.t[n] - tm)) : 0.0;
@@ -163,6 +178,8 @@ __global__ void __launch_bounds__(WIDE_THREADS, TS <= 6 ? 2 : 1) celerite_postva
             pv_row_sums<TS>(rs, ys[0], ty, tx);
             __syncthreads();
             if (tid < R) ws[mp * LDG + tid] = e2 * fma(e, ys[0][tid], -v);
+            if constexpr (COV)
+                if (tid < R) pa.pt[((size_t)th * M + mp) * 2 * R + tid] = fma(e, ys[0][tid], -v);   // r(τ)
             if (tid == 0) {
                 double q = 0.0;
 #pragma unroll
@@ -280,7 +297,25 @@ __global__ void __launch_bounds__(WIDE_THREADS, TS <= 6 ? 2 : 1) celerite_postva
                     part = fma(acc, gc, part);
                 }
                 pv_block_part(part, red[slot], lane, warp);
+                if constexpr (COV) {   // Ξ_n g_τ as row sums (Ξ is symmetric), into the start vector w₀
+                    double rs[8];
+#pragma unroll
+                    for (int i = 0; i < 8; i++) rs[i] = 0.0;
+#pragma unroll
+                    for (int j = 0; j < TS; j++) {
+                        const double gc = tx + 16 * j < R ? g[tx + 16 * j] : 0.0;
+#pragma unroll
+                        for (int i = 0; i < TS; i++) rs[i] = fma(Tm[i][j], gc, rs[i]);
+                    }
+                    pv_row_sums<TS>(rs, ys[slot], ty, tx);
+                }
                 __syncthreads();
+                if constexpr (COV)
+                    if (tid < R) {
+                        const double e2 = exp(-cc[rterm[tid]] * (pa.t[n] - pa.tau[mp]));
+                        double* w0 = pa.pt + ((size_t)th * M + mp) * 2 * R + R;
+                        w0[tid] = fma(e2, ys[slot][tid], w0[tid]);
+                    }
                 if (tid == 0) {
                     double q = 0.0;
 #pragma unroll
