@@ -224,10 +224,12 @@ UNREACHABLE = {
     "shared<5,12>": "needs PIORAN_PAIR=0, as shared<4,12>",
     "blocked_wide<8,9,4>": "rank 64 (the only 8-tile rank with its own data-row tile) goes to the scalar-pipe kernels",
 }
-# reachable, covered by their own rank grids elsewhere: K3 scan (test_gpu_scan.py), dense K4 (test_gpu_dense.py), posterior
-# mean and draws (test_posterior.py), JVP (test_gpu_jvp.py)
-OUT_OF_SCOPE = ("scan_finish", "scan_partial", "dense_finish", "predict<·>", "generic_sim<·,·>", "wide_reg_store<·>",
-                "wide_reg_sim<·>", "jvp<·>")
+# reachable, covered by their own rank grids elsewhere: K3 scan (test_gpu_scan.py), dense K4 (test_gpu_dense.py), JVP
+# (test_gpu_jvp.py); the posterior mean, variance, covariance and draws and the prior draws, with the store and draw modes of
+# the sweeps they run on, by the posterior matrix and its own ledger (test_gpu_posterior_matrix.py)
+OUT_OF_SCOPE = ("scan_finish", "scan_partial", "dense_finish", "jvp<·>", "generic_store<·,·>", "wide_reg_store<·>",
+                "generic_sim<·,·>", "wide_reg_sim<·>", "predict<·>", "postvar<·>", "postvar_cov<·>", "postdraw<·>",
+                "postcov<·>")
 
 
 # ------------------------------------------------------------------------------------------------ cells
