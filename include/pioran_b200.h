@@ -381,6 +381,22 @@ int pioran_celerite_predict_cov(pioran_ctx *ctx, int series_id, int B, int Jt,
 /* Cap in bytes of the device workspace plus output of one step of pioran_celerite_predict_cov (0 = 1 GiB, the default).
  * The result does not depend on it; a small cap splits a batch into many θ-chunks, and a set into column ranges. */
 int pioran_ctx_set_postcov_workspace(pioran_ctx *ctx, long long bytes);
+/* Generalised Lomb–Scargle periodograms (K9) of B series on the times of one resident series: the floating-mean periodogram
+ * (Zechmeister & Kürster 2009) with the :standard normalisation, which LombScargle.jl computes by default (fit_mean,
+ * center_data) and the posterior predictive checks of src/plots_diagnostics.jl:532-546 take for one simulated series per
+ * posterior sample.  y_batch [B × N] (NULL: the resident y, B must be 1); weighted = 1: weights 1/s2 of the resident series
+ * (LombScargle.jl's `errors`), 0: equal weights.  freq [F] > 0 and finite, any order, in the inverse unit of t.  power_out
+ * [B × F] row-major, in [0, 1].  Where the formula divides zero by zero (an all-zero row, N = 1, a frequency at which the
+ * basis is degenerate on these times) the value is NaN; that is data, not an error.  PIORAN_EINVAL for NULL ctx, freq or
+ * power_out, B or F < 1, a NULL y_batch with B > 1, a frequency that is not positive and finite, an unknown series, and
+ * weighted with an s2 of the series that is not positive and finite.  Each value is summed in the same order whatever B,
+ * the chunking or the row's position, so a row's periodogram is the same bit for bit in any batch.  A device group splits
+ * the rows over its devices. */
+int pioran_lombscargle(pioran_ctx *ctx, int series_id, int B, const double *y_batch, int weighted,
+                       int64_t F, const double *freq, double *power_out);
+/* Cap in bytes of the device workspace plus output of one step of pioran_lombscargle (0 = 1 GiB, the default).  The result
+ * does not depend on it; a small cap splits the frequencies and the rows into many chunks. */
+int pioran_ctx_set_lsp_workspace(pioran_ctx *ctx, long long bytes);
 
 #ifdef __cplusplus
 }

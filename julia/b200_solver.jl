@@ -372,6 +372,57 @@ function sim_b200(rng, a, b, c, d, τ, σ2)
 end
 
 """
+    sim_b200(rng, A, B, C, D, τ, σ2; ν = nothing) -> Matrix (N × P)
+
+One draw per coefficient set: A, B, C, D are P × J (row p = the coefficients of posterior sample p), column p of the result is
+`sim_b200(rng, A[p, :], B[p, :], C[p, :], D[p, :], τ, ν[p] .* σ2)` with the normals of column p of `randn(rng, N, P)`
+(ν = nothing: 1).  One call for all P sets.  Not run here: no Julia toolchain.
+"""
+function sim_b200(rng, A::AbstractMatrix, B::AbstractMatrix, C::AbstractMatrix, D::AbstractMatrix, τ, σ2; ν = nothing)
+    P, J = size(A)
+    N = length(τ)
+    q = randn(rng, N, P)                      # column-major N × P = row-major [P × N]
+    s = b200_upload(collect(Float64, τ), zeros(N), collect(Float64, σ2))
+    y = Matrix{Float64}(undef, N, P)
+    row_major(X) = Matrix{Float64}(permutedims(X))   # J × P column-major = the C ABI's [P × J]
+    try
+        _b200_check(ccall((:pioran_celerite_simulate, libpioran_b200), Cint,
+            (Ptr{Cvoid}, Cint, Cint, Cint, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}),
+            b200_context().h, s.id, P, J, row_major(A), row_major(B), row_major(C), row_major(D),
+            ν === nothing ? C_NULL : collect(Float64, ν), q, y))
+    finally
+        b200_free(s)
+    end
+    return y
+end
+
+"""
+    lombscargle_b200(t, Y, dy, freq) -> Matrix (F × P)
+
+Lomb–Scargle power of every column of Y (N × P) on the times t at the positive frequencies freq (inverse unit of t):
+LombScargle.jl's `lombscargle(t, Y[:, p], dy; frequencies = freq)` with its defaults (`fit_mean`, `center_data`, `:standard`)
+for every p in one call (K9).  dy = `nothing`: equal weights.  Column p of the result is the power of column p of Y.  0/0 (a
+constant column, N = 1, a frequency at which the basis is degenerate on these times) gives NaN.  Not run here: no Julia toolchain.
+"""
+function lombscargle_b200(t, Y::AbstractVecOrMat, dy, freq)
+    o = sortperm(t)                           # the power does not depend on the order of the points
+    N, P = size(Y, 1), size(Y, 2)
+    σ2 = dy === nothing ? ones(N) : collect(Float64, dy[o]) .^ 2
+    s = b200_upload(collect(Float64, t[o]), zeros(N), σ2)
+    F = length(freq)
+    power = Matrix{Float64}(undef, F, P)
+    try
+        _b200_check(ccall((:pioran_lombscargle, libpioran_b200), Cint,
+            (Ptr{Cvoid}, Cint, Cint, Ptr{Float64}, Cint, Int64, Ptr{Float64}, Ptr{Float64}),
+            b200_context().h, s.id, P, Matrix{Float64}(reshape(Y, N, P)[o, :]), dy === nothing ? 0 : 1, F,
+            collect(Float64, freq), power))
+    finally
+        b200_free(s)
+    end
+    return power
+end
+
+"""
     logpdf_gradient_batch_lognormal(series, spec, Θ) -> (logℒ::Vector, ∇::Matrix)
 
 Gradient of the log-normal likelihood (docs/src/ultranest.md:197-217 under ForwardDiff): Θ rows = [psd parameters…, variance, ν, μ, c],

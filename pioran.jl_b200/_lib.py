@@ -78,6 +78,8 @@ SYMBOLS = {
     "pioran_celerite_predict_cov": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_int, _dp, _dp, _dp, _dp, _dp, _dp, C.c_int64,
                                               _dp, _dp, _dp]),
     "pioran_ctx_set_postcov_workspace": (C.c_int, [C.c_void_p, C.c_longlong]),
+    "pioran_lombscargle": (C.c_int, [C.c_void_p, C.c_int, C.c_int, _dp, C.c_int, C.c_int64, _dp, _dp]),
+    "pioran_ctx_set_lsp_workspace": (C.c_int, [C.c_void_p, C.c_longlong]),
 }
 
 _lib = None

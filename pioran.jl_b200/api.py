@@ -670,6 +670,29 @@ def rand(fx, q, t=None, *, ctx=None):
     return simulate(fx.f.kernel, t, np.zeros_like(t), q, ctx=ctx) + mt
 
 
+def lombscargle(t, y, dy=None, *, frequencies, ctx=None):
+    """lombscargle(t, y[, dy]; frequencies)  (LombScargle.jl's defaults: fit_mean, center_data, :standard normalisation):
+    the generalised Lomb–Scargle power of y [N] or of each row of y [B × N] at the positive frequencies (inverse unit of t),
+    [F] or [B × F], weighted by 1/dy² when the errors dy are given.  The times may come in any order; they must be distinct.
+    Where the formula divides zero by zero (a constant row, N = 1, a frequency at which the basis is degenerate on these
+    times) the power is NaN."""
+    ctx = ctx or get_context()
+    t = np.asarray(t, dtype=np.float64)
+    y = np.asarray(y, dtype=np.float64)
+    one = y.ndim == 1
+    Y = np.atleast_2d(y)
+    if t.ndim != 1 or Y.ndim != 2 or Y.shape[1] != t.shape[0]:
+        raise ValueError(f"y must be [N] or [B, N] with N = {t.shape[0]}, got {list(y.shape)}")
+    s2 = np.ones_like(t) if dy is None else np.broadcast_to(np.asarray(dy, dtype=np.float64), t.shape) ** 2
+    order = np.argsort(t, kind="stable")   # the periodogram does not depend on the order of the points
+    ser = ctx.upload_series(t[order], np.zeros_like(t), s2[order])
+    try:
+        out = ctx.lombscargle(ser, frequencies, y_batch=Y[:, order], weighted=dy is not None)
+    finally:
+        ser.free()
+    return out[0] if one else out
+
+
 # ----------------------------------------------------------------------------------------------- batched entry
 class BatchedLikelihood:
     """Vectorised log-likelihood of the samplers' model (examples/ultranest/single_pl.jl:65-93):

@@ -349,6 +349,10 @@ class Context:
         """Cap in bytes of the device workspace plus output of one step of celerite_predict_cov (0 = 1 GiB, the default)."""
         check(self.lib.pioran_ctx_set_postcov_workspace(self.h, int(nbytes)))
 
+    def set_lsp_workspace(self, nbytes):
+        """Cap in bytes of the device workspace plus output of one step of lombscargle (0 = 1 GiB, the default)."""
+        check(self.lib.pioran_ctx_set_lsp_workspace(self.h, int(nbytes)))
+
     def approx_logl_grad_dev(self, series, spec, B, theta_ptr, logl_ptr, grad_ptr):
         """Device-resident variant: raw device pointers (ints); logl_ptr may be 0."""
         check(self.lib.pioran_approx_logl_grad_dev(self.h, series.id, C.byref(spec), int(B), C.c_void_p(theta_ptr),
@@ -512,6 +516,24 @@ class Context:
         out = np.empty((B, S, M))
         check(self.lib.pioran_celerite_posterior_draws(self.h, series.id, B, Jt, _p(a), _p(b), _p(c), _p(d), _p(mu), _p(nu),
                                                        _p(y_batch), M, _p(tau), float(sigma2_tau), S, _p(q), _p(out)))
+        return out
+
+    def lombscargle(self, series, freq, y_batch=None, weighted=True):
+        """Generalised Lomb–Scargle periodograms (floating mean, :standard normalisation; K9) of the rows of y_batch [B × N]
+        (None: the resident y) on the series' times at the positive frequencies freq [F]: [B × F], in [0, 1].  weighted:
+        weights 1/σ² of the series, else equal weights.  0/0 (an all-zero row, N = 1, a frequency at which the basis is
+        degenerate on these times) gives NaN."""
+        freq = _f64(freq)
+        if freq.ndim != 1:
+            raise ValueError("freq must be a 1-D array")
+        if y_batch is not None:
+            y_batch = np.ascontiguousarray(np.atleast_2d(np.asarray(y_batch, dtype=np.float64)))
+            if y_batch.ndim != 2 or y_batch.shape[1] != series.N:
+                raise ValueError(f"y_batch must be [B, {series.N}], got {list(y_batch.shape)}")
+        B = 1 if y_batch is None else y_batch.shape[0]
+        out = np.empty((B, freq.shape[0]))
+        check(self.lib.pioran_lombscargle(self.h, series.id, B, _p(y_batch), int(bool(weighted)), freq.shape[0], _p(freq),
+                                          _p(out)))
         return out
 
 

@@ -1,6 +1,7 @@
 // api.cu — C ABI of libpioran_b200.so (include/pioran_b200.h): contexts, resident series, launch logic.
 // No CPU fallback anywhere: every entry point either runs the sm_100a kernels or fails with an error code.
 #include <algorithm>
+#include <climits>
 #include <cmath>
 #include <cstdarg>
 #include <cstdio>
@@ -25,6 +26,7 @@
 #include "postvar.cuh"
 #include "postdraw.cuh"
 #include "postcov.cuh"
+#include "lsp.cuh"
 #include "table.cuh"
 #include "grad.cuh"
 #include "grad_pipe.cuh"
@@ -68,7 +70,7 @@ static int guard_fail() {
     } while (0)
 
 extern "C" const char* pioran_last_error(void) { return g_err.c_str(); }
-extern "C" int pioran_version(void) { return 305; }   // 0.3.5: pioran_celerite_predict_cov
+extern "C" int pioran_version(void) { return 306; }   // 0.3.6: pioran_lombscargle
 
 // ------------------------------------------------------------------------------------------------ context
 namespace {
@@ -108,7 +110,7 @@ using PlanKey = std::tuple<int, int, int, int, double, double, double, double>;
 enum KernelFamily : int {
     KF_NONE = 0, KF_BLOCKED, KF_BLOCKED_WIDE, KF_SHARED, KF_SHARED_PAIR, KF_GENERIC, KF_WIDE_REG, KF_WIDE_REG_STORE, KF_WIDE_REG_SIM,
     KF_WIDE, KF_BLOCKED_GRAD, KF_GRAD, KF_GRAD_PIPE, KF_WIDE_GRAD, KF_JVP, KF_PREDICT, KF_GENERIC_SIM, KF_SCAN_FINISH,
-    KF_SCAN_PARTIAL, KF_DENSE_FINISH, KF_VJP, KF_POSTVAR, KF_POSTDRAW, KF_POSTCOV
+    KF_SCAN_PARTIAL, KF_DENSE_FINISH, KF_VJP, KF_POSTVAR, KF_POSTDRAW, KF_POSTCOV, KF_LSP
 };
 struct KernelTag { int family = KF_NONE; int p[4] = {0, 0, 0, 0}; };
 
@@ -139,6 +141,7 @@ struct pioran_ctx {
     int scan_chunks = 0;   // K3: chunks per parameter vector (0 = automatic)
     size_t vjp_ws_bytes = 0;   // K5r: workspace cap per θ-chunk (0 = 1 GiB; pioran_ctx_set_vjp_workspace)
     size_t postcov_ws_bytes = 0;   // K8: workspace + output cap per step (0 = 1 GiB; pioran_ctx_set_postcov_workspace)
+    size_t lsp_ws_bytes = 0;       // K9: workspace + output cap per step (0 = 1 GiB; pioran_ctx_set_lsp_workspace)
     bool auto_scan = true; // route few-evaluation calls on long series to K3 (pioran_ctx_set_auto_scan)
     int sweep_kernel = PIORAN_SWEEP_AUTO;   // pioran_ctx_set_sweep_kernel
     // pioran_ctx_create_multi: a group context owns one child context per device and no CUDA state of its own; the batched
@@ -429,6 +432,7 @@ extern "C" int pioran_ctx_last_kernel_name(pioran_ctx* c, char* buf, int len) tr
         case KF_POSTVAR: snprintf(name, sizeof name, "postvar<%d>", p[0]); break;
         case KF_POSTDRAW: snprintf(name, sizeof name, "postdraw<%d>", p[0]); break;
         case KF_POSTCOV: snprintf(name, sizeof name, "postcov<%d>", p[0]); break;
+        case KF_LSP: snprintf(name, sizeof name, "lsp<%d,%d,%d>", p[0], p[1], p[2]); break;
         case KF_GENERIC_SIM: snprintf(name, sizeof name, "generic_sim<%d,%d>", p[0], p[1]); break;
         case KF_SCAN_FINISH: snprintf(name, sizeof name, "scan_finish"); break;
         case KF_SCAN_PARTIAL: snprintf(name, sizeof name, "scan_partial"); break;
@@ -2716,6 +2720,106 @@ extern "C" int pioran_ctx_set_postcov_workspace(pioran_ctx* c, long long bytes) 
     if (bytes < 0) return fail(PIORAN_EINVAL, "bytes must be >= 0 (0 = 1 GiB)");
     std::lock_guard<std::mutex> lk(c->mu);
     c->postcov_ws_bytes = (size_t)bytes;
+    return PIORAN_OK;
+} catch (...) { return guard_fail(); }
+
+// ------------------------------------------------------------------------------------------------ Lomb–Scargle periodograms (K9)
+constexpr size_t LSP_TABLE_BYTES = (size_t)64 << 20;   // basis of one frequency chunk: stays in the 126 MB L2 beside the row tiles
+
+extern "C" int pioran_lombscargle(pioran_ctx* c, int series_id, int B, const double* y_batch, int weighted, int64_t F,
+                                  const double* freq, double* power_out) try {
+    if (!c || !freq || !power_out) return fail(PIORAN_EINVAL, "NULL argument");
+    if (B < 1 || F < 1) return fail(PIORAN_EINVAL, "B and F must be >= 1");
+    if (!y_batch && B > 1) return fail(PIORAN_EINVAL, "y_batch is NULL with B = %d: the resident y is one row", B);
+    if (F > INT_MAX) return fail(PIORAN_EINVAL, "F = %lld frequencies exceeds INT_MAX", (long long)F);
+    for (int64_t k = 0; k < F; k++)
+        if (!(freq[k] > 0.0 && std::isfinite(freq[k]))) return fail(PIORAN_EINVAL, "freq[%lld] = %g is not positive and finite", (long long)k, freq[k]);
+    if (is_group(c))
+        return group_fanout(c, series_id, B, [&](pioran_ctx* ch, int id, int64_t N, int beg, int nb) {
+            return pioran_lombscargle(ch, id, nb, at(y_batch, (size_t)beg * N), weighted, F, freq, power_out + (size_t)beg * F);
+        });
+    PIORAN_COMPUTE_LOCK(c);
+    CUDA_TRY(cudaSetDevice(c->device));
+    Series* s = get_series(c, series_id);
+    if (!s) return fail(PIORAN_EINVAL, "unknown series id %d", series_id);
+    const int64_t N = s->N;
+    // normalised weights w_n: 1/σ²_n over their sum, or 1/N
+    std::vector<double> w(N, 1.0 / (double)N);
+    if (weighted) {
+        CUDA_TRY(cudaMemcpyAsync(w.data(), s->s2, sizeof(double) * N, cudaMemcpyDeviceToHost, c->stream));
+        CUDA_TRY(cudaStreamSynchronize(c->stream));
+        double sum = 0.0;
+        for (int64_t n = 0; n < N; n++) {
+            if (!(w[n] > 0.0 && std::isfinite(w[n])))
+                return fail(PIORAN_EINVAL, "weighted periodogram: s2[%lld] = %g of the series is not positive and finite", (long long)n, w[n]);
+            w[n] = 1.0 / w[n];
+            sum += w[n];
+        }
+        for (int64_t n = 0; n < N; n++) w[n] /= sum;
+    }
+    // per step: the basis of fc frequencies [2·fc × Npad] and their normalisers, then as many rows as the rest of the cap holds:
+    // the weighted rows [rc × Npad], YY, the raw rows (y_batch) and the output [rc × fc]
+    constexpr int FT = LSP_BN / 2;   // frequencies per column tile
+    const size_t cap = c->lsp_ws_bytes ? c->lsp_ws_bytes : (size_t)1 << 30;
+    const int64_t Npad = (N + LSP_BK - 1) / LSP_BK * LSP_BK;
+    const size_t per_f = sizeof(double) * 2 * Npad + sizeof(LspNorm);
+    int64_t fc = (int64_t)(std::min(LSP_TABLE_BYTES, cap / 2) / per_f) / FT * FT;
+    fc = std::min<int64_t>(std::max<int64_t>(fc, FT), (F + FT - 1) / FT * FT);
+    const size_t fixed = per_f * fc + sizeof(double) * (Npad + F);
+    const size_t per_r = sizeof(double) * (Npad + 1 + (y_batch ? N : 0) + fc);
+    int rc = theta_chunk(B, per_r, cap > fixed ? cap - fixed : 0);
+    if (rc < B && rc > LSP_BM) rc = rc / LSP_BM * LSP_BM;
+    const int rcpad = (rc + LSP_BM - 1) / LSP_BM * LSP_BM;
+    int err;
+    if ((err = c->post.ensure(per_f * fc + sizeof(double) * ((size_t)rcpad * (Npad + 1) + (y_batch ? (size_t)rc * N : 0) +
+                                                              (size_t)rc * fc + N + F))))
+        return err;
+    double* tab = c->post.as<double>();
+    LspNorm* norm = reinterpret_cast<LspNorm*>(tab + (size_t)2 * fc * Npad);
+    double* A = reinterpret_cast<double*>(norm + fc);
+    double* YY = A + (size_t)rcpad * Npad;
+    double* yraw = YY + rcpad;
+    double* out = yraw + (y_batch ? (size_t)rc * N : 0);
+    double* w_dev = out + (size_t)rc * fc;
+    double* f_dev = w_dev + N;
+    CUDA_TRY(cudaMemcpyAsync(w_dev, w.data(), sizeof(double) * N, cudaMemcpyHostToDevice, c->stream));
+    CUDA_TRY(cudaMemcpyAsync(f_dev, freq, sizeof(double) * F, cudaMemcpyHostToDevice, c->stream));
+    auto product = lsp_product_kernel<LSP_BM, LSP_BN, LSP_BK>;
+    CUDA_TRY(cudaFuncSetAttribute(product, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)LSP_SMEM));
+    // frequency chunks outside, row chunks inside: the basis is built once per frequency chunk; the rows are prepared once
+    // when they fit one chunk, else again for every frequency chunk (B·N work against B·N·fc in the product)
+    cudaEventRecord(c->ev_beg, c->stream);
+    for (int64_t f0 = 0; f0 < F; f0 += fc) {
+        const int nf = (int)std::min<int64_t>(fc, F - f0), nfpad = (nf + FT - 1) / FT * FT;
+        lsp_table_kernel<<<nfpad / 8, 256, 0, c->stream>>>(s->t, w_dev, N, Npad, f_dev + f0, nf, nfpad, tab, norm);
+        c->launches++;
+        for (int r0 = 0; r0 < B; r0 += rc) {
+            const int nr = std::min(rc, B - r0), nrpad = (nr + LSP_BM - 1) / LSP_BM * LSP_BM;
+            if (rc < B || f0 == 0) {
+                if (y_batch)
+                    CUDA_TRY(cudaMemcpyAsync(yraw, y_batch + (size_t)r0 * N, sizeof(double) * nr * N, cudaMemcpyHostToDevice, c->stream));
+                lsp_rows_kernel<<<nrpad / 8, 256, 0, c->stream>>>(y_batch ? yraw : s->y, N, w_dev, N, Npad, nr, nrpad, A, YY);
+                c->launches++;
+            }
+            product<<<dim3(2 * nfpad / LSP_BN, nrpad / LSP_BM), 256, LSP_SMEM, c->stream>>>(A, tab, Npad, YY, norm, nr, nf, out, nf);
+            c->launches++;
+            CUDA_TRY(cudaGetLastError());
+            CUDA_TRY(cudaMemcpy2DAsync(power_out + (size_t)r0 * F + f0, sizeof(double) * F, out, sizeof(double) * nf,
+                                       sizeof(double) * nf, (size_t)nr, cudaMemcpyDeviceToHost, c->stream));
+        }
+    }
+    cudaEventRecord(c->ev_end, c->stream);
+    note_kernel(c, KF_LSP, LSP_BM, LSP_BN, LSP_BK);
+    CUDA_TRY(cudaStreamSynchronize(c->stream));
+    return PIORAN_OK;
+} catch (...) { return guard_fail(); }
+
+extern "C" int pioran_ctx_set_lsp_workspace(pioran_ctx* c, long long bytes) try {
+    if (is_group(c)) return group_each(c, [&](pioran_ctx* ch) { return pioran_ctx_set_lsp_workspace(ch, bytes); });
+    if (!c) return fail(PIORAN_EINVAL, "ctx is NULL");
+    if (bytes < 0) return fail(PIORAN_EINVAL, "bytes must be >= 0 (0 = 1 GiB)");
+    std::lock_guard<std::mutex> lk(c->mu);
+    c->lsp_ws_bytes = (size_t)bytes;
     return PIORAN_OK;
 } catch (...) { return guard_fail(); }
 
