@@ -79,7 +79,7 @@ int pioran_ctx_destroy(pioran_ctx *ctx);
 /* One context over several devices of the box, for a caller that is ONE process with one likelihood callback (the
  * reference's samplers: examples/ultranest/single_pl.jl:113-117; dispatch of src/scalable_GP.jl:24-40, 162-166).
  * pioran_series_upload places the series on every device; the batched host-pointer entries (pioran_approx_logl,
- * pioran_approx_logl_logshift, pioran_approx_logl_grad, pioran_celerite_logl, pioran_direct_logl) cut their B parameter vectors into ndev
+ * pioran_approx_logl_logshift, pioran_approx_logl_sine(_grad), pioran_approx_logl_grad, pioran_celerite_logl, pioran_direct_logl) cut their B parameter vectors into ndev
  * contiguous slices, run each slice on its device concurrently and write the results straight into the caller's arrays -
  * the slices are independent, so no collective is involved.  Every other entry runs on devices[0]; the device-pointer
  * entries (_dev) and pioran_ctx_set_stream need a single-device context and return PIORAN_EUNSUPPORTED on a group. */
@@ -191,6 +191,21 @@ int pioran_ctx_set_sweep_kernel(pioran_ctx *ctx, int which);
  * SingleBendingPowerLaw, ranks <= 62.  logl_out: [B] or NULL. */
 int pioran_approx_logl_logshift_grad(pioran_ctx *ctx, int series_id, const pioran_approx_spec *spec, int B,
                                      const double *theta, double *logl_out, double *grad_out);
+
+/* Sinusoidal mean (examples/ultranest/single_pl_periodicity.jl, the reference's periodicity search):
+ *   logl = logpdf(ScalableGP(m, approx(P, f_min, f_max, J, norm))(t, nu*sigma^2), y),   m(t) = mu + A*sin(2*pi*t/T0 + phi)
+ * theta: [B x (n_psd_par+6)] row-major = psd parameters..., norm, nu, mu, A, phi, T0.  y - A*sin(...) is formed on the device
+ * (one pass over B x N, in theta-chunks of at most 1 GiB) in front of the same K1 + K2 as pioran_approx_logl; mu stays the
+ * sweep's scalar, so A = 0 gives pioran_approx_logl's value bit for bit.  Non-finite results are returned as data.  One
+ * resident series, ranks <= 64 (PIORAN_EUNSUPPORTED above).  logl_out: [B]. */
+int pioran_approx_logl_sine(pioran_ctx *ctx, int series_id, const pioran_approx_spec *spec, int B,
+                            const double *theta, double *logl_out);
+/* Gradient of pioran_approx_logl_sine: grad_out [B x (n_psd_par+6)] in the column order of theta.  The partials of A, phi and
+ * T0 are the innovations of three data rows whose right-hand sides are d(y - m)/d(A, phi, T0), carried by one more warp of the
+ * blocked gradient kernel.  Single- and DoubleBendingPowerLaw, ranks <= 62 (PIORAN_EUNSUPPORTED above, and under
+ * PIORAN_SWEEP_SCALAR).  logl_out: [B] or NULL. */
+int pioran_approx_logl_sine_grad(pioran_ctx *ctx, int series_id, const pioran_approx_spec *spec, int B,
+                                 const double *theta, double *logl_out, double *grad_out);
 
 /* ---- K5g: forward-mode derivatives of the explicit-coefficient likelihood ----------------------------------
  * d/dε of pioran_celerite_logl along P directions per parameter vector (ForwardDiff's chunk over logl): for set i and

@@ -439,6 +439,39 @@ function logpdf_gradient_batch_lognormal(s::B200Series, spec::Ref{B200ApproxSpec
     return out, permutedims(gr)
 end
 
+"""
+    logl_sine_b200(series, spec, Θ) -> Vector
+
+The reference's periodicity run (examples/ultranest/single_pl_periodicity.jl): Θ rows = [psd parameters…, variance, ν, μ, A, ϕ, T₀],
+logpdf(ScalableGP(m, approx(…))(t, ν .* σ.^2), y) with the CustomMean m(t) = μ + A·sin(2πt/T₀ + ϕ); y − A·sin(…) is formed on
+the device.  Upload y and σ² once, untouched.
+"""
+function logl_sine_b200(s::B200Series, spec::Ref{B200ApproxSpec}, Θ::Matrix{Float64})
+    B = size(Θ, 1)
+    Θr = permutedims(Θ)
+    out = Vector{Float64}(undef, B)
+    _b200_check(ccall((:pioran_approx_logl_sine, libpioran_b200), Cint,
+        (Ptr{Cvoid}, Cint, Ptr{B200ApproxSpec}, Cint, Ptr{Float64}, Ptr{Float64}), b200_context().h, s.id, spec, B, Θr, out))
+    return out
+end
+
+"""
+    logl_sine_grad_b200(series, spec, Θ) -> (logℒ::Vector, ∇::Matrix)
+
+Gradient of `logl_sine_b200` (what ForwardDiff.gradient gives HMC/NUTS): ∇[i, :] in the column order of Θ, the partials of
+A, ϕ and T₀ included.  Ranks ≤ 62.
+"""
+function logl_sine_grad_b200(s::B200Series, spec::Ref{B200ApproxSpec}, Θ::Matrix{Float64})
+    B, P = size(Θ)
+    Θr = permutedims(Θ)
+    out = Vector{Float64}(undef, B)
+    gr = Matrix{Float64}(undef, P, B)
+    _b200_check(ccall((:pioran_approx_logl_sine_grad, libpioran_b200), Cint,
+        (Ptr{Cvoid}, Cint, Ptr{B200ApproxSpec}, Cint, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}),
+        b200_context().h, s.id, spec, B, Θr, out, gr))
+    return out, permutedims(gr)
+end
+
 # --------------------------------------------------------------------------------------------------- prior transform on the device
 struct B200PriorSpec   # == struct pioran_prior_spec (24 bytes)
     kind::Int32        # 0 Uniform(p0, p1) · 1 Uniform(θ[ref_col], p1) · 2 LogUniform · 3 Normal · 4 LogNormal · 5 Gamma(shape p0 ∈ ℕ, scale p1)

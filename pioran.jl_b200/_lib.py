@@ -48,6 +48,8 @@ SYMBOLS = {
     "pioran_approx_logl_dev": (C.c_int, [C.c_void_p, C.c_int, _ip, C.POINTER(ApproxSpec), C.c_int, C.c_void_p, C.c_int, C.c_void_p]),
     "pioran_approx_logl_grad": (C.c_int, [C.c_void_p, C.c_int, C.POINTER(ApproxSpec), C.c_int, _dp, _dp, _dp]),
     "pioran_approx_logl_logshift_grad": (C.c_int, [C.c_void_p, C.c_int, C.POINTER(ApproxSpec), C.c_int, _dp, _dp, _dp]),
+    "pioran_approx_logl_sine": (C.c_int, [C.c_void_p, C.c_int, C.POINTER(ApproxSpec), C.c_int, _dp, _dp]),
+    "pioran_approx_logl_sine_grad": (C.c_int, [C.c_void_p, C.c_int, C.POINTER(ApproxSpec), C.c_int, _dp, _dp, _dp]),
     "pioran_approx_logl_grad_dev": (C.c_int, [C.c_void_p, C.c_int, C.POINTER(ApproxSpec), C.c_int, C.c_void_p, C.c_void_p, C.c_void_p]),
     "pioran_celerite_logl_jvp": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int] + [_dp] * 18),
     "pioran_approx_features_logl_grad": (C.c_int, [C.c_void_p, C.c_int, C.POINTER(ApproxSpec), C.c_int, C.c_int, _dp, _dp, _dp]),

@@ -701,11 +701,16 @@ class BatchedLikelihood:
 
     def __init__(self, t, y, σ2, psd_model="SingleBendingPowerLaw", n_components=20, basis_function="SHO",
                  f_min=None, f_max=None, S_low=20.0, S_high=20.0, is_integrated_power=True, ctx=None, log_shift=False,
-                 n_features=0, gradient="forward"):
+                 n_features=0, gradient="forward", periodic_mean=False):
         # n_features: Θ rows end with (S₀, f₀, Q) per QPO feature added to the continuum (docs/src/adding_features.md)
         self.n_features = int(n_features)
         if self.n_features and log_shift:
             raise ValueError("PSD features and the log-shift transform cannot be combined in one fused call")
+        # periodic_mean: Θ rows end with (A, ϕ, T₀) and the mean is μ + A·sin(2πt/T₀ + ϕ)
+        # (examples/ultranest/single_pl_periodicity.jl)
+        self.periodic_mean = bool(periodic_mean)
+        if self.periodic_mean and (self.n_features or log_shift):
+            raise ValueError("the periodic mean cannot be combined with PSD features or the log-shift transform in one fused call")
         # gradient: "forward" (one K5g direction per Θ column) or "reverse" (one K5r sweep); only the gradient with features has
         # both — without them c and d are fixed by the spectral grid and the fused approx-path gradient serves every column
         if gradient not in ("forward", "reverse"):
@@ -726,7 +731,8 @@ class BatchedLikelihood:
             psd_model = psd_model.model_name
         self.spec = make_spec(psd_model, f_min, f_max, n_components, S_low, S_high, is_integrated_power, basis_function)
         self.series = self.ctx.upload_series(t, y, σ2)
-        self.n_par = backend.N_PSD_PAR[self.spec.psd_model] + 3 + int(self.log_shift) + 3 * self.n_features
+        self.n_par = (backend.N_PSD_PAR[self.spec.psd_model] + 3 + int(self.log_shift) + 3 * self.n_features +
+                      3 * int(self.periodic_mean))
 
     def __call__(self, theta):
         theta = np.atleast_2d(np.asarray(theta, dtype=np.float64))
@@ -734,6 +740,8 @@ class BatchedLikelihood:
             return self.ctx.approx_features_logl(self.series, self.spec, self.n_features, theta)
         if self.log_shift:
             return self.ctx.approx_logl_logshift(self.series, self.spec, theta)
+        if self.periodic_mean:
+            return self.ctx.approx_logl_sine(self.series, self.spec, theta)
         return self.ctx.approx_logl(self.series, self.spec, theta)[0]
 
     def value_and_gradient(self, theta):
@@ -746,6 +754,8 @@ class BatchedLikelihood:
             return self.ctx.approx_features_logl_grad(self.series, self.spec, self.n_features, theta)
         if self.log_shift:
             return self.ctx.approx_logl_logshift_grad(self.series, self.spec, theta)
+        if self.periodic_mean:
+            return self.ctx.approx_logl_sine_grad(self.series, self.spec, theta)
         return self.ctx.approx_logl_grad(self.series, self.spec, theta)
 
     def gradient(self, theta):

@@ -229,6 +229,17 @@ class Context:
         check(self.lib.pioran_approx_logl_logshift(self.h, series.id, C.byref(spec), theta.shape[0], _p(theta), _p(out)))
         return out
 
+    def approx_logl_sine(self, series, spec, theta):
+        """Sinusoidal mean (examples/ultranest/single_pl_periodicity.jl): theta rows = [psd parameters…, norm, ν, μ, A, ϕ, T₀];
+        m(t) = μ + A·sin(2πt/T₀ + ϕ), y − A·sin(…) formed on the device.  Returns logL [B]."""
+        npar = N_PSD_PAR[spec.psd_model]
+        theta = np.atleast_2d(_f64(theta))
+        if theta.shape[1] != npar + 6:
+            raise ValueError(f"theta must have {npar + 6} columns (psd parameters, norm, ν, μ, A, ϕ, T₀)")
+        out = np.empty(theta.shape[0])
+        check(self.lib.pioran_approx_logl_sine(self.h, series.id, C.byref(spec), theta.shape[0], _p(theta), _p(out)))
+        return out
+
     def approx_logl_dev(self, series_list, specs, B, theta_ptr, out_ptr, theta_per_series=False):
         """Device-resident variant: raw device pointers (ints), asynchronous on the context's stream."""
         S = len(series_list)
@@ -258,6 +269,17 @@ class Context:
         B = theta.shape[0]
         out, grad = np.empty(B), np.empty((B, npar + 4))
         check(self.lib.pioran_approx_logl_logshift_grad(self.h, series.id, C.byref(spec), B, _p(theta), _p(out), _p(grad)))
+        return out, grad
+
+    def approx_logl_sine_grad(self, series, spec, theta):
+        """Sinusoidal mean: theta rows = [psd parameters…, norm, ν, μ, A, ϕ, T₀] → (logL [B], ∂logL/∂θ [B × (n_psd_par + 6)])."""
+        npar = N_PSD_PAR[spec.psd_model]
+        theta = np.atleast_2d(_f64(theta))
+        if theta.shape[1] != npar + 6:
+            raise ValueError(f"theta must have {npar + 6} columns (psd parameters, norm, ν, μ, A, ϕ, T₀)")
+        B = theta.shape[0]
+        out, grad = np.empty(B), np.empty((B, npar + 6))
+        check(self.lib.pioran_approx_logl_sine_grad(self.h, series.id, C.byref(spec), B, _p(theta), _p(out), _p(grad)))
         return out, grad
 
     # -- K5g: forward-mode derivatives of the explicit-coefficient likelihood

@@ -70,7 +70,7 @@ static int guard_fail() {
     } while (0)
 
 extern "C" const char* pioran_last_error(void) { return g_err.c_str(); }
-extern "C" int pioran_version(void) { return 306; }   // 0.3.6: pioran_lombscargle
+extern "C" int pioran_version(void) { return 307; }   // 0.3.7: pioran_approx_logl_sine, pioran_approx_logl_sine_grad
 
 // ------------------------------------------------------------------------------------------------ context
 namespace {
@@ -110,7 +110,7 @@ using PlanKey = std::tuple<int, int, int, int, double, double, double, double>;
 enum KernelFamily : int {
     KF_NONE = 0, KF_BLOCKED, KF_BLOCKED_WIDE, KF_SHARED, KF_SHARED_PAIR, KF_GENERIC, KF_WIDE_REG, KF_WIDE_REG_STORE, KF_WIDE_REG_SIM,
     KF_WIDE, KF_BLOCKED_GRAD, KF_GRAD, KF_GRAD_PIPE, KF_WIDE_GRAD, KF_JVP, KF_PREDICT, KF_GENERIC_SIM, KF_SCAN_FINISH,
-    KF_SCAN_PARTIAL, KF_DENSE_FINISH, KF_VJP, KF_POSTVAR, KF_POSTDRAW, KF_POSTCOV, KF_LSP
+    KF_SCAN_PARTIAL, KF_DENSE_FINISH, KF_VJP, KF_POSTVAR, KF_POSTDRAW, KF_POSTCOV, KF_LSP, KF_BLOCKED_GRAD_SINE
 };
 struct KernelTag { int family = KF_NONE; int p[4] = {0, 0, 0, 0}; };
 
@@ -423,6 +423,7 @@ extern "C" int pioran_ctx_last_kernel_name(pioran_ctx* c, char* buf, int len) tr
         case KF_WIDE_REG_SIM: snprintf(name, sizeof name, "wide_reg_sim<%d>", p[0]); break;
         case KF_WIDE: snprintf(name, sizeof name, "wide"); break;
         case KF_BLOCKED_GRAD: snprintf(name, sizeof name, "blocked_grad<%d,%d,%s,%d>", p[0], p[1], p[2] ? "true" : "false", p[3]); break;
+        case KF_BLOCKED_GRAD_SINE: snprintf(name, sizeof name, "blocked_grad_sine<%d,%d,%s,%d>", p[0], p[1], p[2] ? "true" : "false", p[3]); break;
         case KF_GRAD: snprintf(name, sizeof name, "grad<%d,%d>", p[0], p[1]); break;
         case KF_GRAD_PIPE: snprintf(name, sizeof name, "grad_pipe<%d,%d>", p[0], p[1]); break;
         case KF_WIDE_GRAD: snprintf(name, sizeof name, "wide_grad<%d>", p[0]); break;
@@ -1222,28 +1223,56 @@ static int theta_chunk(int B, size_t bytes_per_set, size_t cap = (size_t)1 << 30
     return (int)std::max<size_t>(1, std::min<size_t>((size_t)B, cap / bytes_per_set));
 }
 
-// The θ-chunk loop of the log-shift entries over the B × ts rows in c->theta: the chunk's transformed data, then
-// fn(first row, row count, the chunk's θ rows, y batch, σ² batch).  16 N bytes of transformed data per parameter vector, at most
-// 1 GiB at a time (written and read once: ≈ 0.3 ms per 65 536 × 1 000 block against tens of ms of sweep).
-template <typename F>
-static int logshift_chunks(pioran_ctx* c, Series* s, int B, int ts, F fn) {
+// Sinusoidal mean (examples/ultranest/single_pl_periodicity.jl): ỹ = y − A·sin(2π·t/T₀ + ϕ) per parameter vector, the argument
+// formed as the reference forms it; μ stays the sweep's scalar.  Columns A, ϕ, T₀ = a_col, a_col + 1, a_col + 2.  The products
+// are rounded as written (no contraction into an FMA), so A = 0 gives ỹ = y exactly.
+__global__ void sine_mean_kernel(const double* __restrict__ y, const double* __restrict__ t, int64_t N, const double* __restrict__ theta,
+                                 int ts, int a_col, int B, double* __restrict__ yb) {
+    const int64_t total = (int64_t)B * N;
+    for (int64_t k = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; k < total; k += (int64_t)gridDim.x * blockDim.x) {
+        const int64_t i = k / N, n = k - i * N;
+        const double* th = theta + i * ts + a_col;
+        const double arg = __dadd_rn(__dmul_rn(6.283185307179586, t[n]) / th[2], th[1]);
+        yb[k] = __dsub_rn(y[n], __dmul_rn(th[0], sin(arg)));
+    }
+}
+
+// The θ-chunk loop of the entries with per-θ data (log-shift, sinusoidal mean) over the B × ts rows in c->theta: for each chunk
+// xf(grid, the chunk's θ rows, row count, y batch, σ² batch) launches the transform that writes the chunk's data, then
+// fn(first row, row count, θ rows, y batch, σ² batch) evaluates it.  nrow rows of 8 N bytes per parameter vector (the σ² batch is
+// nullptr when nrow = 1), at most 1 GiB at a time (written and read once: ≈ 0.3 ms per 65 536 × 1 000 block against tens of ms
+// of sweep).
+template <typename X, typename F>
+static int per_theta_chunks(pioran_ctx* c, Series* s, int B, int ts, int nrow, X xf, F fn) {
     const int64_t N = s->N;
-    const int chunk = theta_chunk(B, 16 * (size_t)N);
+    const int chunk = theta_chunk(B, 8 * (size_t)nrow * N);
     int rc;
-    if ((rc = c->post.ensure(sizeof(double) * 2 * (size_t)chunk * N))) return rc;
+    if ((rc = c->post.ensure(sizeof(double) * nrow * (size_t)chunk * N))) return rc;
     double* yb = c->post.as<double>();
-    double* sb = yb + (size_t)chunk * N;
+    double* sb = nrow > 1 ? yb + (size_t)chunk * N : nullptr;
     for (int off = 0; off < B; off += chunk) {
         const int nb = std::min(chunk, B - off);
         const double* th = c->theta.as<double>() + (size_t)off * ts;
         const int64_t total = (int64_t)nb * N;
         const int grid = (int)std::min<int64_t>((total + 255) / 256, (int64_t)c->num_sms * 16);
-        log_shift_kernel<<<grid, 256, 0, c->stream>>>(s->y, s->s2, N, th, ts, ts - 1, nb, yb, sb);
+        xf(grid, th, nb, yb, sb);
         c->launches++;
         CUDA_TRY(cudaGetLastError());
         if ((rc = fn(off, nb, th, yb, sb))) return rc;
     }
     return 0;
+}
+// The two transforms of per_theta_chunks: the log-shift (c in the last column; two rows) and the sinusoidal mean (A, ϕ, T₀ in the
+// last three columns; one row, σ² stays the resident one).
+static auto log_shift_xf(pioran_ctx* c, Series* s, int ts) {
+    return [=](int grid, const double* th, int nb, double* yb, double* sb) {
+        log_shift_kernel<<<grid, 256, 0, c->stream>>>(s->y, s->s2, s->N, th, ts, ts - 1, nb, yb, sb);
+    };
+}
+static auto sine_mean_xf(pioran_ctx* c, Series* s, int ts) {
+    return [=](int grid, const double* th, int nb, double* yb, double*) {
+        sine_mean_kernel<<<grid, 256, 0, c->stream>>>(s->y, s->t, s->N, th, ts, ts - 3, nb, yb);
+    };
 }
 
 extern "C" int pioran_approx_logl_logshift(pioran_ctx* c, int series_id, const pioran_approx_spec* spec, int B, const double* theta,
@@ -1266,9 +1295,40 @@ extern "C" int pioran_approx_logl_logshift(pioran_ctx* c, int series_id, const p
     if ((rc = c->theta.ensure(sizeof(double) * (size_t)B * ts))) return rc;
     if ((rc = c->out.ensure(sizeof(double) * (size_t)B))) return rc;
     CUDA_TRY(cudaMemcpyAsync(c->theta.p, theta, sizeof(double) * (size_t)B * ts, cudaMemcpyHostToDevice, c->stream));
-    if ((rc = logshift_chunks(c, s, B, ts, [&](int off, int nb, const double* th, const double* yb, const double* sb) {
-             return approx_logl_dev_locked(c, 1, &series_id, spec, nb, th, 0, c->out.as<double>() + off, ts, yb, sb);
-         })))
+    if ((rc = per_theta_chunks(c, s, B, ts, 2, log_shift_xf(c, s, ts),
+                               [&](int off, int nb, const double* th, const double* yb, const double* sb) {
+                                   return approx_logl_dev_locked(c, 1, &series_id, spec, nb, th, 0, c->out.as<double>() + off, ts, yb, sb);
+                               })))
+        return rc;
+    CUDA_TRY(cudaMemcpyAsync(logl_out, c->out.p, sizeof(double) * (size_t)B, cudaMemcpyDeviceToHost, c->stream));
+    CUDA_TRY(cudaStreamSynchronize(c->stream));
+    return PIORAN_OK;
+} catch (...) { return guard_fail(); }
+
+extern "C" int pioran_approx_logl_sine(pioran_ctx* c, int series_id, const pioran_approx_spec* spec, int B, const double* theta,
+                                       double* logl_out) try {
+    if (!c || !spec || !theta || !logl_out) return fail(PIORAN_EINVAL, "NULL argument");
+    if (B < 1) return fail(PIORAN_EINVAL, "B must be >= 1");
+    const int npar = n_psd_par_of(spec->psd_model);
+    if (npar < 0) return fail(PIORAN_EINVAL, "unknown psd_model %d", spec->psd_model);
+    const int ts = npar + 6;
+    if (is_group(c))
+        return group_fanout(c, series_id, B, [&](pioran_ctx* ch, int id, int64_t, int beg, int nb) {
+            return pioran_approx_logl_sine(ch, id, spec, nb, theta + (size_t)beg * ts, logl_out + beg);
+        });
+    PIORAN_COMPUTE_LOCK(c);
+    CUDA_TRY(cudaSetDevice(c->device));
+    int rc;
+    if ((rc = check_spec(*spec))) return rc;
+    Series* s = get_series(c, series_id);
+    if (!s) return fail(PIORAN_EINVAL, "unknown series id %d", series_id);
+    if ((rc = c->theta.ensure(sizeof(double) * (size_t)B * ts))) return rc;
+    if ((rc = c->out.ensure(sizeof(double) * (size_t)B))) return rc;
+    CUDA_TRY(cudaMemcpyAsync(c->theta.p, theta, sizeof(double) * (size_t)B * ts, cudaMemcpyHostToDevice, c->stream));
+    if ((rc = per_theta_chunks(c, s, B, ts, 1, sine_mean_xf(c, s, ts),
+                               [&](int off, int nb, const double* th, const double* yb, const double*) {
+                                   return approx_logl_dev_locked(c, 1, &series_id, spec, nb, th, 0, c->out.as<double>() + off, ts, yb);
+                               })))
         return rc;
     CUDA_TRY(cudaMemcpyAsync(logl_out, c->out.p, sizeof(double) * (size_t)B, cudaMemcpyDeviceToHost, c->stream));
     CUDA_TRY(cudaStreamSynchronize(c->stream));
@@ -1446,36 +1506,39 @@ static int launch_grad(pioran_ctx* c, const GradArgs& args, int nitems, int tpi)
     return tpi <= SMALL_NW ? launch_grad_nw<BS, SMALL_NW>(c, args, nitems) : launch_grad_nw<BS, GRAD_NW>(c, args, nitems);
 }
 // K5t (blocked_grad.cuh): one CTA per parameter vector, value warp + one tangent warp per direction, all on the tensor pipe
-template <int NT, int NTR, bool HALF, int NTAN>
+// SINE: the sinusoidal-mean variant, one more warp (the mean warp) and three more outputs per parameter vector
+template <int NT, int NTR, bool HALF, int NTAN, bool SINE>
 static int launch_blocked_grad(pioran_ctx* c, const GradArgs& args, int nitems, int R, int amp_stride) {
-    auto kern = celerite_blocked_grad_kernel<NT, NTR, HALF, NTAN>;
+    void (*kern)(const GradArgs, const int, const int, const int, const int);
+    if constexpr (SINE) kern = celerite_blocked_grad_sine_kernel<NT, NTR, HALF, NTAN>;
+    else kern = celerite_blocked_grad_kernel<NT, NTR, HALF, NTAN>;
     const size_t smem = sizeof(double) * ((size_t)BLK_NSTAGE * blk_doubles(NT, NTR) + 2 * (size_t)blk_slot_doubles(NTR) +
-                                          (size_t)(1 + NTAN) * (8 * NTR + 8 * NT) + 2) + BLK_NSTAGE * sizeof(uint64_t) + 16;
+                                          (size_t)(1 + NTAN + SINE) * (8 * NTR + 8 * NT) + 2) + BLK_NSTAGE * sizeof(uint64_t) + 16;
     CUDA_TRY(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     cudaEventRecord(c->ev_beg, c->stream);
-    kern<<<nitems, (1 + NTAN) * 32, smem, c->stream>>>(args, R, amp_stride, blk_layout(R, true).RG, blk_layout(R, true).RM);
+    kern<<<nitems, (1 + NTAN + SINE) * 32, smem, c->stream>>>(args, R, amp_stride, blk_layout(R, true).RG, blk_layout(R, true).RM);
     cudaEventRecord(c->ev_end, c->stream);
-    note_kernel(c, KF_BLOCKED_GRAD, NT, NTR, HALF, NTAN);
+    note_kernel(c, SINE ? KF_BLOCKED_GRAD_SINE : KF_BLOCKED_GRAD, NT, NTR, HALF, NTAN);
     c->launches++;
     CUDA_TRY(cudaGetLastError());
     return 0;
 }
-template <int NTAN>
+template <int NTAN, bool SINE = false>
 static int dispatch_blocked_grad(pioran_ctx* c, const GradArgs& a, int nitems, int R, int amp_stride) {
     const BlkLayout lay = blk_layout(R, true);
     const int NT = lay.NT;
     const bool xrow = lay.NTR != NT, half = lay.half;
 #define PIORAN_BLKG_CASE(nt)                                                                                    \
-    case nt: return xrow ? launch_blocked_grad<nt, nt + 1, false, NTAN>(c, a, nitems, R, amp_stride)            \
-                  : half ? launch_blocked_grad<nt, nt, true, NTAN>(c, a, nitems, R, amp_stride)                 \
-                         : launch_blocked_grad<nt, nt, false, NTAN>(c, a, nitems, R, amp_stride);
+    case nt: return xrow ? launch_blocked_grad<nt, nt + 1, false, NTAN, SINE>(c, a, nitems, R, amp_stride)      \
+                  : half ? launch_blocked_grad<nt, nt, true, NTAN, SINE>(c, a, nitems, R, amp_stride)           \
+                         : launch_blocked_grad<nt, nt, false, NTAN, SINE>(c, a, nitems, R, amp_stride);
     switch (NT) {
         PIORAN_BLKG_CASE(1) PIORAN_BLKG_CASE(2) PIORAN_BLKG_CASE(3) PIORAN_BLKG_CASE(4)
         PIORAN_BLKG_CASE(5) PIORAN_BLKG_CASE(6) PIORAN_BLKG_CASE(7)
         case 8:
             if (xrow) break;
-            return half ? launch_blocked_grad<8, 8, true, NTAN>(c, a, nitems, R, amp_stride)
-                        : launch_blocked_grad<8, 8, false, NTAN>(c, a, nitems, R, amp_stride);
+            return half ? launch_blocked_grad<8, 8, true, NTAN, SINE>(c, a, nitems, R, amp_stride)
+                        : launch_blocked_grad<8, 8, false, NTAN, SINE>(c, a, nitems, R, amp_stride);
     }
 #undef PIORAN_BLKG_CASE
     return fail(PIORAN_EUNSUPPORTED, "rank %d not served by the blocked gradient kernel", R);
@@ -1484,7 +1547,6 @@ static bool blocked_grad_enabled(const pioran_ctx* c, int R, int ND) {
     return blocked_enabled(c, R) && blk_layout(R, true).NTR <= 8 && (ND == 3 || ND == 5);
 }
 
-// logshift: θ rows carry a further column c and (y_batch, s2_batch) hold the per-θ transformed data; the gradient gains ∂/∂c.
 // Gradient at ranks 65 … 96 (wide_grad.cuh): K1 tangents in row form, then one CTA per (parameter vector, direction).
 static int wide_grad_locked(pioran_ctx* c, Series* ser, const pioran_approx_spec* spec, int B, const double* theta_dev,
                             double* logl_dev, double* grad_dev, int R, int npar, int ts) {
@@ -1546,27 +1608,31 @@ static int wide_grad_locked(pioran_ctx* c, Series* ser, const pioran_approx_spec
     return 0;
 }
 
+// logshift: θ rows carry a further column c and (y_batch, s2_batch) hold the per-θ transformed data; the gradient gains ∂/∂c.
+// sine: θ rows carry three further columns A, ϕ, T₀ and y_batch holds y − A·sin(2πt/T₀ + ϕ); the gradient gains their partials.
 static int approx_logl_grad_dev_locked(pioran_ctx* c, int series_id, const pioran_approx_spec* spec, int B,
                                        const double* theta_dev, double* logl_dev, double* grad_dev, bool logshift = false,
-                                       const double* y_batch = nullptr, const double* s2_batch = nullptr) {
+                                       const double* y_batch = nullptr, const double* s2_batch = nullptr, bool sine = false) {
     int rc;
     if (B < 1) return fail(PIORAN_EINVAL, "B must be >= 1");
     if ((rc = check_spec(*spec))) return rc;
     Series* ser = get_series(c, series_id);
     if (!ser) return fail(PIORAN_EINVAL, "unknown series id %d", series_id);
-    const int npar = n_psd_par_of(spec->psd_model), ts = npar + 3 + (logshift ? 1 : 0), ND = npar, P = ts;
+    const int npar = n_psd_par_of(spec->psd_model), ts = npar + 3 + (logshift ? 1 : 0) + (sine ? 3 : 0), ND = npar, P = ts;
     if ((long long)B * P > 0x7fffffffLL / 64) return fail(PIORAN_EINVAL, "B too large");
     const int R = rank_of(spec->basis, spec->n_components);
     const int BS = bs_for_rank(R);
     if (BS > 8) {
-        if (R > 96 || logshift || y_batch || s2_batch)
-            return fail(PIORAN_EUNSUPPORTED, "gradients are built for ranks <= 96 (log-shift model: <= 62); rank %d", R);
+        if (R > 96 || logshift || sine || y_batch || s2_batch)
+            return fail(PIORAN_EUNSUPPORTED, "gradients are built for ranks <= 96 (log-shift and sinusoidal-mean models: <= 62); rank %d", R);
         return wide_grad_locked(c, ser, spec, B, theta_dev, logl_dev, grad_dev, R, npar, ts);
     }
     const int RP = G * BS;
     const bool blkg = blocked_grad_enabled(c, R, ND);
     if (logshift && !(blkg && ND == 3))
         return fail(PIORAN_EUNSUPPORTED, "the log-shift gradient is built for SingleBendingPowerLaw at ranks <= 62 (rank %d, %d PSD parameters)", R, ND);
+    if (sine && !blkg)
+        return fail(PIORAN_EUNSUPPORTED, "the sinusoidal-mean gradient is built for the blocked gradient kernel, ranks <= 62 (rank %d)", R);
     Table tab;
     if ((rc = blkg ? get_btable(c, ser, *spec, &tab, true) : get_table(c, ser, *spec, &tab))) return rc;
     ApproxPlan* plan;
@@ -1608,6 +1674,7 @@ static int approx_logl_grad_dev_locked(pioran_ctx* c, int series_id, const piora
     ga.y_batch = y_batch; ga.s2_batch = s2_batch; ga.ystride = ser->N; ga.cdir = logshift ? 1 : 0;
     const int nitems = c->gwork_items;
     if (blkg && logshift) return dispatch_blocked_grad<5>(c, ga, nitems, R, RP);
+    if (blkg && sine) return ND == 3 ? dispatch_blocked_grad<4, true>(c, ga, nitems, R, RP) : dispatch_blocked_grad<6, true>(c, ga, nitems, R, RP);
     if (blkg) return ND == 3 ? dispatch_blocked_grad<4>(c, ga, nitems, R, RP) : dispatch_blocked_grad<6>(c, ga, nitems, R, RP);
     if (pipe) {
         const int nwarps = 1 + ND + 1;
@@ -1658,9 +1725,46 @@ extern "C" int pioran_approx_logl_logshift_grad(pioran_ctx* c, int series_id, co
     CUDA_TRY(cudaMemcpyAsync(c->theta.p, theta, sizeof(double) * (size_t)B * ts, cudaMemcpyHostToDevice, c->stream));
     double* gl = c->out.as<double>();
     double* gg = gl + B;
-    if ((rc = logshift_chunks(c, s, B, ts, [&](int off, int nb, const double* th, const double* yb, const double* sb) {
-             return approx_logl_grad_dev_locked(c, series_id, spec, nb, th, gl + off, gg + (size_t)off * ts, true, yb, sb);
-         })))
+    if ((rc = per_theta_chunks(c, s, B, ts, 2, log_shift_xf(c, s, ts),
+                               [&](int off, int nb, const double* th, const double* yb, const double* sb) {
+                                   return approx_logl_grad_dev_locked(c, series_id, spec, nb, th, gl + off, gg + (size_t)off * ts, true, yb, sb);
+                               })))
+        return rc;
+    if (logl_out) CUDA_TRY(cudaMemcpyAsync(logl_out, gl, sizeof(double) * (size_t)B, cudaMemcpyDeviceToHost, c->stream));
+    CUDA_TRY(cudaMemcpyAsync(grad_out, gg, sizeof(double) * (size_t)B * ts, cudaMemcpyDeviceToHost, c->stream));
+    CUDA_TRY(cudaStreamSynchronize(c->stream));
+    return PIORAN_OK;
+} catch (...) { return guard_fail(); }
+
+// Gradient of the sinusoidal-mean likelihood (the reference's periodicity run differentiated like its other models,
+// test/test_likelihood.jl:55): ỹ on the device, then K1 tangents + the blocked gradient kernel with the mean warp.
+extern "C" int pioran_approx_logl_sine_grad(pioran_ctx* c, int series_id, const pioran_approx_spec* spec, int B,
+                                            const double* theta, double* logl_out, double* grad_out) try {
+    if (!c || !spec || !theta || !grad_out) return fail(PIORAN_EINVAL, "NULL argument");
+    if (B < 1) return fail(PIORAN_EINVAL, "B must be >= 1");
+    const int npar = n_psd_par_of(spec->psd_model);
+    if (npar < 0) return fail(PIORAN_EINVAL, "unknown psd_model %d", spec->psd_model);
+    const int ts = npar + 6;
+    if (is_group(c))
+        return group_fanout(c, series_id, B, [&](pioran_ctx* ch, int id, int64_t, int beg, int nb) {
+            return pioran_approx_logl_sine_grad(ch, id, spec, nb, theta + (size_t)beg * ts, at(logl_out, beg), grad_out + (size_t)beg * ts);
+        });
+    PIORAN_COMPUTE_LOCK(c);
+    CUDA_TRY(cudaSetDevice(c->device));
+    int rc;
+    if ((rc = check_spec(*spec))) return rc;
+    Series* s = get_series(c, series_id);
+    if (!s) return fail(PIORAN_EINVAL, "unknown series id %d", series_id);
+    if ((rc = c->theta.ensure(sizeof(double) * (size_t)B * ts))) return rc;
+    if ((rc = c->out.ensure(sizeof(double) * (size_t)B * (ts + 1)))) return rc;
+    CUDA_TRY(cudaMemcpyAsync(c->theta.p, theta, sizeof(double) * (size_t)B * ts, cudaMemcpyHostToDevice, c->stream));
+    double* gl = c->out.as<double>();
+    double* gg = gl + B;
+    if ((rc = per_theta_chunks(c, s, B, ts, 1, sine_mean_xf(c, s, ts),
+                               [&](int off, int nb, const double* th, const double* yb, const double*) {
+                                   return approx_logl_grad_dev_locked(c, series_id, spec, nb, th, gl + off, gg + (size_t)off * ts, false, yb,
+                                                                      nullptr, true);
+                               })))
         return rc;
     if (logl_out) CUDA_TRY(cudaMemcpyAsync(logl_out, gl, sizeof(double) * (size_t)B, cudaMemcpyDeviceToHost, c->stream));
     CUDA_TRY(cudaMemcpyAsync(grad_out, gg, sizeof(double) * (size_t)B * ts, cudaMemcpyDeviceToHost, c->stream));

@@ -146,16 +146,22 @@ def vectorized_callbacks_log_normal(t, y, yerr, psd_model="SingleBendingPowerLaw
 
 
 def vectorized_callbacks(t, y, yerr, psd_model="SingleBendingPowerLaw", n_components=20, basis_function="SHO",
-                         log_transform=True, prior=None, ctx=None, device_prior=False, **approx_kw):
+                         log_transform=True, prior=None, ctx=None, device_prior=False, periodic_mean=False, **approx_kw):
     """(loglike, transform, close) for `ultranest.ReactiveNestedSampler(paramnames, loglike, transform=transform,
-    vectorized=True)`.  log_transform follows single_pl.jl:70-73 (σ² = ν σ²/y², yn = log y); the series is uploaded once."""
+    vectorized=True)`.  log_transform follows single_pl.jl:70-73 (σ² = ν σ²/y², yn = log y); the series is uploaded once.
+    periodic_mean: Θ rows end with (A, ϕ, T₀) and the mean is μ + A·sin(2πt/T₀ + ϕ) (single_pl_periodicity.jl, which
+    samples with log_transform=False); its prior must be given, as the reference run's priors of A, ϕ and T₀ are not known here."""
     from .api import BatchedLikelihood
+    if periodic_mean and prior is None:
+        raise ValueError("periodic_mean=True needs an explicit prior (transform over psd parameters…, variance, ν, μ, A, ϕ, T₀)")
+    if periodic_mean and device_prior:
+        raise ValueError("the fused prior-transform entry takes no periodic mean; use device_prior=False")
     t, y, yerr = (np.asarray(x, dtype=np.float64) for x in (t, y, yerr))
     if log_transform:
         yn, s2 = np.log(y), yerr ** 2 / y ** 2
     else:
         yn, s2 = y, yerr ** 2
-    like = BatchedLikelihood(t, yn, s2, psd_model, n_components, basis_function, ctx=ctx, **approx_kw)
+    like = BatchedLikelihood(t, yn, s2, psd_model, n_components, basis_function, ctx=ctx, periodic_mean=periodic_mean, **approx_kw)
     if prior is None:
         f_min, f_max = 1.0 / (t[-1] - t[0]), 1.0 / np.min(np.diff(t)) / 2.0
         prior = single_bending_power_law_prior(f_min, f_max, float(np.mean(yn)), float(np.var(yn, ddof=1)),
